@@ -24,6 +24,9 @@ kernels answer many lookups with one request.  The random-request ceiling of the
 own tables (fmb_measure_gather).
 
 Sizes can be reduced for smoke runs with --text / --reads / --read-len (the JSON line then names the reduced workload).
+
+--dump-outputs DIR writes what the last timed step returned (the hits of the search and the rows of locate) as .npy files, so that
+two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -39,6 +42,8 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 LINE_BYTES = 128.0     # DRAM bytes moved by one random request (profiles/r01_ncu_full_exact2_locate.txt: 116 B per 32-B lookup)
+DUMP_QUERIES = 1 << 14                # --dump-outputs: queries in the fixed sample whose results are written
+DUMP_BYTES = 64 << 20                 # --dump-outputs: upper bound of all files together
 
 
 def log(*a):
@@ -187,6 +192,19 @@ def ref_name_of(scheme, edit, k):
     return "search_no_errors::search (batched)" if scheme is None else f"search_ng26::search<{'true' if edit else 'false'}>(optimum(0,{k}))"
 
 
+def output_sample(res, loc, nq, max_bytes):
+    """what one step returned, for --dump-outputs: the hits and located rows of a fixed, seeded sample of the queries as float64
+    arrays (one column per field, exact below 2^53), sorted by all fields because the device reports them in an order that depends
+    on scheduling; each array is cut to `max_bytes`.  `counts` = rows of the whole output (hits, located rows)."""
+    sample = np.random.default_rng(0).choice(nq, size=min(nq, DUMP_QUERIES), replace=False).astype(np.uint64)
+    out = {"counts": np.array([len(res), len(loc)], dtype=np.float64)}
+    for name, rec in (("hits", res.hits()), ("locs", loc.locs())):
+        rec = np.sort(rec[np.isin(rec["qidx"], sample)], order=list(rec.dtype.names))
+        arr = np.stack([rec[f].astype(np.float64) for f in rec.dtype.names], axis=1)
+        out[name] = arr[: max_bytes // (arr.itemsize * arr.shape[1])]
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -204,7 +222,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target CPU time of the headline cpu_baseline sample (the other workloads get a third)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--image-gb", type=float, default=0.0, help="HBM budget of the index image in GB (fmb_set_image_budget; 0 = every table that fits)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the hits and located rows of the last timed step (fixed sample of the queries, float64) to DIR/<workload>_*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: use it with --impl ours")
 
     wls = list(DNA_SET) if args.workload == "all" else [args.workload]
     head = wls[0]
@@ -215,7 +239,7 @@ def main():
     nq_total = int(args.reads) if args.reads else (250_000 if fam == "repeat" else (1_000_000 if protein else (100_000 if head == "c1" else 10_000_000)))
     L = args.read_len if args.read_len else (20 if head == "locate-heavy" else (50 if protein else (100 if head == "c1" else 150)))
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -368,6 +392,7 @@ def main():
     sampler.start()
     launches0 = capi.kernel_launch_count()
     results, e2e_locs = {}, {}
+    dumps = {} if args.dump_outputs and rank == 0 else None          # rank 0's reads only
     for wl in wls:
         sym, off = data[wl]
         scheme, partition, edit, k = scheme_of(wl, L)
@@ -400,14 +425,18 @@ def main():
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record(stream)
         search_ms, locate_ms, st_s, st_l = [], [], None, None
-        for _ in range(K):
+        for i in range(K):
             res, loc = step()
             search_ms.append(res.stats.main_kernel_ms)
             locate_ms.append(loc.stats.main_kernel_ms)
             st_s, st_l = res.stats, loc.stats
-            del res, loc
+            if i + 1 < K or dumps is None:
+                del res, loc
         ev1.record(stream)
         barrier()
+        if dumps is not None:
+            dumps[wl] = output_sample(res, loc, nq, DUMP_BYTES // (3 * len(wls)))
+            del res, loc
         ms_per_step = max_over_ranks(ev0.elapsed_time(ev1)) / K
         q_all = nq_total if strong else nq * world
         value = q_all / (ms_per_step * 1e-3)
@@ -573,6 +602,11 @@ def main():
     launches = capi.kernel_launch_count() - launches0
     clocks = sampler.stop()
     clocks["window"] = "warm-up + timed steps + e2e loops of all workloads"
+    if dumps is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for wl, arrays in dumps.items():
+            for name, arr in arrays.items():
+                np.save(os.path.join(args.dump_outputs, f"{wl}_{name}.npy"), arr)
 
     h = results[head]
     line = {"metric": metric_head, "value": h["value"], "unit": "queries/s", "n_gpus": world,

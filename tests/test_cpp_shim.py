@@ -71,10 +71,8 @@ int main() {
 
 
 def test_shim_binary_fails_loudly_without_device():
-    import fmb200
-    if fmb200.device_count() > 0:
-        pytest.skip("a CUDA device is visible")
-    r = subprocess.run([_binary("shim_test")], capture_output=True, text=True)
+    # the devices are hidden from the binary, so that the check also runs where a GPU is present
+    r = subprocess.run([_binary("shim_test")], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True)
     assert r.returncode == 2 and "no CPU fallback" in r.stderr
 
 
@@ -152,6 +150,66 @@ int main(int argc, char** argv) {
                    "123410", "threw=1 missing=0", "packed=1 exceptions=4"]
     assert (tmp_path / "out.txt").read_text() == "3 0 17\n4 1 2\n"
     assert (tmp_path / "out.txt2").read_text() == "7 1 99\n"
+
+
+def test_fold_of_expanded_reference_schemes(tmp_path):
+    """search_pseudo's fold() of an expanded scheme re-expands to exactly the same per-symbol scheme -- i.e. the part form handed to
+    the device describes the same search -- for the tables of the reference's generators stored in tests/golden/ref_vectors.json
+    and many lengths (CPU only: no device call)"""
+    import json
+    with open(os.path.join(ROOT, "tests", "golden", "ref_vectors.json")) as f:
+        tables = {k: v for k, v in json.load(f)["schemes"].items() if k.split(":")[1] == "0" and v[0]}
+
+    def lst(v):
+        return "{" + ",".join(str(x) for x in v) + "}"
+    literal = ",\n".join("{" + ",".join("{%s,%s,%s}" % (lst(pi), lst(l), lst(u)) for pi, l, u in zip(*t)) + "}" for t in tables.values())
+    src = tmp_path / "f.cpp"
+    src.write_text(r'''
+#include <algorithm>
+#include <cstdio>
+#include "fmb200/fmb200.hpp"
+namespace ms = fmb200::search_scheme;
+int main() {
+    std::vector<ms::Scheme> schemes = {
+''' + literal + r'''
+    };
+    int checks = 0, bad = 0;
+    for (auto const& mine : schemes) {
+        for (size_t L : {mine[0].pi.size(), mine[0].pi.size() + 1, size_t{7}, size_t{20}, size_t{50}, size_t{151}}) {
+            if (L < mine[0].pi.size()) continue;
+            auto e_mine = ms::expand(mine, L);
+            if (e_mine.empty()) continue;
+            // fold back into parts and expand again with the folded partition: must reproduce pi and u exactly, and a lower bound
+            // sequence that accepts exactly the same (position, errors) pairs: max over the prefix is what counts (e never decreases)
+            auto [folded, partition] = fmb200::search_pseudo::detail_pseudo::fold(e_mine);
+            auto again = ms::expand(folded, partition);
+            ++checks;
+            bool ok = again.size() == e_mine.size() && partition.size() <= 16;
+            for (size_t i = 0; ok && i < again.size(); ++i) {
+                // the first part may be walked in either direction (search_ng26 and the device always walk it to the right): same
+                // symbols, same bounds -- compare it as a set
+                auto first = [&](ms::Search x) { std::sort(x.pi.begin(), x.pi.begin() + partition[folded[i].pi[0]]); return x.pi; };
+                ok = first(again[i]) == first(e_mine[i]) && again[i].u == e_mine[i].u;
+                size_t ma = 0, mb = 0;
+                for (size_t p = 0; ok && p < L; ++p) { ma = std::max(ma, again[i].l[p]); mb = std::max(mb, e_mine[i].l[p]); ok = ma == mb; }
+            }
+            if (!ok) { ++bad; std::printf("fold differs (L=%zu, parts=%zu)\n", L, partition.size()); }
+        }
+    }
+    std::printf("%d checks, %d bad\n", checks, bad);
+    return bad != 0 || checks < 100;
+}
+''')
+    exe = tmp_path / "f"
+    lib = os.path.join(ROOT, "fmindex-collection_b200")
+    import fmb200  # noqa: F401
+    from fmb200 import build as b
+    b.build()
+    subprocess.run(["g++", "-std=c++20", "-O1", "-Wno-comment", "-I", os.path.join(ROOT, "include"), str(src), "-L", lib, "-lfmb200",
+                    f"-Wl,-rpath,{lib}", "-o", str(exe)], check=True)
+    r = subprocess.run([str(exe)], capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert " 0 bad" in r.stdout
 
 
 REF_SRC = "/root/reference/src"

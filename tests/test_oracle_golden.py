@@ -323,26 +323,63 @@ def test_checkSearches_pseudo(check_searches):
     assert located(o, o.search_pseudo(sym, off, expanded, False)) == HAM
 
 
-@pytest.mark.skipif(not Ref.available(), reason="oracle/_ref/libfmref.so not built (needs /root/reference)")
-def test_pseudo_oracle_vs_reference_library():
-    from fmb200 import schemes, synth
+def _pseudo_inputs():
+    from fmb200 import synth
     text = synth.multi_text([1800, 600], 5, 61)
-    o = Oracle.build(text, 5, 4)
-    r = Ref.build(text, 5, 4)
     L = 18
     reads, _ = synth.reads_from_text(text[:1800], 60, L, 5)
     reads = synth.plant_errors(reads, 5, 1, True, 6)
-    sym, off = synth.flatten(reads)
+    return text, L, *synth.flatten(reads)
+
+
+def _pseudo_schemes(k):
+    from fmb200 import schemes
+    return schemes.optimum(0, k), schemes.h2(k + 2, 0, k), schemes.backtracking(k + 1, 0, k)
+
+
+@pytest.mark.skipif(not Ref.available(), reason="oracle/_ref/libfmref.so not built (needs /root/reference)")
+def test_pseudo_oracle_vs_reference_library():
+    from fmb200 import schemes
+    text, L, sym, off = _pseudo_inputs()
+    o = Oracle.build(text, 5, 4)
+    r = Ref.build(text, 5, 4)
     total = 0
     for k in (1, 2):
-        for sch in (schemes.optimum(0, k), schemes.h2(k + 2, 0, k), schemes.backtracking(k + 1, 0, k)):
+        for sch in _pseudo_schemes(k):
             expanded = schemes.expand(sch, schemes.uniform_partition(sch[0].shape[1], L))
             for edit in (False, True):
                 a, b = sort_hits(o.search_pseudo(sym, off, expanded, edit)), sort_hits(r.search_pseudo(sym, off, expanded, edit))
                 assert np.array_equal(a, b), (k, edit)
                 total += len(a)
-            # Hamming: the per-symbol search equals the per-part search of search_ng26 (the argument behind the device's fold)
+    assert total > 1000
+
+
+def test_pseudo_hamming_equals_ng26():
+    """Hamming: the per-symbol search equals the per-part search of search_ng26 (the argument behind the device's fold)"""
+    from fmb200 import schemes
+    text, L, sym, off = _pseudo_inputs()
+    o = Oracle.build(text, 5, 4)
+    for k in (1, 2):
+        for sch in _pseudo_schemes(k):
             ham = schemes.limit_to_hamming(sch)
             part = schemes.uniform_partition(sch[0].shape[1], L)
             assert np.array_equal(sort_hits(o.search_pseudo(sym, off, schemes.expand(ham, part), False)), sort_hits(o.search_ng26(sym, off, ham, part, False)))
-    assert total > 1000
+
+
+def test_pseudo_hamming_matches_reference_vectors(golden):
+    """search_pseudo with Hamming distance on the expanded scheme reports exactly the hits of the reference's own search_ng26 and
+    search facade on the unexpanded one (tests/golden/ref_vectors.json): anchors the oracle's search_pseudo, which the device's
+    pseudo search is checked against, on outputs of the reference"""
+    from fmb200 import schemes, synth
+    total = 0
+    for c in golden["cases"]:
+        o = Oracle.build(np.array(c["text"], dtype=np.uint8), 5, c["rate"])
+        sym, off = synth.flatten(np.array(c["queries"], dtype=np.uint8))
+        for k in (1, 2):
+            sch = schemes.optimum(0, k)
+            for key, (s, part) in ((f"ng26_optimum_k{k}_ham", (sch, schemes.uniform_partition(sch[0].shape[1], c["L"]))),
+                                   (f"facade_k{k}_ham", schemes.facade_scheme(False, k, c["L"]))):
+                got = sort_hits(o.search_pseudo(sym, off, schemes.expand(s, part), False))
+                assert np.array_equal(got, _hits_arr(c["searches"][key]["hits"])), (c["name"], key)
+                total += len(got)
+    assert total > 250
