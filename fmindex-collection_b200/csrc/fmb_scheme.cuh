@@ -540,6 +540,10 @@ __global__ void __launch_bounds__(256, FMB_SCHEME_MINB) scheme_search_kernel(con
         }
         if (top == 0) {
             if (!more_roots) break;
+            // progress: staged text items (ttop <= 31) leave only in groups of 32, so with nothing pending they alone can keep the
+            // refill from having room for a round of roots.  Flushed, they leave top + ttop = 0, which every cap >= 32 (checked on
+            // the host) admits: each iteration pops, pulls roots or ends.
+            if (ttop + 32 > cap) flush_text(ttop);
             continue;
         }
         peak = top > peak ? top : peak;

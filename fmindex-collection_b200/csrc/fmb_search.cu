@@ -110,21 +110,48 @@ int launch_text(const fmb_index* ix, const SchemeParams& sp, const fmb_queries* 
                   : launch_text_t<OccGen, true, false>(ix, ix->view_gen(), sp, q, items, n_items, out, st);
 }
 
+// FMB_SCHEME_CAP: items per warp stack of the frontier kernel (read once per process).  A warp takes roots 32 at a time, so a stack of
+// fewer than 32 items could never take one, and a block whose stacks exceed the device's shared memory cannot launch: both are
+// refused before any launch.
+int scheme_stack_cap(int dev, size_t item_bytes, uint32_t* cap) {
+    static const char* env = getenv("FMB_SCHEME_CAP");
+    unsigned long long v = kStackCapDefault;
+    if (env) {
+        char* end = nullptr;
+        v = strtoull(env, &end, 10);
+        if (end == env || *end != '\0') { set_error("FMB_SCHEME_CAP=%s is not a number", env); return FMB_EINVAL; }
+    }
+    int smem_max = 0;
+    FMB_CUDA(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    const unsigned long long v_max = (unsigned long long)smem_max / (kWarpsPerBlock * item_bytes);
+    if (v < 32 || v > v_max) {
+        set_error("FMB_SCHEME_CAP=%llu: the frontier kernel's warp stacks hold 32..%llu items on device %d", v, v_max, dev);
+        return FMB_EINVAL;
+    }
+    *cap = (uint32_t)v;
+    return FMB_OK;
+}
+
 template <class OCC, bool EDIT, bool ORDERED, bool PSEUDO>
 int launch_scheme_t(const fmb_index* ix, const IndexView<OCC>& view, const SchemeParams& sp, const fmb_queries* q, uint64_t n_roots, const Item* in_items,
                     uint64_t n_in, const SchemeOut& out, cudaStream_t st) {
-    static const uint32_t kStackCap = getenv("FMB_SCHEME_CAP") ? (uint32_t)atoi(getenv("FMB_SCHEME_CAP")) : kStackCapDefault;
-    size_t smem = (size_t)kStackCap * kWarpsPerBlock * (sizeof(Item) + (ORDERED ? sizeof(unsigned long long) : 0));
+    constexpr size_t kItemBytes = sizeof(Item) + (ORDERED ? sizeof(unsigned long long) : 0);
     auto kern = scheme_search_kernel<OCC, EDIT, ORDERED, PSEUDO>;
     // launch geometry, computed once per kernel instantiation (several host threads drive one index in the pipelined path)
     // (cached per device: several replicas of an index may be driven from concurrent threads, fmb200/multi.hpp)
     static std::mutex cfg_mu;
     static int cfg_blocks_per_sm[kMaxDevices] = {}, cfg_sms[kMaxDevices] = {};
+    static uint32_t cfg_cap[kMaxDevices] = {};
     int blocks_per_sm, sms;
+    uint32_t stack_cap;
+    size_t smem;
     {
         std::lock_guard<std::mutex> lk(cfg_mu);
         const int dev = ix->device;
         if (dev < 0 || dev >= kMaxDevices) { set_error("device %d outside [0,%d)", dev, kMaxDevices); return FMB_EINVAL; }
+        if (!cfg_cap[dev]) FMB_TRY(scheme_stack_cap(dev, kItemBytes, &cfg_cap[dev]));
+        stack_cap = cfg_cap[dev];
+        smem = (size_t)stack_cap * kWarpsPerBlock * kItemBytes;
         FMB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));      // per device
         if (!cfg_blocks_per_sm[dev]) {
             int bps = 0;
@@ -145,7 +172,7 @@ int launch_scheme_t(const fmb_index* ix, const IndexView<OCC>& view, const Schem
     static const char* sim_env = getenv("FMB_SCHEME_SIMALL");
     const uint32_t sim_all = sim_env ? (uint32_t)atoi(sim_env) : 1u;
     const uint32_t ff_min = (ff_env ? (uint32_t)atoi(ff_env) : (EDIT ? 16u : 8u)) | (sim_all << 8);
-    kern<<<grid, 256, smem, st>>>(view, sp, q->symbols.p, q->offsets.p, jv, n_roots, in_items, n_in, out, kStackCap, ff_min);
+    kern<<<grid, 256, smem, st>>>(view, sp, q->symbols.p, q->offsets.p, jv, n_roots, in_items, n_in, out, stack_cap, ff_min);
     FMB_CUDA(cudaGetLastError());
     note_launches(1);
     return FMB_OK;

@@ -20,15 +20,50 @@ def big(gpu):
     capi.device_free(0, d_text)
 
 
-def _reads(capi, d_text, kind, k=0, edit=False):
+def _reads(capi, d_text, kind, k=0, edit=False, length=L, nq=NQ):
     if kind == "exact":
-        d = capi.synth_reads_device(0, d_text, N_TEXT, NQ, L, 12)
+        d = capi.synth_reads_device(0, d_text, N_TEXT, nq, length, 12)
     else:
-        d = capi.synth_reads_err_device(0, d_text, N_TEXT, NQ, L, 12, 5, k, edit)
-    sym = np.zeros(NQ * L, dtype=np.uint8)
-    capi.copy_to_host(0, sym, d, NQ * L)
+        d = capi.synth_reads_err_device(0, d_text, N_TEXT, nq, length, 12, 5, k, edit)
+    sym = np.zeros(nq * length, dtype=np.uint8)
+    capi.copy_to_host(0, sym, d, nq * length)
     capi.device_free(0, d)
-    return sym, np.arange(NQ + 1, dtype=np.uint64) * np.uint64(L)
+    return sym, np.arange(nq + 1, dtype=np.uint64) * np.uint64(length)
+
+
+@pytest.fixture(scope="module")
+def big_oracle(big):
+    """the oracle on the device index's own BWT and samples (its checkpoints take ~5 MB per direction at this size)"""
+    from oracle.pyoracle import Oracle
+    gpu, capi, index, _ = big
+    return Oracle.from_bwt(5, *index.export())
+
+
+SAMPLE = 2000
+
+
+def _sample_parity(index, o, search, sym, off, res, length, locate=True):
+    """the device's hits (and located rows) of a fixed sample of SAMPLE reads of the whole batch == the oracle's for those reads alone
+    (search(symbols, offsets): the oracle's hits)"""
+    from helpers import hits_equal, locs_equal
+    nq = off.size - 1
+    size = min(SAMPLE, nq)
+    sample = np.sort(np.random.default_rng(2024).choice(nq, size, replace=False)).astype(np.uint64)
+    renum = np.full(nq, -1, dtype=np.int64)
+    renum[sample] = np.arange(size)
+    ssym = sym.reshape(nq, length)[sample].reshape(-1)
+    soff = np.arange(size + 1, dtype=np.uint64) * np.uint64(length)
+    hits = res.hits()
+    got = hits[renum[hits["qidx"].astype(np.int64)] >= 0]
+    got["qidx"] = renum[got["qidx"].astype(np.int64)]
+    exp = search(ssym, soff)
+    assert len(exp) >= size // 2
+    assert hits_equal(got, exp)
+    if locate:
+        locs = index.locate(res).locs()
+        gl = locs[renum[locs["qidx"].astype(np.int64)] >= 0]
+        gl["qidx"] = renum[gl["qidx"].astype(np.int64)]
+        assert locs_equal(gl, o.locate(exp))
 
 
 def _source_offsets():
@@ -127,6 +162,53 @@ def test_reads_with_planted_errors_are_found(big, k, edit):
     # the jump / k-mer accelerated kernel and the plain frontier kernel report the same multiset
     st = res.stats
     assert 0 < st.line_requests < st.occ_lookups
+
+
+@pytest.mark.parametrize("k,edit", [(1, False), (2, False), (1, True), (2, True)])
+def test_sample_of_the_batch_matches_oracle(big, big_oracle, k, edit):
+    """the whole 10^6-read batch on the device; the hits and located rows of a fixed sample of 2000 reads equal the oracle's"""
+    from fmb200 import schemes
+    gpu, capi, index, d_text = big
+    sym, off = _reads(capi, d_text, "err", k, edit)
+    sch = schemes.optimum(0, k)
+    part = schemes.uniform_partition(sch[0].shape[1], L)
+    res = index.search_scheme(index.upload(sym, off), sch, part, edit)
+    _sample_parity(index, big_oracle, lambda s, f: big_oracle.search_ng26(s, f, sch, part, edit), sym, off, res, L)
+
+
+def _bikmer_k(n):
+    """k of the bidirectional k-mer table of a DNA index of n rows (csrc/fmb_lib.cu build_bikmer): the largest k <= 14 with 8 * 4^k <= n"""
+    k = 0
+    while k < 14 and 8 << (2 * (k + 1)) <= n:
+        k += 1
+    return k
+
+
+@pytest.mark.parametrize("length", [24, 40])
+@pytest.mark.parametrize("edit", [False, True])
+def test_short_reads_skip_the_bidirectional_kmer_table(big, big_oracle, length, edit):
+    """k = 2 on 24- and 40-symbol reads: the error-free first parts (6 and 10 symbols) are shorter than the bidirectional k-mer
+    table's k, so the roots start at the full interval and the wide-interval phase runs on the index.  (Such reads have hundreds of
+    single-row paths per root: batches much larger than these exceed the frontier lists, which the search reports as FMB_EOVERFLOW.)"""
+    from fmb200 import schemes
+    gpu, capi, index, d_text = big
+    sch = schemes.optimum(0, 2)
+    part = schemes.uniform_partition(sch[0].shape[1], length)
+    bk = _bikmer_k(index.info.n)
+    assert bk == 11 and max(part) < bk
+    sym, off = _reads(capi, d_text, "err", 2, edit, length, {24: 250, 40: 1500}[length])
+    res = index.search_scheme(index.upload(sym, off), sch, part, edit)
+    _sample_parity(index, big_oracle, lambda s, f: big_oracle.search_ng26(s, f, sch, part, edit), sym, off, res, length)
+
+
+@pytest.mark.parametrize("length", [8, 10, 11, 12, 13, 16])
+def test_exact_reads_around_the_kmer_table_k(big, big_oracle, length):
+    """exact search of reads as long as the exact k-mer table's k (11 here) and around it; located rows for the reads of 12 symbols and
+    more (the shorter ones have intervals of hundreds of rows)"""
+    gpu, capi, index, d_text = big
+    sym, off = _reads(capi, d_text, "exact", length=length, nq=200_000)
+    res = index.search_exact(index.upload(sym, off))
+    _sample_parity(index, big_oracle, big_oracle.search_exact, sym, off, res, length, locate=length >= 12)
 
 
 @pytest.mark.parametrize("k,edit", [(1, False), (2, True)])
