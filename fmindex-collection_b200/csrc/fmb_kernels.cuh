@@ -371,7 +371,7 @@ __device__ __forceinline__ uint32_t chunk_byte(const uint4& v, uint32_t i) {
     return (w >> (8 * (i & 3))) & 0xFF;
 }
 
-template <bool COUNT, class OCC>
+template <class OCC>
 __global__ void __launch_bounds__(256) exact_search_kernel(const __grid_constant__ IndexView<OCC> ix, const uint8_t* __restrict__ qsym,
                                                            const uint64_t* __restrict__ qoff, uint32_t nq, uint32_t qidx_base,
                                                            HitRec* __restrict__ out_hits, uint32_t* __restrict__ out_len,
@@ -422,7 +422,7 @@ __global__ void __launch_bounds__(256) exact_search_kernel(const __grid_constant
         rows = len;
     }
     // [0] extensions, [1] occ lookups; [4] hits, [5] rows of all hits
-    if (COUNT) block_count2(counters, 0, ext, 1, lookups);
+    block_count2(counters, 0, ext, 1, lookups);
     block_count3(counters, 4, found, 4, 0, 5, rows);
 }
 
@@ -686,9 +686,9 @@ __global__ void __launch_bounds__(256) jump_widen_kernel(const uint2* __restrict
 // broadcast is needed.  Pairs containing the delimiter symbol 0 and the odd leading symbol take one-symbol steps on
 // the 32-byte table (all lanes of the group read the same sector = one request).
 // Results are identical to exact_search_kernel: the final (lb, len) of a pattern does not depend on the step width.
+// 8 blocks per SM: 32 registers, 2048 resident threads per SM.
 // ---------------------------------------------------------------------------------------------------------
-template <bool COUNT, int MINB>
-__global__ void __launch_bounds__(256, MINB) exact_search2_kernel(const __grid_constant__ IndexView<OccDna> ix, const __grid_constant__ Occ2View o2,
+__global__ void __launch_bounds__(256, 8) exact_search2_kernel(const __grid_constant__ IndexView<OccDna> ix, const __grid_constant__ Occ2View o2,
                                                                   const uint8_t* __restrict__ qsym, const uint32_t* __restrict__ qpk,
                                                                   const uint8_t* __restrict__ qflags, const uint64_t* __restrict__ qoff, uint32_t nq,
                                                                   uint32_t qidx_base, HitRec* __restrict__ out_hits, uint32_t* __restrict__ out_len,
@@ -817,7 +817,7 @@ __global__ void __launch_bounds__(256, MINB) exact_search2_kernel(const __grid_c
         }
     }
     // [2] = line requests issued by this kernel (physical work), counted once per group; [4] hits, [5] rows of all hits
-    block_count3(counters, 2, (COUNT && sub == 0) ? lines : 0, 4, found, 5, rows);
+    block_count3(counters, 2, sub == 0 ? lines : 0, 4, found, 5, rows);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -853,7 +853,7 @@ __global__ void hit_lengths_kernel(const HitRec* __restrict__ hits, uint64_t nh,
 // The marker word and the occ block of a row are independent loads and are issued together.
 // starts[] = exclusive prefix sum of the hit interval lengths; a thread finds its hit by binary search.
 // ---------------------------------------------------------------------------------------------------------
-template <bool COUNT, class OCC>
+template <class OCC>
 __global__ void __launch_bounds__(256) locate_kernel(const __grid_constant__ IndexView<OCC> ix, const HitRec* __restrict__ hits,
                                                      const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,
                                                      LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
@@ -888,7 +888,7 @@ __global__ void __launch_bounds__(256) locate_kernel(const __grid_constant__ Ind
         r.qidx = h.qidx; r.seq = sample.x; r.pos = sample.y + steps; r.e = h.e;
         out[t] = r;
     }
-    if (COUNT) block_count2(counters, 2, steps, 1, steps);
+    block_count2(counters, 2, steps, 1, steps);
 }
 
 // K4b: locate with the combined 64-byte locate blocks.  A pair of lanes owns one SA row: the even lane fetches the
@@ -905,7 +905,6 @@ __global__ void build_locblocks_kernel(const DnaBlock* __restrict__ occ, const u
     out[b * 4 + 3] = make_uint4(0, 0, 0, 0);
 }
 
-template <bool COUNT>
 __global__ void __launch_bounds__(256) locate_pair_kernel(const __grid_constant__ IndexView<OccDna> ix, const HitRec* __restrict__ hits,
                                                           const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,
                                                           LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
@@ -970,7 +969,7 @@ __global__ void __launch_bounds__(256) locate_pair_kernel(const __grid_constant_
             ++steps;
         }
     }
-    if (COUNT) block_count2(counters, 2, steps_total, 1, steps_total);
+    block_count2(counters, 2, steps_total, 1, steps_total);
 }
 
 // K4c: locate shortcut table.  locrow[row] = sample_index << step_bits | steps of the LF walk of `row` (built by walking every row
@@ -1049,7 +1048,7 @@ __global__ void __launch_bounds__(256) locrow_build_gen_kernel(const __grid_cons
     }
 }
 
-template <bool COUNT, class OCC>
+template <class OCC>
 __global__ void __launch_bounds__(256) locate_shortcut_kernel(const __grid_constant__ IndexView<OCC> ix, const HitRec* __restrict__ hits,
                                                               const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,
                                                               LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
@@ -1071,7 +1070,7 @@ __global__ void __launch_bounds__(256) locate_shortcut_kernel(const __grid_const
         out[t] = r;
     }
     // the LF steps the walk WOULD take: the algorithmic work of SURVEY.md §8d stays reported
-    if (COUNT) block_count2(counters, 2, steps, 1, steps);
+    block_count2(counters, 2, steps, 1, steps);
 }
 
 // index.locate(row) for arbitrary rows (fmindex/BiFMIndex.h:177-202): same LF walk as locate_kernel, row list input

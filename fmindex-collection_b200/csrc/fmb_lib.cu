@@ -1263,11 +1263,9 @@ int fmb_search_exact(const fmb_index* ix, const fmb_queries* q, fmb_results** ou
     cudaMemsetAsync(res->lens.p + nq, 0, sizeof(uint32_t), st);
     EventTimer tm(st);
     if (nq) {
-        static const bool minb8 = getenv("FMB_EXACT2_MINB1") == nullptr;      // 32 registers -> 2048 resident threads per SM
         const uint32_t base = (uint32_t)q->qidx_base;
-        if (two && minb8) exact_search2_kernel<true, 8><<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), ix->view_occ2(0), q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p);
-        else if (two) exact_search2_kernel<true, 1><<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), ix->view_occ2(0), q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p);
-        else FMB_DISPATCH(ix, v, exact_search_kernel<true><<<grid_for(nq, 256), 256, 0, st>>>(v, q->symbols.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p,
+        if (two) exact_search2_kernel<<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), ix->view_occ2(0), q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p);
+        else FMB_DISPATCH(ix, v, exact_search_kernel<<<grid_for(nq, 256), 256, 0, st>>>(v, q->symbols.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p,
                                                                                               ix->dna ? nullptr : ix->jump4[0].p));
         note_launches(1);
     }
@@ -1353,15 +1351,15 @@ int fmb_locate(const fmb_index* ix, const fmb_results* hits, fmb_results** out) 
     if (total) {
         cudaEventRecord(ev_m0, st);
         if (ix->locrow.p && ix->locate_mode != FMB_LOCATE_WALK) {
-            FMB_DISPATCH(ix, v, locate_shortcut_kernel<true><<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, res->locs.p, ctr.p));
+            FMB_DISPATCH(ix, v, locate_shortcut_kernel<<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, res->locs.p, ctr.p));
         } else if (ix->dna && ix->locblocks.p) {
             auto v = ix->view_dna();
             // persistent grid: every SM full of lane pairs (8 blocks x 256 threads), rows handed out with a grid stride
             const int sms = ix->sm_count;
             unsigned grid = (unsigned)std::min<uint64_t>(grid_for((uint64_t)total * 2, 256), (uint64_t)sms * 8);
-            locate_pair_kernel<true><<<grid, 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, res->locs.p, ctr.p);
+            locate_pair_kernel<<<grid, 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, res->locs.p, ctr.p);
         }
-        else FMB_DISPATCH(ix, v, locate_kernel<true><<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, res->locs.p, ctr.p));
+        else FMB_DISPATCH(ix, v, locate_kernel<<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, res->locs.p, ctr.p));
         cudaEventRecord(ev_m1, st);
         note_launches(1);
     }

@@ -117,6 +117,13 @@ __device__ __forceinline__ unsigned long long order_key_root(const SchemeParams&
     return key;
 }
 
+// slots of the counter block of a search call: the statistics (SchemeOut::counters points at CTR_EXTENSIONS) and the list counters
+enum : uint32_t {
+    CTR_EXTENSIONS = 0, CTR_OCC_LOOKUPS = 1, CTR_LINE_REQUESTS = 2, CTR_PEAK = 3,
+    CTR_HITS = 4, CTR_OVERFLOW = 5, CTR_ROOTS = 6, CTR_TEXT_A = 7, CTR_ROWS = 8, CTR_TEXT_B = 9,
+    CTR_SLOTS = 10
+};
+
 struct SchemeOut {
     HitRec* hits;
     unsigned long long* hit_count;     // total hits found (may exceed capacity)
@@ -125,7 +132,7 @@ struct SchemeOut {
     Item* overflow;
     unsigned long long* overflow_count;
     uint64_t overflow_capacity;
-    unsigned long long* counters;      // [0] extensions, [1] occ lookups, [3] peak items per warp
+    unsigned long long* counters;      // [CTR_EXTENSIONS], [CTR_OCC_LOOKUPS], [CTR_LINE_REQUESTS], [CTR_PEAK] peak items per warp
     unsigned long long* root_counter;
     uint32_t qidx_base;                // added to the reported qidx (chunked query batches)
     uint64_t root_base;                // first root (query x search pair) of this launch's slab
@@ -134,7 +141,7 @@ struct SchemeOut {
     unsigned long long* text_count;
     uint64_t text_capacity;
     // text kernel only: the text list of the NEXT pass -- its text-class hand-overs (a new direction run, a new window) go there
-    // directly instead of through the overflow list and a routing launch of the frontier kernel (null: everything to the overflow list)
+    // directly instead of through the overflow list and a routing launch of the frontier kernel
     Item* text_next;
     unsigned long long* text_next_count;
     // ordered mode: keys of the hits / the spilled items / the items fed in
@@ -399,7 +406,7 @@ __global__ void __launch_bounds__(256, FMB_SCHEME_MINB) scheme_search_kernel(con
                                                             const uint8_t* __restrict__ qsym, const uint64_t* __restrict__ qoff,
                                                             const __grid_constant__ JumpView jv, uint64_t n_roots,
                                                             const Item* __restrict__ in_items, uint64_t n_in,
-                                                            const __grid_constant__ SchemeOut out, uint32_t cap, uint32_t ff_min) {
+                                                            const __grid_constant__ SchemeOut out, uint32_t cap) {
     extern __shared__ uint4 smem_raw[];
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t warp = threadIdx.x >> 5;
@@ -426,8 +433,9 @@ __global__ void __launch_bounds__(256, FMB_SCHEME_MINB) scheme_search_kernel(con
     bool more_roots = true;
     const uint32_t np = sp.n_parts;
     const uint32_t first_symb = ix.first_symb;   // FirstSymb (fmindex/BiFMIndex.h:26): 1 for delimited indices, 0 for NoDelim
-    const bool sim_all = (ff_min >> 8) & 1;      // simulate error children at every error level, not only the last one
-    ff_min &= 0xFF;
+    // a warp keeps fast-forwarding while at least ff_min of its lanes have a single child; edit distance branches
+    // at almost every node, so it only pays there when most of the warp is inside error-free stretches
+    constexpr uint32_t ff_min = EDIT ? 16u : 8u;
 
     for (;;) {
         // ---- refill: pull roots while fewer than 32 items are pending -------------------------------------
@@ -862,7 +870,7 @@ __global__ void __launch_bounds__(256, FMB_SCHEME_MINB) scheme_search_kernel(con
                                 // accounted for -- their extensions are counted -- but never created.
                                 const unsigned long long err_children = cmask & ~(CH_MATCH | CH_JUMP);
                                 const uint2* sim_table = OCC::kSymbolLoad ? jv.jump4[R] : jv.jump[R];
-                                if (EDIT && err_children && sim_table != nullptr && single_sym >= first_symb && (sim_all || st.e + 1 == up)) {
+                                if (EDIT && err_children && sim_table != nullptr && single_sym >= first_symb) {
                                     const uint2 je = __ldg(sim_table + (OCC::kSymbolLoad ? (size_t)lo : ((size_t)lo << jv.jshift[R])));
                                     n_phys += 1;
                                     if (je.x != kJumpInvalid) {
@@ -1035,10 +1043,10 @@ __global__ void __launch_bounds__(256, FMB_SCHEME_MINB) scheme_search_kernel(con
         n_phys += __shfl_xor_sync(0xFFFFFFFFu, n_phys, o);
     }
     if (lane == 0) {
-        atomicAdd(out.counters + 0, (unsigned long long)n_ext);
-        atomicAdd(out.counters + 1, (unsigned long long)n_look);
-        atomicAdd(out.counters + 2, (unsigned long long)n_phys);
-        atomicMax(out.counters + 3, (unsigned long long)peak);
+        atomicAdd(out.counters + CTR_EXTENSIONS, (unsigned long long)n_ext);
+        atomicAdd(out.counters + CTR_OCC_LOOKUPS, (unsigned long long)n_look);
+        atomicAdd(out.counters + CTR_LINE_REQUESTS, (unsigned long long)n_phys);
+        atomicMax(out.counters + CTR_PEAK, (unsigned long long)peak);
     }
 }
 

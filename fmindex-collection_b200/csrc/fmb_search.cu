@@ -133,8 +133,8 @@ int scheme_stack_cap(int dev, size_t item_bytes, uint32_t* cap) {
 }
 
 template <class OCC, bool EDIT, bool ORDERED, bool PSEUDO>
-int launch_scheme_t(const fmb_index* ix, const IndexView<OCC>& view, const SchemeParams& sp, const fmb_queries* q, uint64_t n_roots, const Item* in_items,
-                    uint64_t n_in, const SchemeOut& out, cudaStream_t st) {
+int launch_frontier_t(const fmb_index* ix, const IndexView<OCC>& view, const SchemeParams& sp, const fmb_queries* q, uint64_t n_roots, const Item* in_items,
+                      uint64_t n_in, const SchemeOut& out, cudaStream_t st) {
     constexpr size_t kItemBytes = sizeof(Item) + (ORDERED ? sizeof(unsigned long long) : 0);
     auto kern = scheme_search_kernel<OCC, EDIT, ORDERED, PSEUDO>;
     // launch geometry, computed once per kernel instantiation (several host threads drive one index in the pipelined path)
@@ -166,22 +166,25 @@ int launch_scheme_t(const fmb_index* ix, const IndexView<OCC>& view, const Schem
     uint64_t want_blocks = (work + 255) / 256;
     unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms * blocks_per_sm, want_blocks));
     const JumpView jv = make_jump_view(ix, q);
-    // a warp keeps fast-forwarding while at least ff_min of its lanes have a single child; edit distance branches
-    // at almost every node, so it only pays there when most of the warp is inside error-free stretches
-    static const char* ff_env = getenv("FMB_SCHEME_FFMIN");
-    static const char* sim_env = getenv("FMB_SCHEME_SIMALL");
-    const uint32_t sim_all = sim_env ? (uint32_t)atoi(sim_env) : 1u;
-    const uint32_t ff_min = (ff_env ? (uint32_t)atoi(ff_env) : (EDIT ? 16u : 8u)) | (sim_all << 8);
-    kern<<<grid, 256, smem, st>>>(view, sp, q->symbols.p, q->offsets.p, jv, n_roots, in_items, n_in, out, stack_cap, ff_min);
+    kern<<<grid, 256, smem, st>>>(view, sp, q->symbols.p, q->offsets.p, jv, n_roots, in_items, n_in, out, stack_cap);
     FMB_CUDA(cudaGetLastError());
     note_launches(1);
     return FMB_OK;
 }
-template <bool EDIT, bool ORDERED, bool PSEUDO = false>
-int launch_scheme(const fmb_index* ix, const SchemeParams& sp, const fmb_queries* q, uint64_t n_roots, const Item* in_items,
-                  uint64_t n_in, const SchemeOut& out, cudaStream_t st) {
-    if (ix->dna) return launch_scheme_t<OccDna, EDIT, ORDERED, PSEUDO>(ix, ix->view_dna(), sp, q, n_roots, in_items, n_in, out, st);
-    return launch_scheme_t<OccGen, EDIT, ORDERED, PSEUDO>(ix, ix->view_gen(), sp, q, n_roots, in_items, n_in, out, st);
+template <class OCC>
+int launch_frontier_v(const fmb_index* ix, const IndexView<OCC>& v, const SchemeParams& sp, const fmb_queries* q, bool ordered, bool pseudo,
+                      uint64_t n_roots, const Item* in_items, uint64_t n_in, const SchemeOut& out, cudaStream_t st) {
+    if (ordered) return sp.edit ? launch_frontier_t<OCC, true, true, false>(ix, v, sp, q, n_roots, in_items, n_in, out, st)
+                                : launch_frontier_t<OCC, false, true, false>(ix, v, sp, q, n_roots, in_items, n_in, out, st);
+    if (!sp.edit) return launch_frontier_t<OCC, false, false, false>(ix, v, sp, q, n_roots, in_items, n_in, out, st);
+    return pseudo ? launch_frontier_t<OCC, true, false, true>(ix, v, sp, q, n_roots, in_items, n_in, out, st)
+                  : launch_frontier_t<OCC, true, false, false>(ix, v, sp, q, n_roots, in_items, n_in, out, st);
+}
+// ordered: the hit-limited instantiation (discovery-order keys); pseudo: edit distance without the redundancy filter
+int launch_frontier(const fmb_index* ix, const SchemeParams& sp, const fmb_queries* q, bool ordered, bool pseudo, uint64_t n_roots,
+                    const Item* in_items, uint64_t n_in, const SchemeOut& out, cudaStream_t st) {
+    if (ix->dna) return launch_frontier_v(ix, ix->view_dna(), sp, q, ordered, pseudo, n_roots, in_items, n_in, out, st);
+    return launch_frontier_v(ix, ix->view_gen(), sp, q, ordered, pseudo, n_roots, in_items, n_in, out, st);
 }
 
 // ---- text list by class: the lanes of a warp of the text kernel take consecutive items; items of one (search, part, errors) class
@@ -275,27 +278,143 @@ int order_and_limit(fmb_results* res, DevBuf<unsigned long long>& keys, uint64_t
     return FMB_OK;
 }
 
+// ordered mode: the layout of the discovery-order key (order_key_edge), one slot per error of the search that allows the most
+int key_layout(SchemeParams& sp, uint32_t sigma) {
+    uint32_t K = 0, total = 0;
+    for (uint32_t s = 0; s < sp.n_searches; ++s)
+        for (uint32_t p = 0; p < sp.n_parts; ++p) K = std::max<uint32_t>(K, sp.u[s][p]);
+    for (uint32_t p = 0; p < sp.n_parts; ++p) total += sp.partition[p];
+    sp.key_slots = K;
+    sp.key_maxd = total + 2 * K + 2;
+    sp.key_ords = 2 * sigma + 2;
+    const uint64_t range = (uint64_t)sp.key_maxd + 1 + (uint64_t)sp.key_maxd * sp.key_ords;
+    sp.key_bits = 1;
+    while ((1ull << sp.key_bits) < range) ++sp.key_bits;
+    if (K * sp.key_bits > 56) {
+        set_error("hit-limited search: %u errors on %u-symbol queries need %u key bits (56 available)", K, total, K * sp.key_bits);
+        return FMB_EUNSUPPORTED;
+    }
+    return FMB_OK;
+}
+
+// The item lists of one search call, `cap` items each.  A pass of the frontier kernel reads one overflow list and fills the other.  In
+// text mode it also fills the current text list, which the text kernel of the same pass reads while it appends its text-class
+// hand-overs to the other text list: the two swap roles after every text pass.  Edit distance sorts a text list by class first.
+struct SchemeLists {
+    uint64_t cap = 0;
+    DevBuf<Item> ovf[2], text[2], text_sorted;
+    DevBuf<unsigned long long> ovf_keys[2];           // ordered mode: the keys of the overflow items
+    DevBuf<uint32_t> tkeys[2], tidx[2];
+    DevBuf<uint8_t> sort_tmp;
+    size_t sort_bytes = 0;
+
+    int alloc(uint64_t items, bool text_mode, bool sort, bool ordered, cudaStream_t st) {
+        cap = items;
+        for (int b = 0; b < 2; ++b) {
+            FMB_TRY(ovf[b].alloc(cap));
+            if (text_mode) FMB_TRY(text[b].alloc(cap));
+            if (ordered) FMB_TRY(ovf_keys[b].alloc(cap));
+        }
+        if (sort) {
+            FMB_TRY(text_sorted.alloc(cap));
+            for (int b = 0; b < 2; ++b) { FMB_TRY(tkeys[b].alloc(cap)); FMB_TRY(tidx[b].alloc(cap)); }
+            FMB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, tkeys[0].p, tkeys[1].p, tidx[0].p, tidx[1].p, (int64_t)cap, 0, 10, st));
+            FMB_TRY(sort_tmp.alloc(sort_bytes));
+        }
+        return FMB_OK;
+    }
+};
+
+// the kernels count what does not fit a list and drop it
+int lists_fit(const unsigned long long* h_ctr, uint64_t cap) {
+    if (h_ctr[CTR_OVERFLOW] <= cap && h_ctr[CTR_TEXT_A] <= cap && h_ctr[CTR_TEXT_B] <= cap) return FMB_OK;
+    set_error("scheme search: frontier lists exceeded %llu items; split the query batch", (unsigned long long)cap);
+    return FMB_EOVERFLOW;
+}
+
+// The roots [root_base, root_base + roots), pass by pass: the frontier kernel takes the roots (first pass) and the overflow list of the
+// previous pass; in text mode the text kernel then decides the single-row items the frontier kernel handed over.  The slab ends when
+// every list is empty.  h_ctr: the counter block as the last kernel left it.
+int run_slab(const fmb_index* ix, const SchemeParams& sp, const fmb_queries* q, bool ordered, bool pseudo, SchemeLists& L, SchemeOut& so,
+             unsigned long long* ctr, unsigned long long* h_ctr, uint64_t root_base, uint64_t roots, cudaStream_t st) {
+    static const bool trace = getenv("FMB_TRACE_SCHEME") != nullptr;
+    auto read_back = [&]() -> int {
+        FMB_CUDA(cudaMemcpyAsync(h_ctr, ctr, CTR_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        FMB_CUDA(cudaStreamSynchronize(st));
+        return FMB_OK;
+    };
+    if (root_base) {                                  // slab level: the previous slab left its lists empty
+        FMB_CUDA(cudaMemsetAsync(ctr + CTR_OVERFLOW, 0, 3 * sizeof(unsigned long long), st));   // overflow, roots, text list A
+        FMB_CUDA(cudaMemsetAsync(ctr + CTR_TEXT_B, 0, sizeof(unsigned long long), st));
+    }
+    so.root_base = root_base;
+    so.text = L.text[0].p;                            // the text list the frontier kernel fills and the text kernel reads
+    so.text_count = ctr + CTR_TEXT_A;
+    so.text_next = L.text[1].p;                       // the one the text kernel appends its hand-overs to
+    so.text_next_count = ctr + CTR_TEXT_B;
+    uint64_t n_in = 0;
+    for (int pass = 0;; ++pass) {
+        const int cur = pass & 1;                     // the overflow list this pass fills; it reads the other one
+        so.overflow = L.ovf[cur].p;
+        so.overflow_keys = L.ovf_keys[cur].p;
+        so.in_keys = pass ? L.ovf_keys[cur ^ 1].p : nullptr;
+        EventPair tr;
+        if (trace) cudaEventRecord(tr.a, st);
+        if (roots + n_in > 0) FMB_TRY(launch_frontier(ix, sp, q, ordered, pseudo, roots, pass ? L.ovf[cur ^ 1].p : nullptr, n_in, so, st));
+        if (trace) cudaEventRecord(tr.b, st);
+        FMB_TRY(read_back());
+        const size_t ti = so.text_count - ctr, tn = so.text_next_count - ctr;     // counter slots of the two text lists
+        if (trace) {
+            float ms = 0;
+            cudaEventElapsedTime(&ms, tr.a, tr.b);
+            fprintf(stderr, "[fmb scheme] slab %llu pass %d frontier kernel: %.3f ms, %llu roots + %llu items in -> %llu text, %llu back, %llu hits so far\n",
+                    (unsigned long long)root_base, pass, ms, (unsigned long long)roots, (unsigned long long)n_in, h_ctr[ti], h_ctr[CTR_OVERFLOW], h_ctr[CTR_HITS]);
+        }
+        FMB_TRY(lists_fit(h_ctr, L.cap));
+        if (h_ctr[ti]) {
+            // the single-row items of this pass are decided on the text; what survives joins the next text list (a new direction
+            // run, a new window) or the overflow list (what must be expanded on the index)
+            const unsigned long long n_text = h_ctr[ti], back0 = h_ctr[CTR_OVERFLOW];
+            if (trace) cudaEventRecord(tr.a, st);
+            const Item* text_in = so.text;
+            if (L.text_sorted.p && n_text > 65536) {
+                const unsigned grid = (unsigned)((n_text + 255) / 256);
+                text_class_keys_kernel<<<grid, 256, 0, st>>>(text_in, n_text, L.tkeys[0].p, L.tidx[0].p);
+                FMB_CUDA(cub::DeviceRadixSort::SortPairs(L.sort_tmp.p, L.sort_bytes, L.tkeys[0].p, L.tkeys[1].p, L.tidx[0].p, L.tidx[1].p, (int64_t)n_text, 0, 10, st));
+                gather_items_kernel<<<grid, 256, 0, st>>>(text_in, L.tidx[1].p, n_text, L.text_sorted.p);
+                FMB_CUDA(cudaGetLastError());
+                note_launches(3);
+                text_in = L.text_sorted.p;
+            }
+            FMB_TRY(launch_text(ix, sp, q, text_in, n_text, so, pseudo, st));
+            if (trace) cudaEventRecord(tr.b, st);
+            FMB_CUDA(cudaMemsetAsync(ctr + ti, 0, sizeof(unsigned long long), st));        // pass level: the text list just read
+            FMB_TRY(read_back());
+            if (trace) {
+                float ms = 0;
+                cudaEventElapsedTime(&ms, tr.a, tr.b);
+                fprintf(stderr, "[fmb scheme] slab %llu pass %d text kernel: %.3f ms, %llu items -> %llu to the next text list, %llu back\n",
+                        (unsigned long long)root_base, pass, ms, n_text, h_ctr[tn], h_ctr[CTR_OVERFLOW] - back0);
+            }
+            std::swap(so.text, so.text_next);         // the frontier kernel of the next pass appends to what the text kernel began
+            std::swap(so.text_count, so.text_next_count);
+            FMB_TRY(lists_fit(h_ctr, L.cap));
+        }
+        if (h_ctr[CTR_OVERFLOW] == 0 && h_ctr[CTR_TEXT_A] == 0 && h_ctr[CTR_TEXT_B] == 0) return FMB_OK;
+        // feed the spilled / returned items to the next pass
+        n_in = h_ctr[CTR_OVERFLOW];
+        roots = 0;
+        FMB_CUDA(cudaMemsetAsync(ctr + CTR_OVERFLOW, 0, 2 * sizeof(unsigned long long), st));     // pass level: overflow, roots
+        if (pass > 100000) { set_error("scheme search did not terminate"); return FMB_ECUDA; }
+    }
+}
+
 // n_limit = UINT64_MAX: every hit, in no particular order; else the reference's search_n semantics (SearchNg26.h:408-423)
 // pseudo: edit distance without the redundancy filter of search_ng26 (search_pseudo::search<true>, search/SearchPseudo.h:100-165)
 int run_scheme(const fmb_index* ix, const fmb_queries* q, const SchemeParams& sp_in, fmb_results** out_res, uint64_t n_limit = UINT64_MAX, bool pseudo = false) {
     SchemeParams sp = sp_in;
     const bool ordered = n_limit != UINT64_MAX;
-    if (ordered) {
-        uint32_t K = 0, total = 0;
-        for (uint32_t s = 0; s < sp.n_searches; ++s)
-            for (uint32_t p = 0; p < sp.n_parts; ++p) K = std::max<uint32_t>(K, sp.u[s][p]);
-        for (uint32_t p = 0; p < sp.n_parts; ++p) total += sp.partition[p];
-        sp.key_slots = K;
-        sp.key_maxd = total + 2 * K + 2;
-        sp.key_ords = 2 * ix->sigma + 2;
-        const uint64_t range = (uint64_t)sp.key_maxd + 1 + (uint64_t)sp.key_maxd * sp.key_ords;
-        sp.key_bits = 1;
-        while ((1ull << sp.key_bits) < range) ++sp.key_bits;
-        if (K * sp.key_bits > 56) {
-            set_error("hit-limited search: %u errors on %u-symbol queries need %u key bits (56 available)", K, total, K * sp.key_bits);
-            return FMB_EUNSUPPORTED;
-        }
-    }
+    if (ordered) FMB_TRY(key_layout(sp, ix->sigma));
     FMB_TRY(set_device(ix->device));
     cudaStream_t st = active_stream(ix);
     auto res = new fmb_results();
@@ -305,7 +424,6 @@ int run_scheme(const fmb_index* ix, const fmb_queries* q, const SchemeParams& sp
 
     const uint64_t nq = q->nq;
     const uint64_t n_roots = nq * sp.n_searches;
-    uint64_t hit_cap = std::max<uint64_t>(1u << 20, nq * 8);
     // Text mode: the frontier kernel hands single-row items to the text kernel through a global list and gets
     // the survivors back through the overflow list, so the lists scale with the number of roots in flight: the roots are processed
     // in slabs.  Otherwise: all roots at once, the overflow list only takes what the warp stacks cannot hold.
@@ -315,58 +433,37 @@ int run_scheme(const fmb_index* ix, const fmb_queries* q, const SchemeParams& sp
     static const uint64_t env_slab = getenv("FMB_SCHEME_SLAB") ? strtoull(getenv("FMB_SCHEME_SLAB"), nullptr, 10) : 0;
     // (without text mode the roots go in slabs as well: what a slab spills -- warp stacks that ran full -- stays bounded)
     const uint64_t slab = std::min<uint64_t>(std::max<uint64_t>(n_roots, 1), env_slab ? env_slab : (text_mode ? (uint64_t(16) << 20) : (uint64_t(4) << 20)));      // at 30 M roots: 8 M 63.5 ms, 16 M 61.5, 32 M 60.1 (k = 2 edit)
-    const uint64_t ovf_cap = std::max<uint64_t>(1u << 20, slab * 2 + (1u << 18));       // items of 32 bytes
-    DevBuf<Item> ovf[2], text_list, text_sorted;
-    DevBuf<uint32_t> tkeys[2], tidx[2];
-    DevBuf<uint8_t> tsort_tmp;
-    size_t tsort_bytes = 0;
-    static const bool sort_text = getenv("FMB_NO_TEXT_SORT") == nullptr;
-    DevBuf<unsigned long long> ovf_keys[2], hit_keys;
-    DevBuf<unsigned long long> ctr;          // [0..3] counters, [4] hit_count, [5] overflow_count, [6] root_counter, [7] / [9] text_count of the two text lists, [8] row_count
-    FMB_TRY(ovf[0].alloc(ovf_cap));
-    FMB_TRY(ovf[1].alloc(ovf_cap));
-    if (text_mode) FMB_TRY(text_list.alloc(ovf_cap));
-    // the text kernel appends its text-class hand-overs to the list of the next pass (two lists, swapped after every text launch)
-    DevBuf<Item> text_list2;
-    static const bool direct_text = getenv("FMB_NO_DIRECT_TEXT") == nullptr;
-    if (text_mode && direct_text) FMB_TRY(text_list2.alloc(ovf_cap));
-    if (text_mode && sort_text && (sp.edit || getenv("FMB_TEXT_SORT_HAMMING"))) {
-        // (edit distance only: the Hamming walk has one shape whatever the class)
-        FMB_TRY(text_sorted.alloc(ovf_cap));
-        for (int b = 0; b < 2; ++b) { FMB_TRY(tkeys[b].alloc(ovf_cap)); FMB_TRY(tidx[b].alloc(ovf_cap)); }
-        FMB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tsort_bytes, tkeys[0].p, tkeys[1].p, tidx[0].p, tidx[1].p, (int64_t)ovf_cap, 0, 10, active_stream(ix)));
-        FMB_TRY(tsort_tmp.alloc(tsort_bytes));
-    }
     // small hit limits (n <= 8 rows per query): the kernel keeps the n smallest keys found per query and drops what cannot beat the n-th
-    DevBuf<unsigned long long> best_keys;
-    const bool prune_first = ordered && n_limit >= 1 && n_limit <= kMaxPruneN && getenv("FMB_NO_FIRST_HIT_PRUNING") == nullptr;
+    const bool prune_first = ordered && n_limit >= 1 && n_limit <= kMaxPruneN;
     const uint64_t n_best = std::max<uint64_t>(nq, 1) * (prune_first ? n_limit : 1);
+
+    SchemeLists lists;
+    // (the class sort is for edit distance only: the Hamming walk has one shape whatever the class)
+    FMB_TRY(lists.alloc(std::max<uint64_t>(1u << 20, slab * 2 + (1u << 18)), text_mode, text_mode && sp.edit, ordered, st));
+    DevBuf<unsigned long long> best_keys, hit_keys, ctr;
     if (prune_first) FMB_TRY(best_keys.alloc(n_best));
-    if (ordered) {
-        FMB_TRY(ovf_keys[0].alloc(ovf_cap));
-        FMB_TRY(ovf_keys[1].alloc(ovf_cap));
-    }
-    FMB_TRY(ctr.alloc(16));
+    FMB_TRY(ctr.alloc(CTR_SLOTS));
     EventPair evs;
-    const cudaEvent_t ev0 = evs.a, ev1 = evs.b;
     double total_ms = 0;
-    unsigned long long h_ctr[16];
+    unsigned long long h_ctr[CTR_SLOTS];
+    uint64_t hit_cap = std::max<uint64_t>(1u << 20, nq * 8);
     // (a second attempt runs with the exact size the first one counted; with work-bounding hit limits the count depends on the timing of
     // the pruning, so those retries reserve twice what was counted and may repeat)
     for (int attempt = 0; attempt < (prune_first ? 5 : 2); ++attempt) {
         FMB_TRY(res->hits.alloc(hit_cap));
         if (ordered) FMB_TRY(hit_keys.alloc(hit_cap));
-        FMB_CUDA(cudaMemsetAsync(ctr.p, 0, 16 * sizeof(unsigned long long), st));
+        FMB_CUDA(cudaMemsetAsync(ctr.p, 0, sizeof h_ctr, st));                                   // attempt level: every counter
         SchemeOut so{};
         so.hit_keys = hit_keys.p;
         so.hits = res->hits.p;
-        so.hit_count = ctr.p + 4;
-        so.row_count = ctr.p + 8;
+        so.hit_count = ctr.p + CTR_HITS;
+        so.row_count = ctr.p + CTR_ROWS;
         so.hit_capacity = hit_cap;
-        so.overflow_count = ctr.p + 5;
-        so.overflow_capacity = ovf_cap;
-        so.counters = ctr.p;
-        so.root_counter = ctr.p + 6;
+        so.overflow_count = ctr.p + CTR_OVERFLOW;
+        so.overflow_capacity = lists.cap;
+        so.text_capacity = lists.cap;
+        so.counters = ctr.p + CTR_EXTENSIONS;
+        so.root_counter = ctr.p + CTR_ROOTS;
         so.qidx_base = (uint32_t)q->qidx_base;
         if (prune_first) {
             FMB_CUDA(cudaMemsetAsync(best_keys.p, 0xFF, n_best * sizeof(unsigned long long), st));
@@ -374,123 +471,31 @@ int run_scheme(const fmb_index* ix, const fmb_queries* q, const SchemeParams& sp
             so.n_queries = nq;
             so.prune_n = (uint32_t)n_limit;
         }
-        Item* tlist[2] = {text_list.p, text_list2.p};
-        unsigned long long* tcount[2] = {ctr.p + 7, ctr.p + 9};
-        int tcur = 0;                               // the list the frontier kernel fills and the text kernel reads
-        if (text_mode) {
-            so.text = tlist[0];
-            so.text_count = tcount[0];
-            so.text_capacity = ovf_cap;
-            if (text_list2.p) { so.text_next = tlist[1]; so.text_next_count = tcount[1]; }
-        }
-        cudaEventRecord(ev0, st);
+        cudaEventRecord(evs.a, st);
         for (uint64_t root_base = 0; root_base < std::max<uint64_t>(n_roots, 1); root_base += slab) {
-            uint64_t roots = n_roots ? std::min<uint64_t>(slab, n_roots - root_base) : 0, n_in = 0;
-            int cur = 0;
-            so.root_base = root_base;
-            if (root_base) {
-                FMB_CUDA(cudaMemsetAsync(ctr.p + 5, 0, 3 * sizeof(unsigned long long), st));   // overflow_count, root_counter, text_count
-                FMB_CUDA(cudaMemsetAsync(ctr.p + 9, 0, sizeof(unsigned long long), st));
-            }
-            for (int pass = 0;; ++pass) {
-                so.overflow = ovf[cur].p;
-                so.overflow_keys = ovf_keys[cur].p;
-                so.in_keys = pass ? ovf_keys[cur ^ 1].p : nullptr;
-                const Item* in_items = pass ? ovf[cur ^ 1].p : nullptr;
-                static const bool trace = getenv("FMB_TRACE_SCHEME") != nullptr;
-                EventPair tr;
-                if (trace) cudaEventRecord(tr.a, st);
-                if (roots + n_in > 0) {
-                    int rc = ordered ? (sp.edit ? launch_scheme<true, true>(ix, sp, q, roots, in_items, n_in, so, st)
-                                                : launch_scheme<false, true>(ix, sp, q, roots, in_items, n_in, so, st))
-                             : (pseudo && sp.edit) ? launch_scheme<true, false, true>(ix, sp, q, roots, in_items, n_in, so, st)
-                                     : (sp.edit ? launch_scheme<true, false>(ix, sp, q, roots, in_items, n_in, so, st)
-                                                : launch_scheme<false, false>(ix, sp, q, roots, in_items, n_in, so, st));
-                    if (rc) return rc;
-                }
-                if (trace) cudaEventRecord(tr.b, st);
-                FMB_CUDA(cudaMemcpyAsync(h_ctr, ctr.p, sizeof h_ctr, cudaMemcpyDeviceToHost, st));
-                FMB_CUDA(cudaStreamSynchronize(st));
-                if (trace) {
-                    float ms = 0;
-                    cudaEventElapsedTime(&ms, tr.a, tr.b);
-                    fprintf(stderr, "[fmb scheme] slab %llu pass %d frontier kernel: %.3f ms, %llu roots + %llu items in -> %llu text, %llu back, %llu hits so far\n",
-                            (unsigned long long)root_base, pass, ms, (unsigned long long)roots, (unsigned long long)n_in, h_ctr[tcur ? 9 : 7], h_ctr[5], h_ctr[4]);
-                }
-                const int ti = tcur ? 9 : 7, tn = tcur ? 7 : 9;      // counters of the current / the next text list
-                if (h_ctr[5] > ovf_cap || h_ctr[ti] > ovf_cap) {
-                    set_error("scheme search: frontier lists exceeded %llu items; split the query batch", (unsigned long long)ovf_cap);
-                    return FMB_EOVERFLOW;
-                }
-                unsigned long long n_text_next = 0;
-                if (h_ctr[ti]) {
-                    // the single-row items of this pass are decided on the text; what survives joins the next text list (a new direction
-                    // run, a new window) or the overflow list (what must be expanded on the index)
-                    const unsigned long long n_text = h_ctr[ti], back0 = h_ctr[5];
-                    if (trace) cudaEventRecord(tr.a, st);
-                    const Item* text_in = tlist[tcur];
-                    if (text_sorted.p && n_text > 65536) {
-                        const unsigned grid = (unsigned)((n_text + 255) / 256);
-                        text_class_keys_kernel<<<grid, 256, 0, st>>>(tlist[tcur], n_text, tkeys[0].p, tidx[0].p);
-                        FMB_CUDA(cub::DeviceRadixSort::SortPairs(tsort_tmp.p, tsort_bytes, tkeys[0].p, tkeys[1].p, tidx[0].p, tidx[1].p, (int64_t)n_text, 0, 10, st));
-                        gather_items_kernel<<<grid, 256, 0, st>>>(tlist[tcur], tidx[1].p, n_text, text_sorted.p);
-                        FMB_CUDA(cudaGetLastError());
-                        note_launches(3);
-                        text_in = text_sorted.p;
-                    }
-                    FMB_TRY(launch_text(ix, sp, q, text_in, n_text, so, pseudo, st));
-                    if (trace) cudaEventRecord(tr.b, st);
-                    FMB_CUDA(cudaMemsetAsync(ctr.p + ti, 0, sizeof(unsigned long long), st));
-                    FMB_CUDA(cudaMemcpyAsync(h_ctr, ctr.p, sizeof h_ctr, cudaMemcpyDeviceToHost, st));
-                    FMB_CUDA(cudaStreamSynchronize(st));
-                    h_ctr[ti] = 0;
-                    n_text_next = text_list2.p ? h_ctr[tn] : 0;
-                    if (trace) {
-                        float ms = 0;
-                        cudaEventElapsedTime(&ms, tr.a, tr.b);
-                        fprintf(stderr, "[fmb scheme] slab %llu pass %d text kernel: %.3f ms, %llu items -> %llu to the next text list, %llu back\n",
-                                (unsigned long long)root_base, pass, ms, n_text, n_text_next, h_ctr[5] - back0);
-                    }
-                    if (text_list2.p) {                     // the lists swap roles: the frontier kernel of the next pass appends to what the text kernel began
-                        tcur ^= 1;
-                        so.text = tlist[tcur]; so.text_count = tcount[tcur];
-                        so.text_next = tlist[tcur ^ 1]; so.text_next_count = tcount[tcur ^ 1];
-                    }
-                    if (h_ctr[5] > ovf_cap || n_text_next > ovf_cap) {
-                        set_error("scheme search: frontier lists exceeded %llu items; split the query batch", (unsigned long long)ovf_cap);
-                        return FMB_EOVERFLOW;
-                    }
-                }
-                if (h_ctr[5] == 0 && n_text_next == 0) break;
-                // feed the spilled / returned items to the next pass
-                n_in = h_ctr[5];
-                roots = 0;
-                cur ^= 1;
-                FMB_CUDA(cudaMemsetAsync(ctr.p + 5, 0, 2 * sizeof(unsigned long long), st));   // overflow_count, root_counter
-                if (!text_list2.p) FMB_CUDA(cudaMemsetAsync(ctr.p + 7, 0, sizeof(unsigned long long), st));
-                if (pass > 100000) { set_error("scheme search did not terminate"); return FMB_ECUDA; }
-            }
+            const uint64_t roots = n_roots ? std::min<uint64_t>(slab, n_roots - root_base) : 0;
+            FMB_TRY(run_slab(ix, sp, q, ordered, pseudo, lists, so, ctr.p, h_ctr, root_base, roots, st));
         }
-        cudaEventRecord(ev1, st);
-        cudaEventSynchronize(ev1);
+        cudaEventRecord(evs.b, st);
+        cudaEventSynchronize(evs.b);
         float ms = 0;
-        cudaEventElapsedTime(&ms, ev0, ev1);
+        cudaEventElapsedTime(&ms, evs.a, evs.b);
         total_ms += ms;
-        if (h_ctr[4] <= hit_cap) break;
-        hit_cap = prune_first ? 2 * h_ctr[4] : h_ctr[4];
+        if (h_ctr[CTR_HITS] <= hit_cap) break;
+        hit_cap = prune_first ? 2 * h_ctr[CTR_HITS] : h_ctr[CTR_HITS];
     }
-    if (h_ctr[4] > hit_cap) {
+    if (h_ctr[CTR_HITS] > hit_cap) {
         // (the retries ran with the size counted before: only a hit count that keeps growing between attempts could get here)
-        set_error("scheme search: %llu hits do not fit the %llu reserved", h_ctr[4], (unsigned long long)hit_cap);
+        set_error("scheme search: %llu hits do not fit the %llu reserved", h_ctr[CTR_HITS], (unsigned long long)hit_cap);
         return FMB_EOVERFLOW;
     }
-    res->count = h_ctr[4];
-    res->slots = h_ctr[4];
-    res->total_rows = ordered ? UINT64_MAX : h_ctr[8];      // the hit limit clips intervals afterwards: locate counts again
-    res->stats.extensions = h_ctr[0];
-    res->stats.occ_lookups = h_ctr[1];
-    res->stats.frontier_peak = h_ctr[3];
-    res->stats.line_requests = h_ctr[2];
+    res->count = h_ctr[CTR_HITS];
+    res->slots = h_ctr[CTR_HITS];
+    res->total_rows = ordered ? UINT64_MAX : h_ctr[CTR_ROWS];      // the hit limit clips intervals afterwards: locate counts again
+    res->stats.extensions = h_ctr[CTR_EXTENSIONS];
+    res->stats.occ_lookups = h_ctr[CTR_OCC_LOOKUPS];
+    res->stats.frontier_peak = h_ctr[CTR_PEAK];
+    res->stats.line_requests = h_ctr[CTR_LINE_REQUESTS];
     res->stats.kernel_ms = total_ms;
     res->stats.main_kernel_ms = total_ms;
     if (ordered) FMB_TRY(order_and_limit(res, hit_keys, n_limit, st));

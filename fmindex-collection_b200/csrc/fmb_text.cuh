@@ -30,21 +30,9 @@ constexpr int kTextWords = 9;        // window words per lane: 144 symbols (2-bi
 constexpr int kTextQWords = 10;      // query words per lane, walking order: 160 / 40 symbols
 constexpr int kTextStage = 64;       // staged items (and hits) per warp before they are flushed to the global lists (flushed at 32)
 constexpr int kTextStack = 16;       // private depth-first stack (packed nodes)
-#ifndef FMB_TEXT_BULK2
-#define FMB_TEXT_BULK2 1
-#endif
-constexpr bool kBulk2 = FMB_TEXT_BULK2 != 0;
-#ifndef FMB_TEXT_PREFETCH
-#define FMB_TEXT_PREFETCH 0        // measured: fetching one window word ahead in lockstep costs requests and buys nothing (76.6 vs 79.0 ms, k = 2 edit)
-#endif
-constexpr bool kPrefetch = FMB_TEXT_PREFETCH != 0;
 #ifndef FMB_TEXT_MINB
 #define FMB_TEXT_MINB 4
 #endif
-#ifndef FMB_TEXT_REPORTS
-#define FMB_TEXT_REPORTS 1         // leaves are reported by the text kernel instead of going back to the frontier kernel as items
-#endif
-constexpr bool kTextReports = FMB_TEXT_REPORTS != 0;
 
 struct TNode {             // one pending node, "ready to expand" (the position advance already applied)
     uint32_t m;            // text symbols consumed since the item started: the node looks at window symbol m
@@ -309,10 +297,8 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
         s.kind = kind;
         req[nreq++] = tnode_pack(s);
     };
-    uint32_t reach = 0;            // the farthest window position a node of this lane's item has got to
     auto push = [&](TNode s) {
         s.kind = TN_EXPAND;
-        reach = s.m > reach ? s.m : reach;
         if (top < kTextStack) stk[top++] = tnode_pack(s);
         else request(s, TN_CONT);
     };
@@ -367,7 +353,7 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
                     const bool is_hit = i < n && it.meta == kHitMark;
                     // text class again (every hand-over is a single row of an unflagged query and not a leaf): not flagged `notext`, and
                     // not an error-free stretch of the generic layout (those stay in the frontier kernel, text_class())
-                    const bool is_text = i < n && !is_hit && out.text_next != nullptr && !(it.meta & 0x80u) && !(BYTES && ((it.meta >> 24) & 3u) == MODE_NOERR);
+                    const bool is_text = i < n && !is_hit && !(it.meta & 0x80u) && !(BYTES && ((it.meta >> 24) & 3u) == MODE_NOERR);
                     const bool is_item = i < n && !is_hit && !is_text;
                     const uint32_t hb = __ballot_sync(0xFFFFFFFFu, is_hit), ib = __ballot_sync(0xFFFFFFFFu, is_item), tb = __ballot_sync(0xFFFFFFFFu, is_text);
                     unsigned long long hbase = 0, ibase = 0, tbase = 0;
@@ -421,7 +407,7 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
                     // warp) instead of travelling to the frontier kernel as an item.  (Measured and dropped: letting the lane continue
                     // with one of its own hand-overs -- a new direction run in the same lane -- instead of the next pass: the warps then
                     // mix the classes the host sorted them by, k = 1 / 2 edit 18.8 -> 21.9 / 67.0 -> 82.5 ms.)
-                    const bool leaf = kTextReports && (s.kind == TN_TURN ? s.part + 1 == np : (s.kind == TN_NEXT && s.part == np));
+                    const bool leaf = s.kind == TN_TURN ? s.part + 1 == np : (s.kind == TN_NEXT && s.part == np);
                     if (leaf) {
                         const bool ok = !EDIT || PSEUDO || ((ch.LInfo == INFO_M || ch.LInfo == INFO_I) && (ch.RInfo == INFO_M || ch.RInfo == INFO_I));
                         if (ok && sp.l[search][np - 1] <= s.e && s.e <= sp.u[search][np - 1]) {
@@ -469,7 +455,6 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
                     rows[0] = R ? st.lb_rev : st.lb;
                     have = 0;
                     closed = false;
-                    reach = 0;
                     ok = fetch();
                 }
                 if (!ok) {
@@ -527,9 +512,6 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
                 }
             }
         }
-        // ---- F: window prefetch.  A lane whose walk has entered the last window word it holds fetches the next one NOW, together with
-        //      the other lanes in that situation, instead of stalling the warp alone in the middle of a visit a few iterations later
-        if (kPrefetch && top > 0 && !closed && have < (uint32_t)kTextWords && reach + SPW / 2 >= have * SPW) fetch();
         // ---- V: the popped node, then those of its children whose own children can only continue error free -----------------------
         nmini = 0;
         if (top > 0) mini[nmini++] = stk[--top];
@@ -585,7 +567,7 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
                     queue_run(ch, LC_VISIT);                             // no error left: its own visit, then error free
                 } else if (!PSEUDO && slot == 0 && eq && (EDIT ? ch.e + 1 == cup : true) && ch.pev > 1 && ch.part == s.part) {
                     queue_run(ch, LC_SKIP);                              // the matching stretch (edit distance: at the last error level) is skipped
-                } else if (EDIT && !PSEUDO && !BYTES && kBulk2 && slot == 0 && eq && ch.e + 2 == cup && ch.pev >= 4 && ch.part == s.part) {
+                } else if (EDIT && !PSEUDO && !BYTES && slot == 0 && eq && ch.e + 2 == cup && ch.pev >= 4 && ch.part == s.part) {
                     queue_run(ch, LC_BULK2);                             // two errors left: the stretch is evaluated 16 positions at a time
                 } else if (vi == 0 && !(slot == 0 && eq) && ch.e + 1 == cup && nmini < 4) {
                     ch.kind = TN_EXPAND;
@@ -615,7 +597,7 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
                 push(s);
                 continue;
             }
-            if constexpr (EDIT && !PSEUDO && !BYTES && kBulk2) {
+            if constexpr (EDIT && !PSEUDO && !BYTES) {
                 if (s.kind == LC_BULK2) {
                     // the matching stretch of a path with two errors left, sixteen positions per evaluation (bulk2_eval above); positions
                     // that are not decided there get their own visit here and their two children on the stack
@@ -684,9 +666,9 @@ __global__ void __launch_bounds__(256, FMB_TEXT_MINB) scheme_text_kernel(const _
         n_phys += __shfl_xor_sync(0xFFFFFFFFu, n_phys, o);
     }
     if (lane == 0) {
-        atomicAdd(out.counters + 0, (unsigned long long)n_ext);
-        atomicAdd(out.counters + 1, (unsigned long long)n_ext);
-        atomicAdd(out.counters + 2, (unsigned long long)n_phys);
+        atomicAdd(out.counters + CTR_EXTENSIONS, (unsigned long long)n_ext);
+        atomicAdd(out.counters + CTR_OCC_LOOKUPS, (unsigned long long)n_ext);
+        atomicAdd(out.counters + CTR_LINE_REQUESTS, (unsigned long long)n_phys);
     }
 }
 

@@ -1,8 +1,8 @@
 """GPU parity of the k-error search on the paths of run_scheme and its kernels that only switch on at some batch or table size, or
 under a knob: the text list sorted by class (> 65 536 items in a text pass), roots in several slabs, warp stacks that spill in text
 mode, the second attempt with a larger hit buffer, collections of many short sequences with queries that hold delimiters, and the
-alternative paths the knobs select.  Every case compares hits, located rows and fmb_stats.extensions with the oracle, and asserts
-from the kernel trace or from the result that it reached the path it is about.
+paths of an index without some of its optional tables, which the knobs emulate.  Every case compares hits, located rows and
+fmb_stats.extensions with the oracle, and asserts from the kernel trace or from the result that it reached the path it is about.
 
 The knobs are read once per process, so those cases run their searches in a child process (FMB_TRACE_SCHEME=1); the child writes
 its results to an .npz and the trace to stderr, and the parent compares them with oracle results computed once per module."""
@@ -163,21 +163,17 @@ def largest_text_pass(trace):
 # knob -> the run whose trace must show a text pass above TEXT_SORT_MIN (None: the knob turns text mode off)
 KNOBS = [
     ({}, "edit"),
-    ({"FMB_TEXT_SORT_HAMMING": "1"}, "ham"),
-    ({"FMB_NO_TEXT_SORT": "1"}, "edit"),
-    ({"FMB_NO_DIRECT_TEXT": "1"}, "edit"),
     ({"FMB_NO_TEXT": "1"}, None),
     ({"FMB_NO_SCHEME_JUMP": "1"}, None),            # (no jump tables in the view: no text windows either)
     ({"FMB_NO_BIKMER": "1"}, "edit"),
     ({"FMB_NO_JUMP4": "1"}, "edit"),
-    ({"FMB_SCHEME_SIMALL": "0"}, "edit"),
 ]
 
 
 @pytest.mark.parametrize("env,big_run", KNOBS, ids=[(",".join(e) or "default") for e, _ in KNOBS])
 def test_large_batch_and_knobs(wl_b, tmp_path, env, big_run):
-    """hits, located rows and extension counts equal the oracle's with the default paths and with every knob that selects an
-    alternative path (each is documented to give the same results)"""
+    """hits, located rows and extension counts equal the oracle's with the default paths and with every knob that emulates an index
+    without some of its optional tables (each is documented to give the same results)"""
     res, trace = run_child(tmp_path, wl_b["job"], env, "b")
     if big_run is None:
         assert all(kind == "frontier" for r in trace.values() for kind, _, _, _ in r), "the knob did not turn text mode off"
