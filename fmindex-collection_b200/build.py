@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libfmb200.so")
-SOURCES = ["fmb_lib.cu", "fmb_search.cu", "fmb_engine.cu", "fmb_build.cu", "fmb_io.cu"]
+SOURCES = ["fmb_lib.cu", "fmb_search.cu", "fmb_engine.cu", "fmb_build.cu", "fmb_io.cu", "fmb_extract.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

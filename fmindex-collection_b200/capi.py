@@ -46,6 +46,7 @@ SYMBOLS = [
     "fmb_results_count", "fmb_results_kind", "fmb_results_fetch_hits", "fmb_results_fetch_locs", "fmb_results_fetch_locs32",
     "fmb_results_get_stats", "fmb_results_destroy",
     "fmb_search_and_locate", "fmb_search_and_locate_packed", "fmb_search_and_locate_multi", "fmb_search_and_locate_parts", "fmb_index_replicate", "fmb_index_save", "fmb_index_load", "fmb_checksum64",
+    "fmb_index_sequence_count", "fmb_index_sequence_lengths", "fmb_extract", "fmb_index_reconstruct_text",
     "fmb_index_set_exact_mode", "fmb_index_set_locate_mode", "fmb_synth_text_device", "fmb_synth_reads_device", "fmb_synth_reads_err_device", "fmb_synth_repeat_text_device", "fmb_synth_unit_reads_device", "fmb_index_set_stream", "fmb_set_image_budget", "fmb_measure_gather", "fmb_kernel_launch_count", "fmb_device_free", "fmb_copy_to_host", "fmb_host_alloc_pinned", "fmb_host_free_pinned",
 ]
 
@@ -304,6 +305,41 @@ class Index:
         pos = np.zeros(rows.size, dtype=np.uint32)
         _check(lib().fmb_sample_value(self.h, _ptr(rows), C.c_uint64(rows.size), _ptr(has), _ptr(seq), _ptr(pos)))
         return has, seq, pos
+
+    def sequence_count(self):
+        """number of sequences of the collection (= delimiters)"""
+        c = C.c_uint64()
+        _check(lib().fmb_index_sequence_count(self.h, C.byref(c)))
+        return c.value
+
+    def sequence_lengths(self):
+        """symbols per sequence, delimiter excluded (uint64 array)"""
+        out = np.zeros(self.sequence_count(), dtype=np.uint64)
+        _check(lib().fmb_index_sequence_lengths(self.h, _ptr(out)))
+        return out
+
+    def extract(self, seq, begin, end, with_stats=False):
+        """text of sequence seq[i] at [begin[i], end[i]) for every i, read back from the index on the GPU (fmb_extract).  Scalars give
+        one uint8 array; arrays give a list of uint8 arrays (views of one buffer).  with_stats=True also returns the Stats."""
+        scalar = np.ndim(seq) == 0 and np.ndim(begin) == 0 and np.ndim(end) == 0
+        seq, begin, end = np.broadcast_arrays(_u64(seq).reshape(-1), _u64(begin).reshape(-1), _u64(end).reshape(-1))
+        seq, begin, end = _u64(seq), _u64(begin), _u64(end)
+        count = seq.size
+        offsets = np.zeros(count + 1, dtype=np.uint64)
+        need = int((end.astype(np.int64) - begin.astype(np.int64)).clip(min=0).sum()) if count else 0
+        out = np.zeros(max(need, 1), dtype=np.uint8)
+        st = Stats()
+        _check(lib().fmb_extract(self.h, _ptr(seq), _ptr(begin), _ptr(end), C.c_uint64(count), _ptr(out), C.c_uint64(need),
+                                 _ptr(offsets), C.byref(st)))
+        parts = [out[offsets[i]:offsets[i + 1]] for i in range(count)]
+        res = parts[0] if scalar else parts
+        return (res, st) if with_stats else res
+
+    def reconstruct_text(self):
+        """reconstructText (utils.h:672): the text s0 0 s1 0 ... 0 the index was built from, n bytes"""
+        out = np.zeros(self.info.n, dtype=np.uint8)
+        _check(lib().fmb_index_reconstruct_text(self.h, _ptr(out), C.c_uint64(out.size)))
+        return out
 
     def search_and_locate(self, symbols, offsets, scheme=None, partition=None, edit=False, capacity=None,
                           out=None, packed=None):

@@ -122,6 +122,15 @@ struct fmb_index {
     // engine of the one-call end-to-end path (persistent worker threads + streams, csrc/fmb_engine.cu), created on first use
     mutable void* engine = nullptr;
     mutable std::mutex engine_mu;
+    // text extraction (csrc/fmb_extract.cu), built on the first call that needs it under anchor_mu: per sequence its length, its
+    // offset in the text s0 0 s1 0 ... and the row of its delimiter; then the anchor table -- text positions with known rows, sorted
+    // by position (every sample plus every delimiter), as two parallel arrays
+    mutable std::mutex anchor_mu;
+    mutable bool layout_ready = false;
+    mutable std::vector<uint64_t> seq_len, seq_start;
+    mutable std::vector<uint32_t> seq_delim_row;
+    mutable fmb::DevBuf<uint32_t> anchor_pos, anchor_row;
+    mutable uint64_t n_anchors = 0;
 
     fmb::IndexView<fmb::OccDna> view_dna() const;
     fmb::IndexView<fmb::OccGen> view_gen() const;

@@ -108,7 +108,7 @@ void pool_free(void* p) {
     P.cached_bytes += key.second;
 }
 
-static int use_device(int device) {
+int use_device(int device) {
     int cnt = 0;
     cudaError_t e = cudaGetDeviceCount(&cnt);
     if (e != cudaSuccess || cnt == 0) {
@@ -269,6 +269,7 @@ uint64_t fmb_index::device_bytes() const {
     b += locblocks.p ? locblocks.bytes() : 0;
     b += locrow.p ? locrow.bytes() : 0;
     b += samples.p ? samples.bytes() : 0;
+    b += anchor_pos.p ? anchor_pos.bytes() + anchor_row.bytes() : 0;
     return b;
 }
 
@@ -295,7 +296,7 @@ static uint32_t gen_bikmer_k(const fmb_index* ix) {
     return k;
 }
 static std::atomic<uint64_t> g_image_budget{0};          // bytes, 0 = no limit
-static uint64_t image_budget() {
+uint64_t image_budget() {
     uint64_t b = g_image_budget.load();
     if (!b) {
         static const double env_gb = getenv("FMB_IMAGE_GB") ? atof(getenv("FMB_IMAGE_GB")) : 0.0;
@@ -900,6 +901,7 @@ void fmb_index_destroy(fmb_index* ix) {
 
 int fmb_index_get_info(const fmb_index* ix, fmb_index_info* info) {
     if (!ix || !info) { set_error("NULL argument"); return FMB_EINVAL; }
+    std::lock_guard<std::mutex> lk(ix->anchor_mu);     // the anchor table may be being built by another thread
     memset(info, 0, sizeof *info);
     info->n = ix->n;
     info->sigma = ix->sigma;
@@ -914,6 +916,7 @@ int fmb_index_get_info(const fmb_index* ix, fmb_index_info* info) {
     info->tables = (ix->occ2[0].p ? FMB_TABLE_PAIR : 0) | (ix->kmer.p ? FMB_TABLE_KMER : 0) | (ix->jump[0].p ? FMB_TABLE_JUMP : 0) |
                    (ix->jump[1].p ? FMB_TABLE_JUMP_REV : 0) | (ix->locblocks.p ? FMB_TABLE_LOCBLOCK : 0) | (ix->locrow.p ? FMB_TABLE_LOCROW : 0) |
                    (ix->bikmer.p ? FMB_TABLE_BIKMER : 0) | (ix->jump4[0].p ? FMB_TABLE_JUMP4 : 0) | (ix->jump_shift[0] ? FMB_TABLE_JUMP32 : 0);
+    info->tables |= ix->anchor_pos.p ? FMB_TABLE_ANCHORS : 0;
     return FMB_OK;
 }
 

@@ -78,6 +78,7 @@ typedef struct {
 #define FMB_TABLE_BIKMER   64u  /* bidirectional k-mer table for scheme roots      */
 #define FMB_TABLE_JUMP4    128u /* LF^4 jump tables (tails shorter than 16 symbols) */
 #define FMB_TABLE_JUMP32   256u /* direction 0 holds merged LF^16 / LF^32 entries (32 symbols per lookup in exact search) */
+#define FMB_TABLE_ANCHORS  512u /* anchor table of text extraction (built on the first extraction call)                  */
 
 /* work counters of the last search/locate call on a result set (device-side counting, optional) */
 typedef struct {
@@ -246,6 +247,24 @@ int fmb_locate_rows(const fmb_index* ix, const uint64_t* rows, uint64_t count, u
 /* index.single_locate_step(idx) = annotatedArray.value(idx) (fmindex/BiFMIndex.h:204-206, suffixarray/SparseArray.h:63-70):
  * has[i] = 1 and (seq[i], pos[i]) = the sample when row i is sampled, else has[i] = 0. */
 int fmb_sample_value(const fmb_index* ix, const uint64_t* rows, uint64_t count, uint8_t* has, uint32_t* seq, uint32_t* pos);
+
+/* ---- text extraction: reconstructText (utils.h:672) and substrings of it, on the GPU.  All pointers host. ----
+ * The index holds no copy of the text; the text is read back from the BWT with backward LF walks.  The first call that needs it builds
+ * the anchor table (FMB_TABLE_ANCHORS: every sampled row and every delimiter row with its text position, 8 bytes per anchor, counted
+ * in device_bytes; FMB_ENOMEM when it does not fit the image budget in force at that call, the index stays usable).  A range (seq, begin, end) is the
+ * symbols [begin, end) of sequence seq, delimiter excluded.  Every walk between two anchors takes LF^16 steps of direction 0 where the
+ * index has that table, LF^4 steps for the rest and single LF steps on the occurrence blocks otherwise; stats->line_requests counts
+ * jump-table lookups, stats->lf_steps single LF steps (stats may be NULL).  FMB_EUNSUPPORTED for FMB_INDEX_NO_DELIM indices, which
+ * have no sequence boundaries.  Works on ReuseRev and unidirectional indices. */
+int fmb_index_sequence_count(const fmb_index* ix, uint64_t* count);                       /* = number of delimiters, no launch */
+int fmb_index_sequence_lengths(const fmb_index* ix, uint64_t* lengths /* count */);       /* symbols per sequence, no delimiter */
+/* Range i is written to out + offsets[i] (offsets: count + 1 entries, offsets[count] = bytes written).  FMB_EINVAL, before any launch
+ * once the table exists, for seq >= count, begin > end or end > length; and for capacity < the bytes needed, which offsets[count]
+ * then reports. */
+int fmb_extract(const fmb_index* ix, const uint64_t* seq, const uint64_t* begin, const uint64_t* end, uint64_t count,
+                uint8_t* out, uint64_t capacity, uint64_t* offsets /* count + 1 */, fmb_stats* stats);
+/* the whole text s0 0 s1 0 ... 0, n bytes: the input of fmb_index_build, so build -> reconstruct round-trips (capacity >= n) */
+int fmb_index_reconstruct_text(const fmb_index* ix, uint8_t* out, uint64_t capacity);
 
 /* ---- results ----------------------------------------------------------------------------------------------- */
 uint64_t fmb_results_count(const fmb_results* r);

@@ -156,6 +156,26 @@ auto locate_rows_raw(fmb_index const* ix, Rows const& rows) -> std::vector<std::
 template <typename index_t, typename Rows>
 auto locate_rows(index_t const& index, Rows const& rows) { return locate_rows_raw(index.handle(), rows); }
 
+// a range of text: symbols [begin, end) of sequence seq (delimiter excluded), for extract()
+struct TextRange {
+    uint64_t seq, begin, end;
+};
+// text extraction (fmb_extract, reconstructText utils.h:672): the symbols of every range, one vector per range
+inline auto extract_raw(fmb_index const* ix, std::span<TextRange const> ranges, fmb_stats* stats = nullptr) -> std::vector<std::vector<uint8_t>> {
+    size_t const count = ranges.size();
+    std::vector<uint64_t> seq(count), begin(count), end(count), offsets(count + 1);
+    uint64_t need = 0;
+    for (size_t i = 0; i < count; ++i) {
+        seq[i] = ranges[i].seq, begin[i] = ranges[i].begin, end[i] = ranges[i].end;
+        need += end[i] > begin[i] ? end[i] - begin[i] : 0;
+    }
+    std::vector<uint8_t> buf(need);
+    check(fmb_extract(ix, seq.data(), begin.data(), end.data(), count, buf.data(), need, offsets.data(), stats));
+    std::vector<std::vector<uint8_t>> out(count);
+    for (size_t i = 0; i < count; ++i) out[i].assign(buf.begin() + offsets[i], buf.begin() + offsets[i + 1]);
+    return out;
+}
+
 template <typename Index> struct BiFMIndexCursor;
 template <typename Index> struct LeftBiFMIndexCursor;
 template <typename Index> struct FMIndexCursor;
@@ -203,6 +223,24 @@ struct IndexBase {
         check(fmb_sample_value(h.get(), &row, 1, &has, &seq, &pos));
         if (!has) return std::nullopt;
         return ADEntry{seq, pos};
+    }
+
+    // symbols per sequence, delimiter excluded (fmb_index_sequence_lengths)
+    auto sequence_lengths() const -> std::vector<uint64_t> {
+        uint64_t count{};
+        check(fmb_index_sequence_count(h.get(), &count));
+        std::vector<uint64_t> out(count);
+        check(fmb_index_sequence_lengths(h.get(), out.data()));
+        return out;
+    }
+    // symbols [begin, end) of sequence seq, read back from the index on the GPU (fmb_extract)
+    auto extract(uint64_t seq, uint64_t begin, uint64_t end) const -> std::vector<uint8_t> {
+        TextRange r{seq, begin, end};
+        return std::move(extract_raw(h.get(), std::span<TextRange const>(&r, 1))[0]);
+    }
+    // many ranges in one call
+    auto extract(std::span<TextRange const> ranges, fmb_stats* stats = nullptr) const -> std::vector<std::vector<uint8_t>> {
+        return extract_raw(h.get(), ranges, stats);
     }
 
 protected:
@@ -318,6 +356,14 @@ struct FMIndex : detail::IndexBase<TSigma, false> {
     }
     explicit FMIndex(fmb_index* raw) { Base::adopt(raw); }
 };
+
+// reconstructText (utils.h:672): the delimited text s0 0 s1 0 ... 0 the index was built from (fmb_index_reconstruct_text)
+template <typename Index>
+auto reconstructText(Index const& index) -> std::vector<uint8_t> {
+    std::vector<uint8_t> text(index.size());
+    check(fmb_index_reconstruct_text(index.handle(), text.data(), text.size()));
+    return text;
+}
 
 // ---- persistence (fmindex/diskStorage.h:13-27) -------------------------------------------------------------------------
 // saveIndex(index, path) / loadIndex<Index>(path): the flat file of fmb_index_save (BWT bytes + sampled suffix array; the device

@@ -152,6 +152,27 @@ struct PartitionedBiFMIndex {
         return n;
     }
 
+    // text extraction with sequence numbers of the whole collection: every range goes to the part that holds its sequence
+    auto extract(std::span<TextRange const> ranges, fmb_stats* stats = nullptr) const -> std::vector<std::vector<uint8_t>> {
+        std::vector<std::vector<TextRange>> local(parts.size());
+        std::vector<std::vector<size_t>> where(parts.size());
+        for (size_t i = 0; i < ranges.size(); ++i) {
+            size_t const p = static_cast<size_t>(std::upper_bound(seq_base.begin(), seq_base.end(), ranges[i].seq) - seq_base.begin()) - 1;
+            local[p].push_back({ranges[i].seq - seq_base[p], ranges[i].begin, ranges[i].end});
+            where[p].push_back(i);
+        }
+        std::vector<std::vector<uint8_t>> out(ranges.size());
+        if (stats) *stats = fmb_stats{};
+        for (size_t p = 0; p < parts.size(); ++p) {
+            if (local[p].empty()) continue;
+            fmb_stats s{};
+            auto got = parts[p].extract(std::span<TextRange const>(local[p]), &s);
+            for (size_t k = 0; k < got.size(); ++k) out[where[p][k]] = std::move(got[k]);
+            if (stats) stats->line_requests += s.line_requests, stats->lf_steps += s.lf_steps, stats->kernel_ms += s.kernel_ms;
+        }
+        return out;
+    }
+
     template <Sequences queries_t, detail::SchemeLike scheme_t = search_scheme::Scheme>
     std::vector<fmb_loc32> search_and_locate(queries_t const& queries, bool edit = false, scheme_t const* scheme = nullptr,
                                              std::vector<size_t> const* partition = nullptr, fmb_stats* stats = nullptr) const {
