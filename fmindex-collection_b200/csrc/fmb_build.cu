@@ -16,23 +16,7 @@
 #include "fmb_host.hpp"
 
 namespace fmb {
-
-int build_occ_from_device_bwt(fmb_index* ix, int dir, const uint8_t* d_bwt);
-int compute_C(fmb_index* ix);
-int build_occ2(fmb_index* ix, int dir);
-uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples);
-int build_locblocks(fmb_index* ix);
-int build_jump(fmb_index* ix, int dir);
-int widen_jump0(fmb_index* ix);
-int build_bikmer(fmb_index* ix);
-int new_index(fmb_index** out, int device, uint32_t sigma, uint64_t n, bool bidirectional, uint32_t flags);
-
 namespace {
-
-inline unsigned grid_for(uint64_t items, unsigned block) {
-    uint64_t g = (items + block - 1) / block;
-    return (unsigned)(g ? g : 1);
-}
 
 __global__ void reverse_text_kernel(const uint8_t* __restrict__ t, uint64_t n, uint8_t* __restrict__ out) {
     uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
@@ -359,13 +343,7 @@ extern "C" int fmb_index_build(fmb_index** out, int device, uint32_t sigma, cons
         FMB_TRY(cnt.alloc(words + 1));
         sample_words_kernel<<<grid_for(words + 1, 128), 128, 0, st>>>(sa.p, n, delims.p, (uint32_t)nd, sampling_rate, words, bitmap.p, cnt.p);
         FMB_CUDA(cudaGetLastError());
-        {
-            size_t tmp_bytes = 0;
-            FMB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, cnt.p, cnt.p, (int64_t)(words + 1), st));
-            DevBuf<uint8_t> tmp;
-            FMB_TRY(tmp.alloc(tmp_bytes));
-            FMB_CUDA(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, cnt.p, cnt.p, (int64_t)(words + 1), st));
-        }
+        FMB_TRY(exclusive_sum_u32(cnt.p, cnt.p, words + 1, st));
         uint32_t ns = 0;
         FMB_CUDA(cudaMemcpyAsync(&ns, cnt.p + words, 4, cudaMemcpyDeviceToHost, st));
         FMB_CUDA(cudaStreamSynchronize(st));
@@ -393,12 +371,8 @@ extern "C" int fmb_index_build(fmb_index** out, int device, uint32_t sigma, cons
     }
     bwt.release();
     FMB_TRY(compute_C(ix));
-    if (ix->dna) FMB_TRY(build_occ2(ix, 0));
-    if (!ix->dna) FMB_TRY(build_jump(ix, 0));
-    if (bidirectional) FMB_TRY(build_jump(ix, 1));
-    FMB_TRY(widen_jump0(ix));
-    FMB_TRY(build_bikmer(ix));
-    FMB_TRY(build_locblocks(ix));
+    FMB_TRY(build_search_tables(ix));
+    FMB_TRY(build_locate_tables(ix));
     guard.ix = nullptr;
     *out = ix;
     pool_trim();

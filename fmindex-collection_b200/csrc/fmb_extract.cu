@@ -20,18 +20,9 @@
 #include "fmb_host.hpp"
 
 namespace fmb {
-
-int use_device(int device);
-uint64_t image_budget();
-
 namespace {
 
 constexpr uint32_t kNone = 0xFFFFFFFFu;
-
-inline unsigned grid_for(uint64_t items, unsigned block) {
-    uint64_t g = (items + block - 1) / block;
-    return (unsigned)(g ? g : 1);
-}
 
 // the two work counters of a block, added to counters[0] and counters[1] with one atomic each per block (as block_count2 of
 // fmb_kernels.cuh, which cannot be included here: it defines the library's other kernels).  Every thread of the block calls it.
@@ -53,27 +44,6 @@ __device__ __forceinline__ void block_count(unsigned long long* counters, uint32
         if (s_cnt[1]) atomicAdd(counters + 1, (unsigned long long)s_cnt[1]);
     }
 }
-
-struct EventTimer {           // device time between construction and stop() on stream s
-    cudaEvent_t a = nullptr, b = nullptr;
-    cudaStream_t s;
-    explicit EventTimer(cudaStream_t s_) : s(s_) {
-        cudaEventCreate(&a);
-        cudaEventCreate(&b);
-        cudaEventRecord(a, s);
-    }
-    double stop() {
-        cudaEventRecord(b, s);
-        cudaEventSynchronize(b);
-        float ms = 0;
-        cudaEventElapsedTime(&ms, a, b);
-        return ms;
-    }
-    ~EventTimer() {
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-    }
-};
 
 // one thread per delimiter row: walk back to a sampled row or to position 0 of the sequence (see the header comment)
 template <class OCC>

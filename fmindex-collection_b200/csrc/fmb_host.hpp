@@ -102,12 +102,12 @@ struct fmb_index {
     int locate_mode = 0;                 // FMB_LOCATE_*
     uint64_t n_samples = 0;
     uint64_t C[65] = {0};
-    // two-symbol table (OccDna2), sigma <= 5 only
-    fmb::DevBuf<uint4> occ2[2];
-    fmb::DevBuf<uint32_t> specials[2];
-    uint32_t n_specials[2] = {0, 0};
-    uint32_t special01[2][2] = {{0xFFFFFFFFu, 0xFFFFFFFFu}, {0xFFFFFFFFu, 0xFFFFFFFFu}};
-    uint32_t C2[2][16] = {};
+    // two-symbol table (OccDna2) of direction 0, sigma <= 5 only
+    fmb::DevBuf<uint4> occ2;
+    fmb::DevBuf<uint32_t> specials;
+    uint32_t n_specials = 0;
+    uint32_t special01[2] = {0xFFFFFFFFu, 0xFFFFFFFFu};
+    uint32_t C2[16] = {};
     fmb::DevBuf<uint2> jump[2];          // LF^16 jump tables
     uint32_t jump_shift[2] = {0, 0};     // 1: the table holds 16-byte entries {LF^16, 16 symbols, LF^32, 16 more symbols} (two uint2 per row)
     fmb::DevBuf<uint2> jump4[2];         // LF^4 jump tables (same entry format, 4 symbols in the low 8 bits)
@@ -116,8 +116,8 @@ struct fmb_index {
     fmb::DevBuf<uint4> bikmer;           // bidirectional k-mer table for scheme-search roots
     uint32_t bikmer_k = 0;
     int exact_mode = 0;                  // FMB_EXACT_*
-    // optional tables this image is allowed to hold (FMB_TABLE_* bits), decided once from the image budget (fmb_set_image_budget /
-    // FMB_IMAGE_GB; default: everything the device can hold)
+    // optional tables this image is allowed to hold (FMB_TABLE_* bits), decided once by plan_tables (csrc/fmb_lib.cu) from the image
+    // budget (fmb_set_image_budget / FMB_IMAGE_GB; default: everything the device can hold) and the FMB_NO_* knobs of its knob table
     uint32_t allowed_tables = 0xFFFFFFFFu;
     // engine of the one-call end-to-end path (persistent worker threads + streams, csrc/fmb_engine.cu), created on first use
     mutable void* engine = nullptr;
@@ -134,8 +134,31 @@ struct fmb_index {
 
     fmb::IndexView<fmb::OccDna> view_dna() const;
     fmb::IndexView<fmb::OccGen> view_gen() const;
-    fmb::Occ2View view_occ2(int dir) const;
+    fmb::Occ2View view_occ2() const;
     uint64_t device_bytes() const;
+
+    // The image's device buffers, the one list that device_bytes() and fmb_index_replicate walk: f(buffer of a, the same buffer of
+    // b, replicated).  The anchor table is counted in the image but not replicated: a replica builds its own on first use.
+    template <class A, class B, class F>
+    static void for_each_buffer(A& a, B& b, F&& f) {
+        for (int d = 0; d < 2; ++d) {
+            f(a.occ_dna[d], b.occ_dna[d], true);
+            f(a.occ_gen[d], b.occ_gen[d], true);
+            f(a.delim_rows[d], b.delim_rows[d], true);
+            f(a.jump[d], b.jump[d], true);
+            f(a.jump4[d], b.jump4[d], true);
+        }
+        f(a.occ2, b.occ2, true);
+        f(a.specials, b.specials, true);
+        f(a.marks, b.marks, true);
+        f(a.samples, b.samples, true);
+        f(a.locblocks, b.locblocks, true);
+        f(a.locrow, b.locrow, true);
+        f(a.kmer, b.kmer, true);
+        f(a.bikmer, b.bikmer, true);
+        f(a.anchor_pos, b.anchor_pos, false);
+        f(a.anchor_row, b.anchor_row, false);
+    }
 };
 
 namespace fmb {
@@ -144,6 +167,48 @@ namespace fmb {
 extern thread_local cudaStream_t tls_stream_override;
 inline cudaStream_t active_stream(const fmb_index* ix) { return tls_stream_override ? tls_stream_override : ix->stream; }
 void engine_destroy(fmb_index* ix);   // joins the worker threads of the index's engine, if it has one
+
+// ---- index image construction (K1, csrc/fmb_lib.cu), shared by fmb_index_create_ex and fmb_index_build --------------------------
+int use_device(int device);
+int new_index(fmb_index** out, int device, uint32_t sigma, uint64_t n, bool bidirectional, uint32_t flags);
+uint64_t image_budget();                                           // bytes, 0 = no limit
+uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples);     // the FMB_TABLE_* bits for ix->allowed_tables
+int build_occ_from_device_bwt(fmb_index* ix, int dir, const uint8_t* d_bwt);
+int compute_C(fmb_index* ix);
+// after compute_C: pair + k-mer tables (DNA layout), the LF jump tables of directions 0 and 1, the merged LF^32 entries and the
+// bidirectional k-mer table
+int build_search_tables(fmb_index* ix);
+// after the marks: locate blocks (DNA layout), then the locate shortcut
+int build_locate_tables(fmb_index* ix);
+
+inline unsigned grid_for(uint64_t items, unsigned block) {
+    uint64_t g = (items + block - 1) / block;
+    return (unsigned)(g ? g : 1);
+}
+
+struct EventTimer {           // device time between construction and stop() on stream s
+    cudaEvent_t a = nullptr, b = nullptr;
+    cudaStream_t s;
+    explicit EventTimer(cudaStream_t s_) : s(s_) {
+        cudaEventCreate(&a);
+        cudaEventCreate(&b);
+        cudaEventRecord(a, s);
+    }
+    double stop() {
+        cudaEventRecord(b, s);
+        cudaEventSynchronize(b);
+        float ms = 0;
+        cudaEventElapsedTime(&ms, a, b);
+        return ms;
+    }
+    ~EventTimer() {
+        cudaEventDestroy(a);
+        cudaEventDestroy(b);
+    }
+};
+
+// exclusive prefix sum of u32 -> u32 on `stream`, synchronised (CUB; plumbing, not a hot kernel)
+int exclusive_sum_u32(const uint32_t* in, uint32_t* out, uint64_t count, cudaStream_t stream);
 }  // namespace fmb
 
 struct fmb_queries {

@@ -140,39 +140,24 @@ static int raw_alloc(uint8_t** p, size_t bytes) {
     return FMB_OK;
 }
 
-static inline unsigned grid_for(uint64_t items, unsigned block) {
-    return (unsigned)std::max<uint64_t>(1, (items + block - 1) / block);
-}
-
-struct EventTimer {
-    cudaEvent_t a = nullptr, b = nullptr;
-    cudaStream_t s;
-    explicit EventTimer(cudaStream_t s_) : s(s_) {
-        cudaEventCreate(&a);
-        cudaEventCreate(&b);
-        cudaEventRecord(a, s);
-    }
-    double stop() {
-        cudaEventRecord(b, s);
-        cudaEventSynchronize(b);
-        float ms = 0;
-        cudaEventElapsedTime(&ms, a, b);
-        return ms;
-    }
-    ~EventTimer() {
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-    }
-};
-
-// exclusive prefix sum of u32 -> u32 on `stream` (CUB; plumbing, not a hot kernel)
-static int exclusive_sum_u32(const uint32_t* in, uint32_t* out, uint64_t count, cudaStream_t stream) {
+int exclusive_sum_u32(const uint32_t* in, uint32_t* out, uint64_t count, cudaStream_t stream) {
     size_t tmp_bytes = 0;
     FMB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, in, out, (int64_t)count, stream));
     DevBuf<uint8_t> tmp;
     FMB_TRY(tmp.alloc(tmp_bytes));
     FMB_CUDA(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, in, out, (int64_t)count, stream));
     FMB_CUDA(cudaStreamSynchronize(stream));
+    return FMB_OK;
+}
+
+// in-place exclusive scan of `count` values of a custom type with `op` on `stream`, not synchronised (CUB)
+template <typename T, typename Op>
+static int exclusive_scan(T* data, uint64_t count, Op op, T init, cudaStream_t stream) {
+    size_t tmp_bytes = 0;
+    FMB_CUDA(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, data, data, op, init, (int64_t)count, stream));
+    DevBuf<uint8_t> tmp;
+    FMB_TRY(tmp.alloc(tmp_bytes));
+    FMB_CUDA(cub::DeviceScan::ExclusiveScan(tmp.p, tmp_bytes, data, data, op, init, (int64_t)count, stream));
     return FMB_OK;
 }
 
@@ -242,34 +227,25 @@ fmb::IndexView<fmb::OccGen> fmb_index::view_gen() const {
         }                                           \
     } while (0)
 
-fmb::Occ2View fmb_index::view_occ2(int dir) const {
+fmb::Occ2View fmb_index::view_occ2() const {
     fmb::Occ2View v{};
-    v.lines = occ2[dir].p;
-    v.specials = specials[dir].p;
-    v.n_specials = n_specials[dir];
-    v.s0 = special01[dir][0];
-    v.s1 = special01[dir][1];
-    for (int i = 0; i < 16; ++i) v.C2[i] = C2[dir][i];
-    v.jump = jump[dir].p;
-    v.jump_wide = jump_shift[dir];
-    v.jump4 = jump4[dir].p;
-    v.kmer = dir == 0 ? kmer.p : nullptr;
-    v.kmer_k = dir == 0 ? kmer_k : 0;
+    v.lines = occ2.p;
+    v.specials = specials.p;
+    v.n_specials = n_specials;
+    v.s0 = special01[0];
+    v.s1 = special01[1];
+    for (int i = 0; i < 16; ++i) v.C2[i] = C2[i];
+    v.jump = jump[0].p;
+    v.jump_wide = jump_shift[0];
+    v.jump4 = jump4[0].p;
+    v.kmer = kmer.p;
+    v.kmer_k = kmer_k;
     return v;
 }
 
 uint64_t fmb_index::device_bytes() const {
     uint64_t b = 0;
-    for (int d = 0; d < 2; ++d) b += occ2[d].p ? occ2[d].bytes() + specials[d].bytes() : 0;
-    b += kmer.p ? kmer.bytes() : 0;
-    b += bikmer.p ? bikmer.bytes() : 0;
-    for (int d = 0; d < 2; ++d) b += (jump[d].p ? jump[d].bytes() : 0) + (jump4[d].p ? jump4[d].bytes() : 0);
-    for (int d = 0; d < 2; ++d) b += occ_dna[d].p ? occ_dna[d].bytes() : 0, b += occ_gen[d].p ? occ_gen[d].bytes() : 0, b += delim_rows[d].p ? delim_rows[d].bytes() : 0;
-    b += marks.p ? marks.bytes() : 0;
-    b += locblocks.p ? locblocks.bytes() : 0;
-    b += locrow.p ? locrow.bytes() : 0;
-    b += samples.p ? samples.bytes() : 0;
-    b += anchor_pos.p ? anchor_pos.bytes() + anchor_row.bytes() : 0;
+    for_each_buffer(*this, *this, [&](const auto& buf, const auto&, bool) { b += buf.bytes(); });
     return b;
 }
 
@@ -278,15 +254,18 @@ uint64_t fmb_index::device_bytes() const {
 // ---------------------------------------------------------------------------------------------------------
 namespace fmb {
 
-int build_jump(fmb_index* ix, int dir);
-int widen_jump0(fmb_index* ix);
-
 // ---- image budget: which accelerating tables an index may hold ----------------------------------------------------------------
 // Every table beyond the occurrence blocks is optional (results never depend on them); they trade HBM for speed.  With a budget
 // the tables are admitted in the order of what they buy per byte (measured: profiles/r02_image_budget_curve.json):
 //   pair table + k-mer table (exact search: two symbols per line, the first 14 symbols in one lookup), locate blocks,
 //   LF^16 table of direction 0 (sixteen symbols per lookup once an interval is a single row), LF^16 of direction 1 (text windows of
 //   the k-error searches in both directions), bidirectional k-mer table, locate shortcut, merged LF^32 entries, LF^4 tables.
+// DNA layout, both k-mer tables: largest k <= 14 with 8 * 4^k <= n (the exact-search table, 8 bytes per k-mer, stays below ~n bytes)
+static uint32_t dna_kmer_k(uint64_t n) {
+    uint32_t k = 0;
+    while (k < 14 && (uint64_t(8) << (2 * (k + 1))) <= n) ++k;
+    return k;
+}
 // generic layout: largest k <= 8 whose table of (sigma - first_symb)^k entries stays below 2 n bytes (1 Gaa, sigma = 21: k = 6, 1 GB)
 static uint32_t gen_bikmer_k(const fmb_index* ix) {
     const uint64_t base = ix->sigma - ix->first_symb;
@@ -304,7 +283,7 @@ uint64_t image_budget() {
     }
     return b;
 }
-uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
+static uint32_t budget_tables(const fmb_index* ix, uint64_t n_samples) {
     const uint64_t budget = image_budget();
     if (!budget) return 0xFFFFFFFFu;
     const double n = (double)ix->n;
@@ -316,15 +295,12 @@ uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
         return false;
     };
     if (ix->dna) {
-        uint32_t k = 0;
-        while (k < 14 && (uint64_t(8) << (2 * (k + 1))) <= ix->n) ++k;
+        const uint32_t k = dna_kmer_k(ix->n);
         admit(FMB_TABLE_PAIR | FMB_TABLE_KMER, n + 8.0 * (double)(uint64_t(1) << (2 * k)));
         admit(FMB_TABLE_LOCBLOCK, n);
         const bool j0 = admit(FMB_TABLE_JUMP, 8 * n);
         const bool j1 = ix->bidirectional && admit(FMB_TABLE_JUMP_REV, 8 * n);
-        uint32_t bk = 0;
-        while (bk < 14 && (uint64_t(8) << (2 * (bk + 1))) <= ix->n) ++bk;
-        if (ix->bidirectional) admit(FMB_TABLE_BIKMER, 16.0 * (double)(uint64_t(1) << (2 * bk)));
+        if (ix->bidirectional) admit(FMB_TABLE_BIKMER, 16.0 * (double)(uint64_t(1) << (2 * k)));
         if (allowed & FMB_TABLE_LOCBLOCK) admit(FMB_TABLE_LOCROW, 4 * n);
         if (j0) admit(FMB_TABLE_JUMP32, 8 * n);
         if (j0) admit(FMB_TABLE_JUMP4, 8 * n * (j1 ? 2 : 1));
@@ -337,6 +313,31 @@ uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
             admit(FMB_TABLE_BIKMER, 16 * cnt);
         }
     }
+    return allowed;
+}
+
+// The tables admitted by the budget, less those of the knobs set in the environment, read on every build.  The knobs are applied
+// after admission, so a knob frees no budget for later tables.  Knob table:
+//   knob               DNA layout (sigma <= 5 with delimiter) clears   generic layout clears
+//   FMB_NO_JUMP        JUMP, JUMP_REV, JUMP4, JUMP32                    JUMP4 (its only jump tables)
+//   FMB_NO_JUMP32      JUMP32                                           -
+//   FMB_NO_JUMP4       JUMP4                                            -
+//   FMB_NO_BIKMER      BIKMER                                           BIKMER
+//   FMB_NO_LOCBLOCKS   LOCBLOCK, LOCROW (the shortcut walks the blocks) -
+//   FMB_NO_LOCROW      LOCROW                                           LOCROW
+// FMB_KMER_K (build_occ2) sizes the exact-search k-mer table; FMB_KMER_K=0 leaves it out.
+uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
+    static const struct { const char* name; uint32_t dna, gen; } knobs[] = {
+        {"FMB_NO_JUMP", FMB_TABLE_JUMP | FMB_TABLE_JUMP_REV | FMB_TABLE_JUMP4 | FMB_TABLE_JUMP32, FMB_TABLE_JUMP4},
+        {"FMB_NO_JUMP32", FMB_TABLE_JUMP32, 0},
+        {"FMB_NO_JUMP4", FMB_TABLE_JUMP4, 0},
+        {"FMB_NO_BIKMER", FMB_TABLE_BIKMER, FMB_TABLE_BIKMER},
+        {"FMB_NO_LOCBLOCKS", FMB_TABLE_LOCBLOCK | FMB_TABLE_LOCROW, 0},
+        {"FMB_NO_LOCROW", FMB_TABLE_LOCROW, FMB_TABLE_LOCROW},
+    };
+    uint32_t allowed = budget_tables(ix, n_samples);
+    for (const auto& k : knobs)
+        if (getenv(k.name)) allowed &= ~(ix->dna ? k.dna : k.gen);
     return allowed;
 }
 
@@ -365,13 +366,7 @@ int build_occ_from_device_bwt(fmb_index* ix, int dir, const uint8_t* d_bwt) {
         FMB_CUDA(cudaStreamSynchronize(st));
         if (h_bad) { set_error("BWT contains a symbol >= sigma (%u)", ix->sigma); return FMB_EINVAL; }
         // number of delimiter rows = total count of symbol 0 (last block's scanned count + its local count): take it from C later
-        {
-            size_t tmp_bytes = 0;
-            FMB_CUDA(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, counts.p, counts.p, Cnt32Add{}, Cnt32{}, (int64_t)nblocks, st));
-            DevBuf<uint8_t> tmp;
-            FMB_TRY(tmp.alloc(tmp_bytes));
-            FMB_CUDA(cub::DeviceScan::ExclusiveScan(tmp.p, tmp_bytes, counts.p, counts.p, Cnt32Add{}, Cnt32{}, (int64_t)nblocks, st));
-        }
+        FMB_TRY(exclusive_scan(counts.p, nblocks, Cnt32Add{}, Cnt32{}, st));
         store_gen_counts_kernel<<<grid_for(nblocks, 128), 128, 0, st>>>(ix->occ_gen[dir].p, ix->gen_stride, planes, ix->sigma, counts.p, nblocks);
         FMB_CUDA(cudaGetLastError());
         FMB_CUDA(cudaStreamSynchronize(st));
@@ -394,14 +389,7 @@ int build_occ_from_device_bwt(fmb_index* ix, int dir, const uint8_t* d_bwt) {
         set_error("BWT contains a symbol >= sigma (%u)", ix->sigma);
         return FMB_EINVAL;
     }
-    // exclusive scan of the per-block symbol counts
-    {
-        size_t tmp_bytes = 0;
-        FMB_CUDA(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, counts.p, counts.p, Uint4Add{}, make_uint4(0, 0, 0, 0), (int64_t)nblocks, st));
-        DevBuf<uint8_t> tmp;
-        FMB_TRY(tmp.alloc(tmp_bytes));
-        FMB_CUDA(cub::DeviceScan::ExclusiveScan(tmp.p, tmp_bytes, counts.p, counts.p, Uint4Add{}, make_uint4(0, 0, 0, 0), (int64_t)nblocks, st));
-    }
+    FMB_TRY(exclusive_scan(counts.p, nblocks, Uint4Add{}, make_uint4(0, 0, 0, 0), st));      // per-block symbol counts
     store_counts_kernel<<<grid_for(nblocks, 256), 256, 0, st>>>(ix->occ_dna[dir].p, counts.p, nblocks);
     FMB_CUDA(cudaGetLastError());
     // delimiter rows: scan per-block delimiter counts, then scatter the rows
@@ -447,9 +435,9 @@ __global__ void compute_C2_kernel(IndexView<OccDna> ix, int dir, uint32_t* out) 
     out[code] = (x < ix.sigma && y < ix.sigma) ? ix.C[x] + occ.rank(b, at, x) : 0u;
 }
 
-// bidirectional k-mer table (16 bytes per k-mer): largest k <= 13 with 16 * 4^k <= n / 2; needs both occ tables and C
-int build_bikmer(fmb_index* ix) {
-    if (!ix->bidirectional || getenv("FMB_NO_BIKMER") || !(ix->allowed_tables & FMB_TABLE_BIKMER)) return FMB_OK;
+// bidirectional k-mer table (16 bytes per k-mer, k from dna_kmer_k / gen_bikmer_k); needs both occ tables and C
+static int build_bikmer(fmb_index* ix) {
+    if (!ix->bidirectional || !(ix->allowed_tables & FMB_TABLE_BIKMER)) return FMB_OK;
     if (!ix->dna) {
         const uint32_t k = gen_bikmer_k(ix), base = ix->sigma - ix->first_symb;
         if (k < 2) return FMB_OK;
@@ -464,8 +452,7 @@ int build_bikmer(fmb_index* ix) {
         ix->bikmer_k = k;
         return FMB_OK;
     }
-    uint32_t k = 0;
-    while (k < 14 && (uint64_t(8) << (2 * (k + 1))) <= ix->n) ++k;
+    const uint32_t k = dna_kmer_k(ix->n);
     if (k < 2) return FMB_OK;
     const uint64_t count = uint64_t(1) << (2 * k);
     cudaStream_t st = active_stream(ix);
@@ -477,149 +464,116 @@ int build_bikmer(fmb_index* ix) {
     return FMB_OK;
 }
 
-// combined 64-byte locate records (needs occ table 0 and the marks); skipped when FMB_NO_LOCBLOCKS is set
-int build_locblocks(fmb_index* ix) {
-    if (!ix->dna && ix->marks.p && ix->n_samples && !getenv("FMB_NO_LOCROW") && (ix->allowed_tables & FMB_TABLE_LOCROW)) {
-        // generic layout: the locate shortcut alone (every row walked once, one thread per row)
-        uint32_t idx_bits = 1;
-        while (idx_bits < 32 && (uint64_t(1) << idx_bits) < ix->n_samples) ++idx_bits;
-        const uint32_t step_bits = 32 - idx_bits;
-        size_t free_b = 0, total_b = 0;
-        pool_trim();
-        FMB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-        if (step_bits < 1 || (double)free_b < 4.0 * (double)ix->n * 1.5 + (double)(1u << 28)) return FMB_OK;
-        cudaStream_t st = active_stream(ix);
-        FMB_TRY(ix->locrow.alloc(ix->n));
-        DevBuf<uint32_t> ovf;
-        FMB_TRY(ovf.alloc(1));
-        FMB_CUDA(cudaMemsetAsync(ovf.p, 0, sizeof(uint32_t), st));
-        ix->loc_step_bits = step_bits;
-        locrow_build_gen_kernel<<<grid_for(ix->n, 256), 256, 0, st>>>(ix->view_gen(), step_bits, ix->locrow.p, ovf.p);
-        FMB_CUDA(cudaGetLastError());
-        note_launches(1);
-        uint32_t h_ovf = 0;
-        FMB_CUDA(cudaMemcpyAsync(&h_ovf, ovf.p, sizeof h_ovf, cudaMemcpyDeviceToHost, st));
-        FMB_CUDA(cudaStreamSynchronize(st));
-        if (h_ovf) {                 // some walk is longer than the step field allows (or never reaches a sample)
-            ix->locrow.release();
-            ix->loc_step_bits = 0;
-        }
-        return FMB_OK;
-    }
-    if (getenv("FMB_NO_LOCBLOCKS") || !ix->dna || !ix->marks.p || ix->n_samples == 0 || !(ix->allowed_tables & FMB_TABLE_LOCBLOCK)) return FMB_OK;
+// combined 64-byte locate records of the DNA layout (needs occ table 0 and the marks)
+static int build_locblocks(fmb_index* ix) {
+    if (!ix->marks.p || ix->n_samples == 0 || !(ix->allowed_tables & FMB_TABLE_LOCBLOCK)) return FMB_OK;
     const uint64_t nblocks = ix->n / 64 + 1;
     cudaStream_t st = active_stream(ix);
     FMB_TRY(ix->locblocks.alloc(nblocks * 4));
     build_locblocks_kernel<<<grid_for(nblocks, 256), 256, 0, st>>>(ix->occ_dna[0].p, ix->marks.p, nblocks, ix->locblocks.p);
     FMB_CUDA(cudaGetLastError());
     FMB_CUDA(cudaStreamSynchronize(st));
-    // locate shortcut table: walk every row once.  The word packs sample index and step count; when they do not fit 32 bits (very
-    // sparse or irregular sampling) the table is dropped and locate keeps walking.  FMB_NO_LOCROW disables it.
-    if (!getenv("FMB_NO_LOCROW") && (ix->allowed_tables & FMB_TABLE_LOCROW)) {
-        uint32_t idx_bits = 1;
-        while (idx_bits < 32 && (uint64_t(1) << idx_bits) < ix->n_samples) ++idx_bits;
-        const uint32_t step_bits = 32 - idx_bits;
-        size_t free_b = 0, total_b = 0;
-        pool_trim();
-        FMB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-        if (step_bits >= 1 && (double)free_b > 4.0 * (double)ix->n * 1.5 + (double)(1u << 28)) {
-            FMB_TRY(ix->locrow.alloc(ix->n));
-            DevBuf<uint32_t> ovf;
-            FMB_TRY(ovf.alloc(1));
-            FMB_CUDA(cudaMemsetAsync(ovf.p, 0, sizeof(uint32_t), st));
-            int sms = 0;
-            FMB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ix->device));
-            ix->loc_step_bits = step_bits;
-            unsigned grid = (unsigned)std::min<uint64_t>(grid_for(ix->n * 2, 256), (uint64_t)sms * 8);
-            locrow_build_kernel<<<grid, 256, 0, st>>>(ix->view_dna(), step_bits, ix->locrow.p, ovf.p);
-            FMB_CUDA(cudaGetLastError());
-            uint32_t h_ovf = 0;
-            FMB_CUDA(cudaMemcpyAsync(&h_ovf, ovf.p, sizeof h_ovf, cudaMemcpyDeviceToHost, st));
-            FMB_CUDA(cudaStreamSynchronize(st));
-            if (h_ovf) {                 // some walk is longer than the step field allows
-                ix->locrow.release();
-                ix->loc_step_bits = 0;
-            }
-        }
+    return FMB_OK;
+}
+
+// locate shortcut table: walk every row once.  The word packs sample index and step count; when they do not fit 32 bits (very sparse
+// or irregular sampling), or some walk never reaches a sample, the table is dropped and locate keeps walking.  On the DNA layout the
+// walk reads the locate blocks: plan_tables allows LOCROW only together with LOCBLOCK, so build_locblocks has built them.
+static int build_locrow(fmb_index* ix) {
+    if (!ix->marks.p || ix->n_samples == 0 || !(ix->allowed_tables & FMB_TABLE_LOCROW)) return FMB_OK;
+    uint32_t idx_bits = 1;
+    while (idx_bits < 32 && (uint64_t(1) << idx_bits) < ix->n_samples) ++idx_bits;
+    const uint32_t step_bits = 32 - idx_bits;
+    size_t free_b = 0, total_b = 0;
+    pool_trim();
+    FMB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    if (step_bits < 1 || (double)free_b <= 4.0 * (double)ix->n * 1.5 + (double)(1u << 28)) return FMB_OK;
+    cudaStream_t st = active_stream(ix);
+    FMB_TRY(ix->locrow.alloc(ix->n));
+    DevBuf<uint32_t> ovf;
+    FMB_TRY(ovf.alloc(1));
+    FMB_CUDA(cudaMemsetAsync(ovf.p, 0, sizeof(uint32_t), st));
+    ix->loc_step_bits = step_bits;
+    if (ix->dna) {               // persistent grid
+        const unsigned grid = (unsigned)std::min<uint64_t>(grid_for(ix->n * 2, 256), (uint64_t)ix->sm_count * 8);
+        locrow_build_kernel<<<grid, 256, 0, st>>>(ix->view_dna(), step_bits, ix->locrow.p, ovf.p);
+    } else {                     // one thread per row
+        locrow_build_gen_kernel<<<grid_for(ix->n, 256), 256, 0, st>>>(ix->view_gen(), step_bits, ix->locrow.p, ovf.p);
+        note_launches(1);
+    }
+    FMB_CUDA(cudaGetLastError());
+    uint32_t h_ovf = 0;
+    FMB_CUDA(cudaMemcpyAsync(&h_ovf, ovf.p, sizeof h_ovf, cudaMemcpyDeviceToHost, st));
+    FMB_CUDA(cudaStreamSynchronize(st));
+    if (h_ovf) {
+        ix->locrow.release();
+        ix->loc_step_bits = 0;
     }
     return FMB_OK;
 }
 
-// Builds the two-symbol table of direction `dir` from the one-symbol table (needs C).  sigma <= 5 only.
-int build_occ2(fmb_index* ix, int dir) {
-    if (!(ix->allowed_tables & FMB_TABLE_PAIR)) return build_jump(ix, dir);       // image budget: no pair / k-mer table
+// Builds the two-symbol table and the k-mer table of direction 0 from the one-symbol table (needs C).  sigma <= 5 only.
+static int build_occ2(fmb_index* ix) {
+    if (!(ix->allowed_tables & FMB_TABLE_PAIR)) return FMB_OK;
     const uint64_t n = ix->n;
     const uint64_t nblocks = n / 128 + 1, nquarters = nblocks * 4;
     cudaStream_t st = active_stream(ix);
     auto v = ix->view_dna();
     DevBuf<uint8_t> codes;
     FMB_TRY(codes.alloc(n));
-    pair_codes_kernel<<<grid_for(n, 256), 256, 0, st>>>(v, dir, codes.p);
+    pair_codes_kernel<<<grid_for(n, 256), 256, 0, st>>>(v, 0, codes.p);
     FMB_CUDA(cudaGetLastError());
-    FMB_TRY(ix->occ2[dir].alloc(nblocks * 8));
+    FMB_TRY(ix->occ2.alloc(nblocks * 8));
     DevBuf<uint32_t> qcounts, scount;
     DevBuf<Cnt16> bcounts;
     FMB_TRY(qcounts.alloc(nquarters * 16));
     FMB_TRY(scount.alloc(nquarters + 1));
     FMB_TRY(bcounts.alloc(nblocks));
-    pack_pairs_kernel<<<grid_for(nquarters + 1, 256), 256, 0, st>>>(codes.p, n, nblocks, ix->occ2[dir].p, qcounts.p, scount.p);
+    pack_pairs_kernel<<<grid_for(nquarters + 1, 256), 256, 0, st>>>(codes.p, n, nblocks, ix->occ2.p, qcounts.p, scount.p);
     FMB_CUDA(cudaGetLastError());
     block_counts_kernel<<<grid_for(nblocks * 16, 256), 256, 0, st>>>(qcounts.p, nblocks, bcounts.p);
     FMB_CUDA(cudaGetLastError());
-    {
-        size_t tmp_bytes = 0;
-        FMB_CUDA(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, bcounts.p, bcounts.p, Cnt16Add{}, Cnt16{}, (int64_t)nblocks, st));
-        DevBuf<uint8_t> tmp;
-        FMB_TRY(tmp.alloc(tmp_bytes));
-        FMB_CUDA(cub::DeviceScan::ExclusiveScan(tmp.p, tmp_bytes, bcounts.p, bcounts.p, Cnt16Add{}, Cnt16{}, (int64_t)nblocks, st));
-    }
-    store_pair_counts_kernel<<<grid_for(nquarters, 256), 256, 0, st>>>(ix->occ2[dir].p, bcounts.p, nblocks);
+    FMB_TRY(exclusive_scan(bcounts.p, nblocks, Cnt16Add{}, Cnt16{}, st));
+    store_pair_counts_kernel<<<grid_for(nquarters, 256), 256, 0, st>>>(ix->occ2.p, bcounts.p, nblocks);
     FMB_CUDA(cudaGetLastError());
     FMB_TRY(exclusive_sum_u32(scount.p, scount.p, nquarters + 1, st));
     uint32_t ns = 0;
     FMB_CUDA(cudaMemcpy(&ns, scount.p + nquarters, sizeof ns, cudaMemcpyDeviceToHost));
-    FMB_TRY(ix->specials[dir].alloc((size_t)ns + 2));
-    FMB_CUDA(cudaMemsetAsync(ix->specials[dir].p, 0xFF, ((size_t)ns + 2) * sizeof(uint32_t), st));
+    FMB_TRY(ix->specials.alloc((size_t)ns + 2));
+    FMB_CUDA(cudaMemsetAsync(ix->specials.p, 0xFF, ((size_t)ns + 2) * sizeof(uint32_t), st));
     if (ns) {
-        scatter_specials_kernel<<<grid_for(nquarters, 256), 256, 0, st>>>(codes.p, n, nquarters, scount.p, ix->specials[dir].p);
+        scatter_specials_kernel<<<grid_for(nquarters, 256), 256, 0, st>>>(codes.p, n, nquarters, scount.p, ix->specials.p);
         FMB_CUDA(cudaGetLastError());
     }
-    ix->n_specials[dir] = ns;
-    FMB_CUDA(cudaMemcpyAsync(ix->special01[dir], ix->specials[dir].p, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    ix->n_specials = ns;
+    FMB_CUDA(cudaMemcpyAsync(ix->special01, ix->specials.p, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     DevBuf<uint32_t> c2;
     FMB_TRY(c2.alloc(16));
-    compute_C2_kernel<<<1, 32, 0, st>>>(v, dir, c2.p);
+    compute_C2_kernel<<<1, 32, 0, st>>>(v, 0, c2.p);
     FMB_CUDA(cudaGetLastError());
-    FMB_CUDA(cudaMemcpyAsync(ix->C2[dir], c2.p, 16 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    FMB_CUDA(cudaMemcpyAsync(ix->C2, c2.p, 16 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     FMB_CUDA(cudaStreamSynchronize(st));
-    if (dir == 0) {
-        // k-mer table: largest k <= 14 whose table (8 bytes per k-mer) stays below ~n bytes, i.e. 4^k <= n / 8
-        uint32_t k = 0;
-        while (k < 14 && (uint64_t(8) << (2 * (k + 1))) <= n) ++k;
-        const char* env = getenv("FMB_KMER_K");
-        if (env) k = (uint32_t)std::min<long>(14, std::max<long>(0, atol(env)));
-        ix->kmer_k = 0;
-        if (k >= 2) {
-            const uint64_t count = uint64_t(1) << (2 * k);
-            FMB_TRY(ix->kmer.alloc(count));
-            kmer_table_kernel<<<grid_for(count, 256), 256, 0, st>>>(v, k, count, ix->kmer.p);
-            FMB_CUDA(cudaGetLastError());
-            FMB_CUDA(cudaStreamSynchronize(st));
-            ix->kmer_k = k;
-        }
+    uint32_t k = dna_kmer_k(n);                          // k-mer table
+    const char* env = getenv("FMB_KMER_K");
+    if (env) k = (uint32_t)std::min<long>(14, std::max<long>(0, atol(env)));
+    ix->kmer_k = 0;
+    if (k >= 2) {
+        const uint64_t count = uint64_t(1) << (2 * k);
+        FMB_TRY(ix->kmer.alloc(count));
+        kmer_table_kernel<<<grid_for(count, 256), 256, 0, st>>>(v, k, count, ix->kmer.p);
+        FMB_CUDA(cudaGetLastError());
+        FMB_CUDA(cudaStreamSynchronize(st));
+        ix->kmer_k = k;
     }
-    FMB_TRY(build_jump(ix, dir));
     return FMB_OK;
 }
 
 // LF^16 jump table of direction `dir` (8 bytes per row) by four rounds of pointer doubling.  Skipped -- the search then
-// keeps taking two-symbol steps -- when the device cannot hold the two build buffers, or when FMB_NO_JUMP is set.
-int build_jump(fmb_index* ix, int dir) {
-    if (getenv("FMB_NO_JUMP")) return FMB_OK;
+// keeps taking two-symbol steps -- when the device cannot hold the two build buffers, or when the plan does not allow it.
+static int build_jump(fmb_index* ix, int dir) {
     if (ix->dna ? !(ix->allowed_tables & (dir ? FMB_TABLE_JUMP_REV : FMB_TABLE_JUMP)) : !(ix->allowed_tables & FMB_TABLE_JUMP4)) return FMB_OK;
     const uint64_t n = ix->n;
     size_t free_b = 0, total_b = 0;
-    FMB_CUDA(cudaMemGetInfo(&free_b, &total_b));
     pool_trim();
     FMB_CUDA(cudaMemGetInfo(&free_b, &total_b));
     if ((double)free_b < 2.0 * 8.0 * (double)n * 1.25 + (double)(1u << 28)) return FMB_OK;
@@ -642,9 +596,8 @@ int build_jump(fmb_index* ix, int dir) {
     }
     jump_init_kernel<<<grid_for(n, 256), 256, 0, st>>>(ix->view_dna(), dir, a.p);
     FMB_CUDA(cudaGetLastError());
-    // LF^4 entries (after the second round) are kept as well when memory allows: they serve the tails that are shorter than 16
-    // symbols (FMB_NO_JUMP4 disables them)
-    const bool want4 = !getenv("FMB_NO_JUMP4") && (ix->allowed_tables & FMB_TABLE_JUMP4) && (double)free_b > 3.0 * 8.0 * (double)n * 1.25 + (double)(size_t(24) << 30);
+    // LF^4 entries (after the second round) are kept as well when memory allows: they serve the tails shorter than 16 symbols
+    const bool want4 = (ix->allowed_tables & FMB_TABLE_JUMP4) && (double)free_b > 3.0 * 8.0 * (double)n * 1.25 + (double)(size_t(24) << 30);
     for (uint32_t shift = 2; shift <= 16; shift *= 2) {
         // direction 0 is compared with query symbols to the LEFT of the match (farthest symbol = lowest position = low bits),
         // direction 1 with symbols to the RIGHT (nearest symbol = lowest position = low bits): both equal the packed query order
@@ -663,9 +616,9 @@ int build_jump(fmb_index* ix, int dir) {
 
 // Merged LF^16 / LF^32 table of direction 0 (16 bytes per row instead of 8): exact search then covers 32 symbols of a single-row
 // interval per lookup.  Built after both LF^16 tables exist; skipped (the 8-byte table stays) when the device cannot hold the wide
-// copy next to the narrow one plus what the remaining tables need, or when FMB_NO_JUMP32 is set.
-int widen_jump0(fmb_index* ix) {
-    if (!ix->dna || !ix->jump[0].p || ix->jump_shift[0] || getenv("FMB_NO_JUMP32") || !(ix->allowed_tables & FMB_TABLE_JUMP32)) return FMB_OK;
+// copy next to the narrow one plus what the remaining tables need, or when the plan does not allow it.
+static int widen_jump0(fmb_index* ix) {
+    if (!ix->dna || !ix->jump[0].p || ix->jump_shift[0] || !(ix->allowed_tables & FMB_TABLE_JUMP32)) return FMB_OK;
     const uint64_t n = ix->n;
     size_t free_b = 0, total_b = 0;
     pool_trim();
@@ -684,6 +637,19 @@ int widen_jump0(fmb_index* ix) {
     ix->jump_shift[0] = 1;
     pool_trim();
     return FMB_OK;
+}
+
+int build_search_tables(fmb_index* ix) {
+    if (ix->dna) FMB_TRY(build_occ2(ix));
+    FMB_TRY(build_jump(ix, 0));
+    if (ix->bidirectional) FMB_TRY(build_jump(ix, 1));
+    FMB_TRY(widen_jump0(ix));
+    return build_bikmer(ix);
+}
+
+int build_locate_tables(fmb_index* ix) {
+    if (ix->dna) FMB_TRY(build_locblocks(ix));
+    return build_locrow(ix);
 }
 
 // sample tables from a device bitmap ((n+63)/64 words; rows >= n clear) and device sample arrays
@@ -801,15 +767,7 @@ int fmb_index_create_ex(fmb_index** out, int device, uint32_t sigma, uint64_t n,
     }
     int rc = compute_C(ix);
     if (rc) return fail(rc);
-    if (ix->dna) rc = build_occ2(ix, 0);
-    if (rc) return fail(rc);
-    if (!ix->dna) rc = build_jump(ix, 0);
-    if (rc) return fail(rc);
-    if (ix->bidirectional) rc = build_jump(ix, 1);
-    if (rc) return fail(rc);
-    rc = widen_jump0(ix);
-    if (rc) return fail(rc);
-    rc = build_bikmer(ix);
+    rc = build_search_tables(ix);
     if (rc) return fail(rc);
     {
         const uint64_t have = (n + 63) / 64;
@@ -826,7 +784,7 @@ int fmb_index_create_ex(fmb_index** out, int device, uint32_t sigma, uint64_t n,
         rc = build_marks_from_device(ix, d_bm.p, d_seq.p, d_pos.p, n_samples);
         if (rc) return fail(rc);
     }
-    rc = build_locblocks(ix);
+    rc = build_locate_tables(ix);
     if (rc) return fail(rc);
     *out = ix;
     pool_trim();
@@ -858,27 +816,17 @@ int fmb_index_replicate(const fmb_index* src, int device, fmb_index** out) {
         if (se != cudaSuccess) { set_error("fmb_index_replicate: %s", cudaGetErrorString(se)); return fail(FMB_ECUDA); }
     }
     int rc = FMB_OK;
-    for (int d = 0; d < 2 && !rc; ++d) {
-        if (!rc) rc = replicate_buf(ix->occ_dna[d], src->occ_dna[d], device, src->device, st);
-        if (!rc) rc = replicate_buf(ix->occ_gen[d], src->occ_gen[d], device, src->device, st);
-        if (!rc) rc = replicate_buf(ix->delim_rows[d], src->delim_rows[d], device, src->device, st);
-        if (!rc) rc = replicate_buf(ix->occ2[d], src->occ2[d], device, src->device, st);
-        if (!rc) rc = replicate_buf(ix->specials[d], src->specials[d], device, src->device, st);
-        if (!rc) rc = replicate_buf(ix->jump[d], src->jump[d], device, src->device, st);
-        if (!rc) rc = replicate_buf(ix->jump4[d], src->jump4[d], device, src->device, st);
-        ix->delim0[d] = src->delim0[d];
-        ix->n_specials[d] = src->n_specials[d];
-        ix->jump_shift[d] = src->jump_shift[d];
-        for (int i = 0; i < 2; ++i) ix->special01[d][i] = src->special01[d][i];
-        for (int i = 0; i < 16; ++i) ix->C2[d][i] = src->C2[d][i];
-    }
-    if (!rc) rc = replicate_buf(ix->marks, src->marks, device, src->device, st);
-    if (!rc) rc = replicate_buf(ix->samples, src->samples, device, src->device, st);
-    if (!rc) rc = replicate_buf(ix->locblocks, src->locblocks, device, src->device, st);
-    if (!rc) rc = replicate_buf(ix->locrow, src->locrow, device, src->device, st);
-    if (!rc) rc = replicate_buf(ix->kmer, src->kmer, device, src->device, st);
-    if (!rc) rc = replicate_buf(ix->bikmer, src->bikmer, device, src->device, st);
+    fmb_index::for_each_buffer(*ix, *src, [&](auto& to, const auto& from, bool replicated) {
+        if (!rc && replicated) rc = replicate_buf(to, from, device, src->device, st);
+    });
     if (rc) return fail(rc);
+    for (int d = 0; d < 2; ++d) {
+        ix->delim0[d] = src->delim0[d];
+        ix->jump_shift[d] = src->jump_shift[d];
+    }
+    ix->n_specials = src->n_specials;
+    for (int i = 0; i < 2; ++i) ix->special01[i] = src->special01[i];
+    for (int i = 0; i < 16; ++i) ix->C2[i] = src->C2[i];
     ix->gen_stride = src->gen_stride; ix->gen_planes = src->gen_planes;
     ix->n_delims = src->n_delims; ix->n_samples = src->n_samples;
     ix->loc_step_bits = src->loc_step_bits; ix->locate_mode = src->locate_mode; ix->exact_mode = src->exact_mode;
@@ -913,7 +861,7 @@ int fmb_index_get_info(const fmb_index* ix, fmb_index_info* info) {
     info->occ_block_rows = 64;
     info->device = ix->device;
     info->flags = (ix->first_symb ? 0u : FMB_INDEX_NO_DELIM) | (ix->reuse_rev ? FMB_INDEX_REUSE_REV : 0u);
-    info->tables = (ix->occ2[0].p ? FMB_TABLE_PAIR : 0) | (ix->kmer.p ? FMB_TABLE_KMER : 0) | (ix->jump[0].p ? FMB_TABLE_JUMP : 0) |
+    info->tables = (ix->occ2.p ? FMB_TABLE_PAIR : 0) | (ix->kmer.p ? FMB_TABLE_KMER : 0) | (ix->jump[0].p ? FMB_TABLE_JUMP : 0) |
                    (ix->jump[1].p ? FMB_TABLE_JUMP_REV : 0) | (ix->locblocks.p ? FMB_TABLE_LOCBLOCK : 0) | (ix->locrow.p ? FMB_TABLE_LOCROW : 0) |
                    (ix->bikmer.p ? FMB_TABLE_BIKMER : 0) | (ix->jump4[0].p ? FMB_TABLE_JUMP4 : 0) | (ix->jump_shift[0] ? FMB_TABLE_JUMP32 : 0);
     info->tables |= ix->anchor_pos.p ? FMB_TABLE_ANCHORS : 0;
@@ -1260,14 +1208,14 @@ int fmb_search_exact(const fmb_index* ix, const fmb_queries* q, fmb_results** ou
     DevBuf<unsigned long long> ctr;
     int rc;
     if ((rc = res->hits.alloc(nq)) || (rc = res->lens.alloc(nq + 1)) || (rc = ctr.alloc(8))) return fail(rc);
-    const bool two = ix->dna && ix->occ2[0].p && q->packed.p && ix->exact_mode != FMB_EXACT_ONE_SYMBOL;
-    if (ix->exact_mode == FMB_EXACT_TWO_SYMBOL && !ix->occ2[0].p) { set_error("index has no two-symbol table"); return fail(FMB_EUNSUPPORTED); }
+    const bool two = ix->dna && ix->occ2.p && q->packed.p && ix->exact_mode != FMB_EXACT_ONE_SYMBOL;
+    if (ix->exact_mode == FMB_EXACT_TWO_SYMBOL && !ix->occ2.p) { set_error("index has no two-symbol table"); return fail(FMB_EUNSUPPORTED); }
     cudaMemsetAsync(ctr.p, 0, 8 * sizeof(unsigned long long), st);
     cudaMemsetAsync(res->lens.p + nq, 0, sizeof(uint32_t), st);
     EventTimer tm(st);
     if (nq) {
         const uint32_t base = (uint32_t)q->qidx_base;
-        if (two) exact_search2_kernel<<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), ix->view_occ2(0), q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p);
+        if (two) exact_search2_kernel<<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), ix->view_occ2(), q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p);
         else FMB_DISPATCH(ix, v, exact_search_kernel<<<grid_for(nq, 256), 256, 0, st>>>(v, q->symbols.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p,
                                                                                               ix->dna ? nullptr : ix->jump4[0].p));
         note_launches(1);
@@ -1548,7 +1496,7 @@ int fmb_measure_gather(const fmb_index* ix, int table, uint64_t requests, double
     uint64_t bytes = 0;
     uint32_t per = 0, lanes = 0;
     switch (table) {
-        case FMB_GATHER_PAIR_LINE: tab = (const char*)ix->occ2[0].p; bytes = (ix->n / 128 + 1) * 128; per = 32; lanes = 4; break;
+        case FMB_GATHER_PAIR_LINE: tab = (const char*)ix->occ2.p; bytes = (ix->n / 128 + 1) * 128; per = 32; lanes = 4; break;
         case FMB_GATHER_OCC_BLOCK:
             if (ix->dna) { tab = (const char*)ix->occ_dna[0].p; bytes = (ix->n / 64 + 1) * 32; per = 32; lanes = 1; }
             else { tab = (const char*)ix->occ_gen[0].p; bytes = (ix->n / 64 + 1) * (uint64_t)ix->gen_stride; per = 32; lanes = ix->gen_stride / 32; }
@@ -1602,7 +1550,7 @@ int fmb_index_set_stream(fmb_index* ix, void* stream) {
 }
 int fmb_index_set_exact_mode(fmb_index* ix, int mode) {
     if (!ix || mode < 0 || mode > 2) { set_error("bad argument"); return FMB_EINVAL; }
-    if (mode == FMB_EXACT_TWO_SYMBOL && !ix->occ2[0].p) { set_error("index has no two-symbol table"); return FMB_EUNSUPPORTED; }
+    if (mode == FMB_EXACT_TWO_SYMBOL && !ix->occ2.p) { set_error("index has no two-symbol table"); return FMB_EUNSUPPORTED; }
     ix->exact_mode = mode;
     return FMB_OK;
 }

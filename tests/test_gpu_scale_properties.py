@@ -177,7 +177,7 @@ def test_sample_of_the_batch_matches_oracle(big, big_oracle, k, edit):
 
 
 def _bikmer_k(n):
-    """k of the bidirectional k-mer table of a DNA index of n rows (csrc/fmb_lib.cu build_bikmer): the largest k <= 14 with 8 * 4^k <= n"""
+    """k of the bidirectional k-mer table of a DNA index of n rows (csrc/fmb_lib.cu dna_kmer_k): the largest k <= 14 with 8 * 4^k <= n"""
     k = 0
     while k < 14 and 8 << (2 * (k + 1)) <= n:
         k += 1
