@@ -1216,8 +1216,10 @@ int fmb_search_exact(const fmb_index* ix, const fmb_queries* q, fmb_results** ou
     if (nq) {
         const uint32_t base = (uint32_t)q->qidx_base;
         if (two) exact_search2_kernel<<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), ix->view_occ2(), q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p);
+        // (the one-symbol mode counts the algorithmic work: a four-symbol jump that fails counts four steps where the walk stops at the
+        //  first mismatch, so that mode takes no jumps on the generic layout either)
         else FMB_DISPATCH(ix, v, exact_search_kernel<<<grid_for(nq, 256), 256, 0, st>>>(v, q->symbols.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p,
-                                                                                              ix->dna ? nullptr : ix->jump4[0].p));
+                                                                                              ix->dna || ix->exact_mode == FMB_EXACT_ONE_SYMBOL ? nullptr : ix->jump4[0].p));
         note_launches(1);
     }
     unsigned long long h_ctr[8] = {0};

@@ -319,7 +319,8 @@ int fmb_search_and_locate_parts(const fmb_index* const* parts, uint32_t n_index_
                                 fmb_loc32* out, uint64_t part_capacity, uint64_t* n_out /* n_index_parts */, fmb_stats* stats);
 
 /* Exact-search kernel selection.  FMB_EXACT_AUTO (default): two-symbol steps on the 128-byte pair table when the
- * index has one (sigma <= 5), else one-symbol steps.  FMB_EXACT_ONE_SYMBOL: the one-symbol kernel, which also fills
+ * index has one (sigma <= 5), else one-symbol steps (generic layout: four-symbol jumps once the interval is one row).
+ * FMB_EXACT_ONE_SYMBOL: the one-symbol kernel, one symbol per step on every layout, which also fills
  * the algorithmic work counters fmb_stats.extensions / occ_lookups (SURVEY.md §8d) -- the two-symbol kernel reports
  * fmb_stats.line_requests instead.  Results are identical in every mode. */
 #define FMB_EXACT_AUTO        0
