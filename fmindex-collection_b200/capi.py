@@ -16,7 +16,8 @@ LOC32_DTYPE = np.dtype([("qidx", "<u4"), ("seq", "<u4"), ("pos", "<u4"), ("e", "
 class IndexInfo(C.Structure):
     _fields_ = [("n", C.c_uint64), ("sigma", C.c_uint32), ("bidirectional", C.c_uint32), ("n_samples", C.c_uint64),
                 ("n_delims", C.c_uint64), ("device_bytes", C.c_uint64), ("occ_block_bytes", C.c_uint32),
-                ("occ_block_rows", C.c_uint32), ("device", C.c_int32), ("tables", C.c_uint32), ("flags", C.c_uint32)]
+                ("occ_block_rows", C.c_uint32), ("device", C.c_int32), ("tables", C.c_uint32), ("flags", C.c_uint32),
+                ("text_tables", C.c_uint32)]
 
 
 class Stats(C.Structure):

@@ -157,8 +157,18 @@ struct Occ2View {
     // jump_wide != 0: `jump` holds 16-byte entries {LF^16(row), symbols 1..16, LF^32(row), symbols 17..32} -- one lookup serves a
     // 16- or a 32-symbol jump (.z = 0xFFFFFFFF when one of symbols 17..32 is a delimiter)
     uint32_t jump_wide;
+    // text check (fmb_index::isa / text2 / seq_start_d; isa == nullptr: none): a single-row interval r with pos query symbols left
+    // lies at (seq, p) = samples[locrow[r] >> loc_step_bits] + the steps in the low bits; the read can only be the text
+    // [p - pos, p) of seq, compared with the query a 128-byte line (512 symbols) at a time, and its row is isa[seq_start[seq] + p - pos]
+    const uint32_t* isa;
+    const uint32_t* text32;      // 16 symbols per word, 32 words per 128-byte line
+    const uint32_t* seq_start;
+    const uint32_t* locrow;
+    const uint2* samples;
+    uint32_t loc_step_bits;
 };
 constexpr uint32_t kJumpInvalid = 0xFFFFFFFFu;
+constexpr uint32_t kNoSeq = 0xFFFFFFFFu;      // fmb_results::at of a hit the text check did not find
 
 struct Quarter {
     uint32_t cnt[4];

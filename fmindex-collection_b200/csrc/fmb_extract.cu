@@ -198,7 +198,9 @@ int check_index(const fmb_index* ix) {
     return use_device(ix->device);
 }
 
-// sequence lengths, offsets and delimiter rows (held under ix->anchor_mu)
+}  // namespace
+
+// sequence lengths, offsets and delimiter rows (held under ix->anchor_mu, or while the index is being built)
 int ensure_layout(const fmb_index* ix) {
     if (ix->layout_ready) return FMB_OK;
     const uint64_t nd = ix->n_delims;
@@ -248,6 +250,8 @@ int ensure_layout(const fmb_index* ix) {
     ix->layout_ready = true;
     return FMB_OK;
 }
+
+namespace {
 
 int ensure_anchors(const fmb_index* ix) {
     FMB_TRY(ensure_layout(ix));

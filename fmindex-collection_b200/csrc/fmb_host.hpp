@@ -116,6 +116,12 @@ struct fmb_index {
     fmb::DevBuf<uint4> bikmer;           // bidirectional k-mer table for scheme-search roots
     uint32_t bikmer_k = 0;
     int exact_mode = 0;                  // FMB_EXACT_*
+    // text check of exact search (FMB_TEXT_CHECK, built from the locate shortcut): isa[g] = row of text position g of s0 0 s1 0 ...,
+    // text2 = the text as 2-bit codes (symbol - 1), 16 per word, position g at bits 2 (g % 16) of word g / 16, and seq_start[s] = g of
+    // the first symbol of sequence s (+ n at the end).  text_rate = R when a row is sampled iff its position is a multiple of R
+    // (FMB_TEXT_LOCATE: the located row of a checked read needs pos % R LF steps), else 0.
+    fmb::DevBuf<uint32_t> isa, text2, seq_start_d;
+    uint32_t text_rate = 0;
     // optional tables this image is allowed to hold (FMB_TABLE_* bits), decided once by plan_tables (csrc/fmb_lib.cu) from the image
     // budget (fmb_set_image_budget / FMB_IMAGE_GB; default: everything the device can hold) and the FMB_NO_* knobs of its knob table
     uint32_t allowed_tables = 0xFFFFFFFFu;
@@ -156,6 +162,9 @@ struct fmb_index {
         f(a.locrow, b.locrow, true);
         f(a.kmer, b.kmer, true);
         f(a.bikmer, b.bikmer, true);
+        f(a.isa, b.isa, true);
+        f(a.text2, b.text2, true);
+        f(a.seq_start_d, b.seq_start_d, true);
         f(a.anchor_pos, b.anchor_pos, false);
         f(a.anchor_row, b.anchor_row, false);
     }
@@ -173,12 +182,14 @@ int use_device(int device);
 int new_index(fmb_index** out, int device, uint32_t sigma, uint64_t n, bool bidirectional, uint32_t flags);
 uint64_t image_budget();                                           // bytes, 0 = no limit
 uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples);     // the FMB_TABLE_* bits for ix->allowed_tables
+constexpr uint32_t kTableTextCheck = 1u << 16;                     // allowed_tables bit of the text check tables (FMB_TEXT_CHECK)
+int ensure_layout(const fmb_index* ix);                            // sequence lengths and starts (csrc/fmb_extract.cu)
 int build_occ_from_device_bwt(fmb_index* ix, int dir, const uint8_t* d_bwt);
 int compute_C(fmb_index* ix);
 // after compute_C: pair + k-mer tables (DNA layout), the LF jump tables of directions 0 and 1, the merged LF^32 entries and the
 // bidirectional k-mer table
 int build_search_tables(fmb_index* ix);
-// after the marks: locate blocks (DNA layout), then the locate shortcut
+// after the marks: locate blocks (DNA layout), the locate shortcut, then the text check tables built from it
 int build_locate_tables(fmb_index* ix);
 
 inline unsigned grid_for(uint64_t items, unsigned block) {
@@ -235,6 +246,7 @@ struct fmb_results {
     uint64_t slots = 0;               // records in `hits` (== count unless dense)
     bool dense = false;
     fmb::DevBuf<uint32_t> lens;       // dense results: len of every record (+ one trailing 0), the input of locate's scan
+    fmb::DevBuf<uint2> at;            // dense exact results with the text check: (seq, pos) of every checked hit, kNoSeq elsewhere
     uint64_t total_rows = UINT64_MAX; // sum of the interval lengths when the search kernel counted it, else unknown
     fmb_stats stats{};
 };

@@ -687,17 +687,21 @@ __global__ void __launch_bounds__(256) jump_widen_kernel(const uint2* __restrict
 // the 32-byte table (all lanes of the group read the same sector = one request).
 // Results are identical to exact_search_kernel: the final (lb, len) of a pattern does not depend on the step width.
 // 8 blocks per SM: 32 registers, 2048 resident threads per SM.
+// Text check (Occ2View::isa): a single-row interval with at least kTextCheckMin symbols left is decided on the text instead of the LF
+// jumps; out_at (may be nullptr) receives the (seq, pos) of such hits for locate, kNoSeq for every other query.
 // ---------------------------------------------------------------------------------------------------------
+constexpr uint32_t kTextCheckMin = 16;
 __global__ void __launch_bounds__(256, 8) exact_search2_kernel(const __grid_constant__ IndexView<OccDna> ix, const __grid_constant__ Occ2View o2,
                                                                   const uint8_t* __restrict__ qsym, const uint32_t* __restrict__ qpk,
                                                                   const uint8_t* __restrict__ qflags, const uint64_t* __restrict__ qoff, uint32_t nq,
                                                                   uint32_t qidx_base, HitRec* __restrict__ out_hits, uint32_t* __restrict__ out_len,
-                                                                  unsigned long long* __restrict__ counters) {
+                                                                  uint2* __restrict__ out_at, unsigned long long* __restrict__ counters) {
     const uint32_t q = (uint32_t)((blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) >> 2);      // 4 lanes per query: the thread index may exceed 32 bits
     const uint32_t sub = threadIdx.x & 3;
     const uint32_t gmask = 0xFu << (threadIdx.x & 28);
     uint32_t lines = 0, found = 0;
     unsigned long long rows = 0;
+    bool checked = false;
     if (q < nq) {
         const uint64_t off = qoff[q];
         const uint32_t L = (uint32_t)(qoff[q + 1] - off);
@@ -735,6 +739,35 @@ __global__ void __launch_bounds__(256, 8) exact_search2_kernel(const __grid_cons
                 lines += 1;
             }
             while (pos > 0 && len > 0) {
+                if (len == 1 && pos >= kTextCheckMin && o2.isa) {
+                    // single row with pos symbols left: where the row sits in the text decides the rest (Occ2View::isa).  Every lane
+                    // issues the same single lookups (one request each); each lane compares one 32-byte quarter of a text line.
+                    const uint32_t w = __ldg(o2.locrow + lb);
+                    const uint2 smp = __ldg(o2.samples + (w >> o2.loc_step_bits));
+                    const uint32_t p = smp.y + (w & ((1u << o2.loc_step_bits) - 1u));
+                    lines += 2;
+                    if (p < pos) { len = 0; break; }             // the read would start before its sequence
+                    const uint32_t g0 = __ldg(o2.seq_start + smp.x) + (p - pos);
+                    lines += 1;
+                    if (out_at && sub == 3) out_at[q] = make_uint2(smp.x, p - pos);      // replaced by kNoSeq below on a mismatch
+                    // lane `sub` compares the read's words sub, sub + 4, ... (symbols [16 j, 16 j + 16)) with the text at g0 + 16 j: the
+                    // group's four lanes read four consecutive text words per step, within one or two 128-byte lines
+                    uint32_t bad = 0;
+                    for (uint32_t j = sub; 16 * j < pos; j += 4) {
+                        const uint32_t x = g0 + 16 * j, cnt = min(16u, pos - 16 * j);
+                        const uint32_t t = __funnelshift_r(__ldg(o2.text32 + (x >> 4)), __ldg(o2.text32 + (x >> 4) + 1), 2 * (x & 15));
+                        const uint32_t m = cnt >= 16 ? 0xFFFFFFFFu : (1u << (2 * cnt)) - 1u;
+                        bad |= (t ^ field(16 * j, 32)) & m;
+                    }
+                    bad |= __shfl_xor_sync(gmask, bad, 1);
+                    bad |= __shfl_xor_sync(gmask, bad, 2);
+                    lines += ((g0 + pos - 1) >> 9) - (g0 >> 9) + 1;
+                    if (bad) { len = 0; break; }
+                    lb = __ldg(o2.isa + g0);
+                    lines += 1;
+                    checked = true;
+                    break;
+                }
                 if (len == 1 && pos >= 16 && o2.jump) {
                     // single-row interval: 16 symbols per lookup through the LF^16 jump table -- or 32 when the table holds the merged
                     // 16-byte entries and the next 32 symbols stay inside one sequence
@@ -809,7 +842,10 @@ __global__ void __launch_bounds__(256, 8) exact_search2_kernel(const __grid_cons
             if (sub == 0) rec[0] = make_uint2(q + qidx_base, lb);           // qidx, lb
             else if (sub == 1) rec[1] = make_uint2(0u, len);                 // lb_rev, len
             else if (sub == 2) rec[2] = make_uint2(L, 0u);                   // steps, e
-            else out_len[q] = len;
+            else {
+                out_len[q] = len;
+                if (out_at && !checked) out_at[q] = make_uint2(kNoSeq, 0u);
+            }
         }
         if (sub == 0) {
             found = len ? 1u : 0u;
@@ -1048,9 +1084,46 @@ __global__ void __launch_bounds__(256) locrow_build_gen_kernel(const __grid_cons
     }
 }
 
+// at (may be nullptr): (seq, pos) per record found by the text check of exact search (kNoSeq: not checked); with text-regular sampling
+// at rate `rate` such a row needs pos % rate LF steps and no index access
+// Text check tables (fmb_index::isa / text2), one thread per row: (seq, pos) of the row from the locate shortcut, g = start[seq] + pos;
+// isa[g] = row, and BWT[row] is the symbol at g - 1 (a delimiter when pos == 0: those positions keep code 0, no read window reaches
+// them).  flags[0] = a row outside its sequence, flags[1] = the largest LF step count of any row.
+__global__ void __launch_bounds__(256) text_tables_kernel(const __grid_constant__ IndexView<OccDna> ix, const uint32_t* __restrict__ start, uint32_t nseq,
+                                                          uint32_t* __restrict__ isa, uint32_t* __restrict__ text, uint32_t* __restrict__ flags) {
+    const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    uint32_t steps = 0;
+    if (r < ix.n) {
+        const uint32_t w = __ldg(ix.locrow + r);
+        steps = w & ((1u << ix.loc_step_bits) - 1u);
+        const uint2 s = __ldg(ix.samples + (w >> ix.loc_step_bits));
+        const uint32_t p = s.y + steps;
+        if (s.x >= nseq || p >= __ldg(start + s.x + 1) - __ldg(start + s.x)) {
+            atomicOr(flags, 1u);
+        } else {
+            const uint32_t g = __ldg(start + s.x) + p;
+            isa[g] = (uint32_t)r;
+            if (p) {
+                const DnaBlock b = ix.occ[0].load((uint32_t)(r >> 6), 0);
+                const uint32_t c = ix.occ[0].symbol(b, (row_t)r);
+                atomicOr(text + ((g - 1) >> 4), ((c - 1) & 3u) << (2 * ((g - 1) & 15)));
+            }
+        }
+    }
+    steps = __reduce_max_sync(0xFFFFFFFFu, steps);
+    if ((threadIdx.x & 31) == 0 && steps) atomicMax(flags + 1, steps);
+}
+// text-regular sampling at rate R = 1 + the largest step count: every sample at a multiple of R (then the step count of every row is
+// pos % R: its sample is the one multiple of R in (pos - R, pos])
+__global__ void __launch_bounds__(256) sample_rate_kernel(const uint2* __restrict__ samples, uint64_t count, uint32_t rate, uint32_t* __restrict__ bad) {
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i < count && samples[i].y % rate) atomicOr(bad, 1u);
+}
+
 template <class OCC>
 __global__ void __launch_bounds__(256) locate_shortcut_kernel(const __grid_constant__ IndexView<OCC> ix, const HitRec* __restrict__ hits,
                                                               const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,
+                                                              const uint2* __restrict__ at, uint32_t rate,
                                                               LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
     uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t steps = 0;
@@ -1061,12 +1134,19 @@ __global__ void __launch_bounds__(256) locate_shortcut_kernel(const __grid_const
             if (__ldg(starts + mid) <= t) lo = mid; else hi = mid;
         }
         const HitRec* h = hits + lo;
-        const row_t row = __ldg(&h->lb) + (single ? 0u : t - __ldg(starts + lo));
-        const uint32_t w = __ldg(ix.locrow + row);
-        steps = w & ((1u << ix.loc_step_bits) - 1u);
-        const uint2 sample = __ldg(ix.samples + (w >> ix.loc_step_bits));
         LocRec r;
-        r.qidx = __ldg(&h->qidx); r.seq = sample.x; r.pos = sample.y + steps; r.e = __ldg(&h->e);
+        r.qidx = __ldg(&h->qidx); r.e = __ldg(&h->e);
+        const uint2 a = at ? __ldg(at + lo) : make_uint2(kNoSeq, 0u);      // a checked hit is a single row
+        if (a.x != kNoSeq) {
+            steps = a.y % rate;
+            r.seq = a.x; r.pos = a.y;
+        } else {
+            const row_t row = __ldg(&h->lb) + (single ? 0u : t - __ldg(starts + lo));
+            const uint32_t w = __ldg(ix.locrow + row);
+            steps = w & ((1u << ix.loc_step_bits) - 1u);
+            const uint2 sample = __ldg(ix.samples + (w >> ix.loc_step_bits));
+            r.seq = sample.x; r.pos = sample.y + steps;
+        }
         out[t] = r;
     }
     // the LF steps the walk WOULD take: the algorithmic work of SURVEY.md §8d stays reported

@@ -240,6 +240,12 @@ fmb::Occ2View fmb_index::view_occ2() const {
     v.jump4 = jump4[0].p;
     v.kmer = kmer.p;
     v.kmer_k = kmer_k;
+    v.isa = isa.p;
+    v.text32 = text2.p;
+    v.seq_start = seq_start_d.p;
+    v.locrow = locrow.p;
+    v.samples = samples.p;
+    v.loc_step_bits = loc_step_bits;
     return v;
 }
 
@@ -259,7 +265,8 @@ namespace fmb {
 // the tables are admitted in the order of what they buy per byte (measured: profiles/r02_image_budget_curve.json):
 //   pair table + k-mer table (exact search: two symbols per line, the first 14 symbols in one lookup), locate blocks,
 //   LF^16 table of direction 0 (sixteen symbols per lookup once an interval is a single row), LF^16 of direction 1 (text windows of
-//   the k-error searches in both directions), bidirectional k-mer table, locate shortcut, merged LF^32 entries, LF^4 tables.
+//   the k-error searches in both directions), bidirectional k-mer table, locate shortcut, merged LF^32 entries, LF^4 tables, text check
+//   tables (ISA + 2-bit text: exact-search reads decided on the text; last because they serve exact search alone).
 // DNA layout, both k-mer tables: largest k <= 14 with 8 * 4^k <= n (the exact-search table, 8 bytes per k-mer, stays below ~n bytes)
 static uint32_t dna_kmer_k(uint64_t n) {
     uint32_t k = 0;
@@ -304,6 +311,7 @@ static uint32_t budget_tables(const fmb_index* ix, uint64_t n_samples) {
         if (allowed & FMB_TABLE_LOCBLOCK) admit(FMB_TABLE_LOCROW, 4 * n);
         if (j0) admit(FMB_TABLE_JUMP32, 8 * n);
         if (j0) admit(FMB_TABLE_JUMP4, 8 * n * (j1 ? 2 : 1));
+        if (allowed & FMB_TABLE_LOCROW) admit(kTableTextCheck, 4.25 * n);
     } else {
         admit(FMB_TABLE_JUMP4, 8 * n * (ix->bidirectional ? 2 : 1));      // generic layout: byte-symbol LF^4 tables ...
         admit(FMB_TABLE_LOCROW, 4 * n);                                    // ... the locate shortcut ...
@@ -325,6 +333,8 @@ static uint32_t budget_tables(const fmb_index* ix, uint64_t n_samples) {
 //   FMB_NO_BIKMER      BIKMER                                           BIKMER
 //   FMB_NO_LOCBLOCKS   LOCBLOCK, LOCROW (the shortcut walks the blocks) -
 //   FMB_NO_LOCROW      LOCROW                                           LOCROW
+//   FMB_NO_TEXTCHECK   the text check tables (kTableTextCheck)          -
+// (the text check tables are built from the locate shortcut: without LOCROW there are none)
 // FMB_KMER_K (build_occ2) sizes the exact-search k-mer table; FMB_KMER_K=0 leaves it out.
 uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
     static const struct { const char* name; uint32_t dna, gen; } knobs[] = {
@@ -334,6 +344,7 @@ uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
         {"FMB_NO_BIKMER", FMB_TABLE_BIKMER, FMB_TABLE_BIKMER},
         {"FMB_NO_LOCBLOCKS", FMB_TABLE_LOCBLOCK | FMB_TABLE_LOCROW, 0},
         {"FMB_NO_LOCROW", FMB_TABLE_LOCROW, FMB_TABLE_LOCROW},
+        {"FMB_NO_TEXTCHECK", kTableTextCheck, 0},
     };
     uint32_t allowed = budget_tables(ix, n_samples);
     for (const auto& k : knobs)
@@ -647,9 +658,54 @@ int build_search_tables(fmb_index* ix) {
     return build_bikmer(ix);
 }
 
+// Text check tables of exact search (DNA layout): ISA (4 bytes per row), the text as 2-bit codes and the sequence starts, built from
+// the locate shortcut (every row's text position).  Skipped without the shortcut, when the plan does not allow them, when the device
+// cannot hold them or when the samples do not describe a collection (the search then keeps its LF jumps).  text_rate is set when the
+// sampling is text-regular, the condition under which locate can report the step counts of the rows the check finds.
+static int build_text_check(fmb_index* ix) {
+    if (!ix->dna || !ix->locrow.p || !(ix->allowed_tables & kTableTextCheck)) return FMB_OK;
+    const uint64_t n = ix->n, words = (n / 512 + 2) * 32;       // whole 128-byte lines and one more
+    size_t free_b = 0, total_b = 0;
+    pool_trim();
+    FMB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    if ((double)free_b <= 4.25 * (double)n * 1.1 + (double)(size_t(1) << 30)) return FMB_OK;
+    if (ensure_layout(ix) != FMB_OK) return FMB_OK;
+    const uint64_t nseq = ix->seq_start.size();
+    std::vector<uint32_t> h_start(nseq + 1);
+    for (uint64_t s = 0; s < nseq; ++s) h_start[s] = (uint32_t)ix->seq_start[s];
+    h_start[nseq] = (uint32_t)n;
+    cudaStream_t st = active_stream(ix);
+    DevBuf<uint32_t> start, isa, text, flags;
+    FMB_TRY(start.alloc(nseq + 1));
+    FMB_TRY(isa.alloc(n));
+    FMB_TRY(text.alloc(words));
+    FMB_TRY(flags.alloc(3));
+    FMB_CUDA(cudaMemcpyAsync(start.p, h_start.data(), (nseq + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    FMB_CUDA(cudaMemsetAsync(text.p, 0, words * sizeof(uint32_t), st));
+    FMB_CUDA(cudaMemsetAsync(flags.p, 0, 3 * sizeof(uint32_t), st));
+    text_tables_kernel<<<grid_for(n, 256), 256, 0, st>>>(ix->view_dna(), start.p, (uint32_t)nseq, isa.p, text.p, flags.p);
+    FMB_CUDA(cudaGetLastError());
+    uint32_t h_flags[3] = {0, 0, 0};
+    FMB_CUDA(cudaMemcpyAsync(h_flags, flags.p, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    FMB_CUDA(cudaStreamSynchronize(st));
+    if (h_flags[0]) return FMB_OK;
+    const uint32_t rate = h_flags[1] + 1;
+    sample_rate_kernel<<<grid_for(ix->n_samples, 256), 256, 0, st>>>(ix->samples.p, ix->n_samples, rate, flags.p + 2);
+    FMB_CUDA(cudaGetLastError());
+    FMB_CUDA(cudaMemcpyAsync(h_flags + 2, flags.p + 2, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    FMB_CUDA(cudaStreamSynchronize(st));
+    note_launches(2);
+    ix->isa = std::move(isa);
+    ix->text2 = std::move(text);
+    ix->seq_start_d = std::move(start);
+    ix->text_rate = h_flags[2] ? 0u : rate;
+    return FMB_OK;
+}
+
 int build_locate_tables(fmb_index* ix) {
     if (ix->dna) FMB_TRY(build_locblocks(ix));
-    return build_locrow(ix);
+    FMB_TRY(build_locrow(ix));
+    return build_text_check(ix);
 }
 
 // sample tables from a device bitmap ((n+63)/64 words; rows >= n clear) and device sample arrays
@@ -830,6 +886,7 @@ int fmb_index_replicate(const fmb_index* src, int device, fmb_index** out) {
     ix->gen_stride = src->gen_stride; ix->gen_planes = src->gen_planes;
     ix->n_delims = src->n_delims; ix->n_samples = src->n_samples;
     ix->loc_step_bits = src->loc_step_bits; ix->locate_mode = src->locate_mode; ix->exact_mode = src->exact_mode;
+    ix->text_rate = src->text_rate;
     ix->kmer_k = src->kmer_k; ix->bikmer_k = src->bikmer_k;
     for (uint32_t s = 0; s <= src->sigma; ++s) ix->C[s] = src->C[s];
     cudaError_t e = cudaStreamSynchronize(st);
@@ -865,6 +922,7 @@ int fmb_index_get_info(const fmb_index* ix, fmb_index_info* info) {
                    (ix->jump[1].p ? FMB_TABLE_JUMP_REV : 0) | (ix->locblocks.p ? FMB_TABLE_LOCBLOCK : 0) | (ix->locrow.p ? FMB_TABLE_LOCROW : 0) |
                    (ix->bikmer.p ? FMB_TABLE_BIKMER : 0) | (ix->jump4[0].p ? FMB_TABLE_JUMP4 : 0) | (ix->jump_shift[0] ? FMB_TABLE_JUMP32 : 0);
     info->tables |= ix->anchor_pos.p ? FMB_TABLE_ANCHORS : 0;
+    info->text_tables = (ix->isa.p ? FMB_TEXT_CHECK : 0u) | (ix->isa.p && ix->text_rate ? FMB_TEXT_LOCATE : 0u);
     return FMB_OK;
 }
 
@@ -1209,13 +1267,19 @@ int fmb_search_exact(const fmb_index* ix, const fmb_queries* q, fmb_results** ou
     int rc;
     if ((rc = res->hits.alloc(nq)) || (rc = res->lens.alloc(nq + 1)) || (rc = ctr.alloc(8))) return fail(rc);
     const bool two = ix->dna && ix->occ2.p && q->packed.p && ix->exact_mode != FMB_EXACT_ONE_SYMBOL;
+    Occ2View o2 = ix->view_occ2();
+    if (ix->exact_mode == FMB_EXACT_NO_TEXT) o2.isa = nullptr;
+    // (seq, pos) of the hits the text check finds, for locate: only written when locate can use them
+    const bool want_at = two && o2.isa && ix->text_rate && nq;
+    if (want_at && (rc = res->at.alloc(nq))) return fail(rc);
     if (ix->exact_mode == FMB_EXACT_TWO_SYMBOL && !ix->occ2.p) { set_error("index has no two-symbol table"); return fail(FMB_EUNSUPPORTED); }
     cudaMemsetAsync(ctr.p, 0, 8 * sizeof(unsigned long long), st);
     cudaMemsetAsync(res->lens.p + nq, 0, sizeof(uint32_t), st);
     EventTimer tm(st);
     if (nq) {
         const uint32_t base = (uint32_t)q->qidx_base;
-        if (two) exact_search2_kernel<<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), ix->view_occ2(), q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p);
+        if (two) exact_search2_kernel<<<grid_for(nq * 4, 256), 256, 0, st>>>(ix->view_dna(), o2, q->symbols.p, q->packed.p, q->flags.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p,
+                                                                             want_at ? res->at.p : nullptr, ctr.p);
         // (the one-symbol mode counts the algorithmic work: a four-symbol jump that fails counts four steps where the walk stops at the
         //  first mismatch, so that mode takes no jumps on the generic layout either)
         else FMB_DISPATCH(ix, v, exact_search_kernel<<<grid_for(nq, 256), 256, 0, st>>>(v, q->symbols.p, q->offsets.p, (uint32_t)nq, base, res->hits.p, res->lens.p, ctr.p,
@@ -1304,7 +1368,9 @@ int fmb_locate(const fmb_index* ix, const fmb_results* hits, fmb_results** out) 
     if (total) {
         cudaEventRecord(ev_m0, st);
         if (ix->locrow.p && ix->locate_mode != FMB_LOCATE_WALK) {
-            FMB_DISPATCH(ix, v, locate_shortcut_kernel<<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, res->locs.p, ctr.p));
+            const uint2* at = hits->dense && ix->text_rate ? hits->at.p : nullptr;
+            FMB_DISPATCH(ix, v, locate_shortcut_kernel<<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, at, ix->text_rate,
+                                                                                             res->locs.p, ctr.p));
         } else if (ix->dna && ix->locblocks.p) {
             auto v = ix->view_dna();
             // persistent grid: every SM full of lane pairs (8 blocks x 256 threads), rows handed out with a grid stride
@@ -1551,8 +1617,8 @@ int fmb_index_set_stream(fmb_index* ix, void* stream) {
     return FMB_OK;
 }
 int fmb_index_set_exact_mode(fmb_index* ix, int mode) {
-    if (!ix || mode < 0 || mode > 2) { set_error("bad argument"); return FMB_EINVAL; }
-    if (mode == FMB_EXACT_TWO_SYMBOL && !ix->occ2.p) { set_error("index has no two-symbol table"); return FMB_EUNSUPPORTED; }
+    if (!ix || mode < 0 || mode > 3) { set_error("bad argument"); return FMB_EINVAL; }
+    if ((mode == FMB_EXACT_TWO_SYMBOL || mode == FMB_EXACT_NO_TEXT) && !ix->occ2.p) { set_error("index has no two-symbol table"); return FMB_EUNSUPPORTED; }
     ix->exact_mode = mode;
     return FMB_OK;
 }

@@ -68,6 +68,7 @@ typedef struct {
     int32_t  device;
     uint32_t tables;           /* optional accelerating tables the image holds, FMB_TABLE_* bits  */
     uint32_t flags;            /* FMB_INDEX_* variant bits                                  */
+    uint32_t text_tables;      /* text check tables of exact search, FMB_TEXT_* bits        */
 } fmb_index_info;
 #define FMB_TABLE_PAIR     1u   /* two-symbol pair table (128-byte lines)          */
 #define FMB_TABLE_KMER     2u   /* k-mer interval table                            */
@@ -79,6 +80,10 @@ typedef struct {
 #define FMB_TABLE_JUMP4    128u /* LF^4 jump tables (tails shorter than 16 symbols) */
 #define FMB_TABLE_JUMP32   256u /* direction 0 holds merged LF^16 / LF^32 entries (32 symbols per lookup in exact search) */
 #define FMB_TABLE_ANCHORS  512u /* anchor table of text extraction (built on the first extraction call)                  */
+/* fmb_index_info.text_tables (sigma <= 5 with delimiter, needs the locate shortcut): once the interval of an exact search is one row,
+ * the rest of the read is compared with the text at that row's position and the final row is read from the inverse suffix array */
+#define FMB_TEXT_CHECK     1u   /* inverse suffix array (4 bytes per row) + 2-bit text + sequence starts                 */
+#define FMB_TEXT_LOCATE    2u   /* text-regular sampling: locate takes the rows the text check found (no index access)   */
 
 /* work counters of the last search/locate call on a result set (device-side counting, optional) */
 typedef struct {
@@ -322,10 +327,12 @@ int fmb_search_and_locate_parts(const fmb_index* const* parts, uint32_t n_index_
  * index has one (sigma <= 5), else one-symbol steps (generic layout: four-symbol jumps once the interval is one row).
  * FMB_EXACT_ONE_SYMBOL: the one-symbol kernel, one symbol per step on every layout, which also fills
  * the algorithmic work counters fmb_stats.extensions / occ_lookups (SURVEY.md §8d) -- the two-symbol kernel reports
- * fmb_stats.line_requests instead.  Results are identical in every mode. */
+ * fmb_stats.line_requests instead.  FMB_EXACT_NO_TEXT: the two-symbol kernel without the text check of single-row intervals
+ * (FMB_TEXT_CHECK): the LF^16 / LF^32 / LF^4 jumps walk the rest of the read.  Results are identical in every mode. */
 #define FMB_EXACT_AUTO        0
 #define FMB_EXACT_ONE_SYMBOL  1
 #define FMB_EXACT_TWO_SYMBOL  2
+#define FMB_EXACT_NO_TEXT     3
 int  fmb_index_set_exact_mode(fmb_index* ix, int mode);
 
 /* Locate kernel selection.  FMB_LOCATE_AUTO (default): the locate shortcut table when the index has one (per row the
