@@ -11,6 +11,9 @@ _LIB = None
 HIT_DTYPE = np.dtype([("qidx", "<u8"), ("lb", "<u8"), ("lb_rev", "<u8"), ("len", "<u8"), ("steps", "<u8"), ("e", "<u8")])
 LOC_DTYPE = np.dtype([("qidx", "<u8"), ("seq", "<u8"), ("pos", "<u8"), ("e", "<u8")])
 LOC32_DTYPE = np.dtype([("qidx", "<u4"), ("seq", "<u4"), ("pos", "<u4"), ("e", "<u4")])
+SMEM_DTYPE = np.dtype([("qidx", "<u8"), ("begin", "<u8"), ("end", "<u8"), ("lb", "<u8"), ("len", "<u8")])
+SMEM_LOC_DTYPE = np.dtype([("qidx", "<u8"), ("begin", "<u8"), ("end", "<u8"), ("seq", "<u8"), ("pos", "<u8")])
+UINT64_MAX = (1 << 64) - 1
 
 
 class IndexInfo(C.Structure):
@@ -44,6 +47,7 @@ SYMBOLS = [
     "fmb_cursor_extend", "fmb_cursor_extend_all",
     "fmb_queries_upload", "fmb_queries_upload_revcomp", "fmb_queries_upload_packed", "fmb_pack_symbols", "fmb_queries_destroy", "fmb_queries_count",
     "fmb_search_exact", "fmb_search_scheme", "fmb_search_scheme_n", "fmb_search_scheme_pseudo", "fmb_search_backtracking", "fmb_locate", "fmb_locate_rows", "fmb_sample_value",
+    "fmb_search_smems", "fmb_locate_smems", "fmb_results_fetch_smems", "fmb_results_fetch_smem_locs",
     "fmb_results_count", "fmb_results_kind", "fmb_results_fetch_hits", "fmb_results_fetch_locs", "fmb_results_fetch_locs32",
     "fmb_results_get_stats", "fmb_results_destroy",
     "fmb_search_and_locate", "fmb_search_and_locate_packed", "fmb_search_and_locate_multi", "fmb_search_and_locate_parts", "fmb_index_replicate", "fmb_index_save", "fmb_index_load", "fmb_checksum64",
@@ -289,6 +293,19 @@ class Index:
         _check(lib().fmb_locate(self.h, hits.h, C.byref(r)))
         return Results(r)
 
+    def search_smems(self, queries, min_len=1):
+        """super-maximal exact matches of every query (fmb_search_smems): the stretches of a query that occur in one sequence of the
+        collection and cannot be extended on either side, at least min_len symbols long, ordered by qidx, then begin"""
+        r = C.c_void_p()
+        _check(lib().fmb_search_smems(self.h, queries.h, C.c_uint32(min_len), C.byref(r)))
+        return Results(r)
+
+    def locate_smems(self, results, max_occ=None):
+        """the first min(len, max_occ) rows of every SMEM's interval, located (fmb_locate_smems; max_occ None: every row)"""
+        r = C.c_void_p()
+        _check(lib().fmb_locate_smems(self.h, results.h, C.c_uint64(UINT64_MAX if max_occ is None else int(max_occ)), C.byref(r)))
+        return Results(r)
+
     def locate_rows(self, rows):
         """index.locate(row) for many rows: (seq, pos, steps) arrays"""
         rows = _u64(rows)
@@ -501,6 +518,18 @@ class Results:
     def locs32(self):
         out = np.zeros(len(self), dtype=LOC32_DTYPE)
         _check(lib().fmb_results_fetch_locs32(self.h, _ptr(out), C.c_uint64(out.size)))
+        return out
+
+    def smems(self):
+        """SMEM records (qidx, begin, end, lb, len) of fmb_search_smems"""
+        out = np.zeros(len(self), dtype=SMEM_DTYPE)
+        _check(lib().fmb_results_fetch_smems(self.h, _ptr(out), C.c_uint64(out.size)))
+        return out
+
+    def smem_locs(self):
+        """located SMEM rows (qidx, begin, end, seq, pos) of fmb_locate_smems"""
+        out = np.zeros(len(self), dtype=SMEM_LOC_DTYPE)
+        _check(lib().fmb_results_fetch_smem_locs(self.h, _ptr(out), C.c_uint64(out.size)))
         return out
 
     def close(self):

@@ -74,6 +74,9 @@ struct HitRec {
     uint32_t qidx, lb, lb_rev, len, steps, e;
 };
 typedef fmb_loc32 LocRec;
+struct SmemRec {                  // fmb_smem with 32-bit fields
+    uint32_t qidx, begin, end, lb, len;
+};
 
 }  // namespace fmb
 
@@ -237,16 +240,18 @@ struct fmb_queries {
 
 struct fmb_results {
     int device = 0;
-    int kind = 0;                     // 0 = hits, 1 = located rows
-    uint64_t count = 0;               // hits (cursors with a non-empty interval) / located rows
+    int kind = 0;                     // 0 = hits, 1 = located rows, 2 = SMEMs, 3 = located rows of SMEMs
+    uint64_t count = 0;               // hits (cursors with a non-empty interval) / located rows / SMEMs
     fmb::DevBuf<fmb::HitRec> hits;
-    fmb::DevBuf<fmb::LocRec> locs;
+    fmb::DevBuf<fmb::LocRec> locs;    // kind 3: qidx holds the number of the SMEM record the row belongs to
+    fmb::DevBuf<fmb::SmemRec> smems;  // kinds 2 and 3 (csrc/fmb_smem.cu); kind 2 also fills `at` per record
     // exact search leaves its hits DENSE: one record per query (`slots` of them, len == 0 for queries without hit) plus the
     // interval lengths as a separate array -- locate works on that directly, the records are compacted only when they are fetched
     uint64_t slots = 0;               // records in `hits` (== count unless dense)
     bool dense = false;
     fmb::DevBuf<uint32_t> lens;       // dense results: len of every record (+ one trailing 0), the input of locate's scan
     fmb::DevBuf<uint2> at;            // dense exact results with the text check: (seq, pos) of every checked hit, kNoSeq elsewhere
+                                      // (SMEMs: of every record the text path found)
     uint64_t total_rows = UINT64_MAX; // sum of the interval lengths when the search kernel counted it, else unknown
     fmb_stats stats{};
 };

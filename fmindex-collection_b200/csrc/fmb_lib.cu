@@ -1456,7 +1456,7 @@ int fmb_results_kind(const fmb_results* r) { return r ? r->kind : -1; }
 
 int fmb_results_fetch_hits(const fmb_results* r, fmb_hit* out, uint64_t capacity) {
     if (!r || (!out && r->count)) { set_error("NULL argument"); return FMB_EINVAL; }
-    if (r->kind != 0) { set_error("result set holds located rows, not hits"); return FMB_EINVAL; }
+    if (r->kind != 0) { set_error("result set holds no hits (kind %d)", r->kind); return FMB_EINVAL; }
     if (capacity < r->count) { set_error("capacity %llu < %llu hits", (unsigned long long)capacity, (unsigned long long)r->count); return FMB_EOVERFLOW; }
     FMB_TRY(use_device(r->device));
     const uint64_t slots = r->dense ? r->slots : r->count;
@@ -1473,7 +1473,7 @@ int fmb_results_fetch_hits(const fmb_results* r, fmb_hit* out, uint64_t capacity
 }
 int fmb_results_fetch_locs32(const fmb_results* r, fmb_loc32* out, uint64_t capacity) {
     if (!r || (!out && r->count)) { set_error("NULL argument"); return FMB_EINVAL; }
-    if (r->kind != 1) { set_error("result set holds hits, not located rows"); return FMB_EINVAL; }
+    if (r->kind != 1) { set_error("result set holds no located rows (kind %d)", r->kind); return FMB_EINVAL; }
     if (capacity < r->count) { set_error("capacity %llu < %llu rows", (unsigned long long)capacity, (unsigned long long)r->count); return FMB_EOVERFLOW; }
     FMB_TRY(use_device(r->device));
     if (r->count) FMB_CUDA(cudaMemcpy(out, r->locs.p, r->count * sizeof(LocRec), cudaMemcpyDeviceToHost));
@@ -1481,7 +1481,7 @@ int fmb_results_fetch_locs32(const fmb_results* r, fmb_loc32* out, uint64_t capa
 }
 int fmb_results_fetch_locs(const fmb_results* r, fmb_loc* out, uint64_t capacity) {
     if (!r || (!out && r->count)) { set_error("NULL argument"); return FMB_EINVAL; }
-    if (r->kind != 1) { set_error("result set holds hits, not located rows"); return FMB_EINVAL; }
+    if (r->kind != 1) { set_error("result set holds no located rows (kind %d)", r->kind); return FMB_EINVAL; }
     if (capacity < r->count) { set_error("capacity too small"); return FMB_EOVERFLOW; }
     std::vector<fmb_loc32> h(r->count);
     FMB_TRY(fmb_results_fetch_locs32(r, h.data(), r->count));

@@ -271,9 +271,33 @@ int fmb_extract(const fmb_index* ix, const uint64_t* seq, const uint64_t* begin,
 /* the whole text s0 0 s1 0 ... 0, n bytes: the input of fmb_index_build, so build -> reconstruct round-trips (capacity >= n) */
 int fmb_index_reconstruct_text(const fmb_index* ix, uint8_t* out, uint64_t capacity);
 
+/* ---- super-maximal exact matches (SMEMs): the seeds of reads that exact and k-error search cannot place -------------------------
+ * A query symbol 0 (the delimiter) or >= sigma never matches.  The interval [i, j) (j > i) of a query Q of length m OCCURS when Q[i:j]
+ * holds no non-matching symbol and is a substring of one sequence of the collection (never across a delimiter); its SA interval
+ * (lb, len) of direction 0 is then what fmb_search_exact reports for the query Q[i:j].  [i, j) is an SMEM when it occurs, i == 0 or
+ * [i-1, j) does not occur, and j == m or [i, j+1) does not occur: the occurring intervals that are maximal under containment.  Starts
+ * and ends both increase strictly from one SMEM of a query to the next.  The reference library has no counterpart. */
+typedef struct { uint64_t qidx, begin, end, lb, len; } fmb_smem;          /* SA interval of direction 0, as exact search reports it */
+typedef struct { uint64_t qidx, begin, end, seq, pos; } fmb_smem_loc;     /* pos = text position of Q[begin] in sequence seq        */
+/* Every SMEM of every query of the batch with end - begin >= min_len (min_len <= 1: all of them), ordered by qidx, then begin (result
+ * kind 2).  stats: extensions / occ_lookups count the bidirectional steps as the one-symbol exact kernel counts its steps, line_requests
+ * the lookups of the bidirectional k-mer table, and the locate shortcut, sample, sequence start and text word lookups of the text
+ * path (FMB_TEXT_CHECK; results never depend on which tables the image holds).  FMB_EUNSUPPORTED, before any launch, for a
+ * unidirectional index (no right step) and for FMB_INDEX_NO_DELIM indices (no sequence borders).  FMB_EOVERFLOW when the record list
+ * cannot grow to what the batch needs or holds 2^32 records or more. */
+int fmb_search_smems(const fmb_index* ix, const fmb_queries* q, uint32_t min_len, fmb_results** out);
+/* Per SMEM of `smems` (kind 2) the first min(len, max_occ) rows lb, lb + 1, ... of its interval, located (result kind 3): every
+ * occurrence when len <= max_occ, a deterministic cap on repeats otherwise (max_occ = UINT64_MAX: no cap).  Rows come grouped by SMEM
+ * in record order, within an SMEM in row order.  FMB_EINVAL for another result kind, FMB_EOVERFLOW for 2^32 rows or more (as
+ * fmb_locate), FMB_EUNSUPPORTED as fmb_search_smems. */
+int fmb_locate_smems(const fmb_index* ix, const fmb_results* smems, uint64_t max_occ, fmb_results** out);
+int fmb_results_fetch_smems(const fmb_results* r, fmb_smem* out, uint64_t capacity);              /* kind 2 only, else FMB_EINVAL */
+int fmb_results_fetch_smem_locs(const fmb_results* r, fmb_smem_loc* out, uint64_t capacity);      /* kind 3 only, else FMB_EINVAL */
+
 /* ---- results ----------------------------------------------------------------------------------------------- */
 uint64_t fmb_results_count(const fmb_results* r);
-int  fmb_results_kind(const fmb_results* r);                /* 0 = hits (cursors), 1 = located rows */
+/* 0 = hits (cursors), 1 = located rows, 2 = SMEMs (fmb_search_smems), 3 = located rows of SMEMs (fmb_locate_smems) */
+int  fmb_results_kind(const fmb_results* r);
 int  fmb_results_fetch_hits(const fmb_results* r, fmb_hit* out, uint64_t capacity);
 int  fmb_results_fetch_locs(const fmb_results* r, fmb_loc* out, uint64_t capacity);
 int  fmb_results_fetch_locs32(const fmb_results* r, fmb_loc32* out, uint64_t capacity);

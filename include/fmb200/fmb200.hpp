@@ -6,4 +6,5 @@
 #include "multi.hpp"
 #include "search.hpp"
 #include "search_scheme.hpp"
+#include "smem.hpp"
 #include "io.hpp"
