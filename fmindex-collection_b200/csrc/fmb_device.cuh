@@ -158,17 +158,43 @@ struct Occ2View {
     // 16- or a 32-symbol jump (.z = 0xFFFFFFFF when one of symbols 17..32 is a delimiter)
     uint32_t jump_wide;
     // text check (fmb_index::isa / text2 / seq_start_d; isa == nullptr: none): a single-row interval r with pos query symbols left
-    // lies at (seq, p) = samples[locrow[r] >> loc_step_bits] + the steps in the low bits; the read can only be the text
-    // [p - pos, p) of seq, compared with the query a 128-byte line (512 symbols) at a time, and its row is isa[seq_start[seq] + p - pos]
+    // lies at text position g = sa[r] (or, without the suffix array, (seq, p) = samples[locrow[r] >> loc_step_bits] + the steps in the
+    // low bits); the read can only be the text [g - pos, g) of g's sequence, compared with the query a 128-byte line (512 symbols) at a
+    // time, and its row is isa[g - pos]
     const uint32_t* isa;
     const uint32_t* text32;      // 16 symbols per word, 32 words per 128-byte line
     const uint32_t* seq_start;
+    const uint32_t* sa;          // nullptr: locrow + samples
+    const uint2* seq_of_block;
     const uint32_t* locrow;
     const uint2* samples;
     uint32_t loc_step_bits;
 };
 constexpr uint32_t kJumpInvalid = 0xFFFFFFFFu;
 constexpr uint32_t kNoSeq = 0xFFFFFFFFu;      // fmb_results::at of a hit the text check did not find
+
+// Sequence of text position g of s0 0 s1 0 ... (fmb_index::seq_of_block): per 4096-symbol block b, {s | inner << 31, seq_start[s]}
+// with s the sequence holding the block's first symbol and inner set when another sequence starts inside the block.  Without such a
+// start the answer is the one entry (one cached load: the table is n / 512 bytes); else a binary search of seq_start between s and the
+// sequence of the next block's first symbol.  `lines` counts the loads.
+struct SeqStart {
+    uint32_t seq, start;
+};
+__device__ __forceinline__ SeqStart seq_of(const uint2* __restrict__ blocks, const uint32_t* __restrict__ seq_start, uint32_t g, uint32_t& lines) {
+    const uint2 e = __ldg(blocks + (g >> 12));
+    lines += 1;
+    SeqStart r{e.x & 0x7FFFFFFFu, e.y};
+    if (e.x >> 31) {
+        uint32_t hi = (__ldg(&blocks[(g >> 12) + 1].x) & 0x7FFFFFFFu) + 1;      // seq_start[hi] > g (seq_start[nseq] = n)
+        lines += 1;
+        while (hi - r.seq > 1) {
+            const uint32_t mid = (r.seq + hi) >> 1, v = __ldg(seq_start + mid);
+            lines += 1;
+            if (v <= g) r = SeqStart{mid, v}; else hi = mid;
+        }
+    }
+    return r;
+}
 
 struct Quarter {
     uint32_t cnt[4];

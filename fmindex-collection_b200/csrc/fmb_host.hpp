@@ -125,6 +125,11 @@ struct fmb_index {
     // (FMB_TEXT_LOCATE: the located row of a checked read needs pos % R LF steps), else 0.
     fmb::DevBuf<uint32_t> isa, text2, seq_start_d;
     uint32_t text_rate = 0;
+    // suffix array (FMB_TABLE_LOCROW in place of `locrow` when text_rate is set on the DNA layout): sa[row] = g of the row's suffix,
+    // one fetch per located row (the LF steps the walk would take are pos % text_rate); seq_of_block finds the sequence of a g
+    // (fmb_device.cuh seq_of)
+    fmb::DevBuf<uint32_t> sa;
+    fmb::DevBuf<uint2> seq_of_block;
     // optional tables this image is allowed to hold (FMB_TABLE_* bits), decided once by plan_tables (csrc/fmb_lib.cu) from the image
     // budget (fmb_set_image_budget / FMB_IMAGE_GB; default: everything the device can hold) and the FMB_NO_* knobs of its knob table
     uint32_t allowed_tables = 0xFFFFFFFFu;
@@ -168,6 +173,8 @@ struct fmb_index {
         f(a.isa, b.isa, true);
         f(a.text2, b.text2, true);
         f(a.seq_start_d, b.seq_start_d, true);
+        f(a.sa, b.sa, true);
+        f(a.seq_of_block, b.seq_of_block, true);
         f(a.anchor_pos, b.anchor_pos, false);
         f(a.anchor_row, b.anchor_row, false);
     }
@@ -186,6 +193,7 @@ int new_index(fmb_index** out, int device, uint32_t sigma, uint64_t n, bool bidi
 uint64_t image_budget();                                           // bytes, 0 = no limit
 uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples);     // the FMB_TABLE_* bits for ix->allowed_tables
 constexpr uint32_t kTableTextCheck = 1u << 16;                     // allowed_tables bit of the text check tables (FMB_TEXT_CHECK)
+constexpr uint32_t kTableSuffixArray = 1u << 17;                   // ... and of the suffix array in place of the locate shortcut
 int ensure_layout(const fmb_index* ix);                            // sequence lengths and starts (csrc/fmb_extract.cu)
 int build_occ_from_device_bwt(fmb_index* ix, int dir, const uint8_t* d_bwt);
 int compute_C(fmb_index* ix);

@@ -742,14 +742,24 @@ __global__ void __launch_bounds__(256, 8) exact_search2_kernel(const __grid_cons
                 if (len == 1 && pos >= kTextCheckMin && o2.isa) {
                     // single row with pos symbols left: where the row sits in the text decides the rest (Occ2View::isa).  Every lane
                     // issues the same single lookups (one request each); each lane compares one 32-byte quarter of a text line.
-                    const uint32_t w = __ldg(o2.locrow + lb);
-                    const uint2 smp = __ldg(o2.samples + (w >> o2.loc_step_bits));
-                    const uint32_t p = smp.y + (w & ((1u << o2.loc_step_bits) - 1u));
-                    lines += 2;
-                    if (p < pos) { len = 0; break; }             // the read would start before its sequence
-                    const uint32_t g0 = __ldg(o2.seq_start + smp.x) + (p - pos);
+                    uint32_t g;
+                    SeqStart ss;
+                    if (o2.sa) {
+                        g = __ldg(o2.sa + lb);
+                        lines += 1;
+                        ss = seq_of(o2.seq_of_block, o2.seq_start, g, lines);
+                    } else {
+                        const uint32_t w = __ldg(o2.locrow + lb);
+                        const uint2 smp = __ldg(o2.samples + (w >> o2.loc_step_bits));
+                        ss = SeqStart{smp.x, __ldg(o2.seq_start + smp.x)};
+                        g = ss.start + smp.y + (w & ((1u << o2.loc_step_bits) - 1u));
+                        lines += 3;
+                    }
+                    if (g - ss.start < pos) { len = 0; break; }    // the read would start before its sequence
+                    const uint32_t g0 = g - pos;
+                    lb = __ldg(o2.isa + g0);       // the final row, fetched together with the text lines (only kept on a match)
                     lines += 1;
-                    if (out_at && sub == 3) out_at[q] = make_uint2(smp.x, p - pos);      // replaced by kNoSeq below on a mismatch
+                    if (out_at && sub == 3) out_at[q] = make_uint2(ss.seq, g0 - ss.start);      // replaced by kNoSeq below on a mismatch
                     // lane `sub` compares the read's words sub, sub + 4, ... (symbols [16 j, 16 j + 16)) with the text at g0 + 16 j: the
                     // group's four lanes read four consecutive text words per step, within one or two 128-byte lines
                     uint32_t bad = 0;
@@ -763,8 +773,6 @@ __global__ void __launch_bounds__(256, 8) exact_search2_kernel(const __grid_cons
                     bad |= __shfl_xor_sync(gmask, bad, 2);
                     lines += ((g0 + pos - 1) >> 9) - (g0 >> 9) + 1;
                     if (bad) { len = 0; break; }
-                    lb = __ldg(o2.isa + g0);
-                    lines += 1;
                     checked = true;
                     break;
                 }
@@ -1084,8 +1092,6 @@ __global__ void __launch_bounds__(256) locrow_build_gen_kernel(const __grid_cons
     }
 }
 
-// at (may be nullptr): (seq, pos) per record found by the text check of exact search (kNoSeq: not checked); with text-regular sampling
-// at rate `rate` such a row needs pos % rate LF steps and no index access
 // Text check tables (fmb_index::isa / text2), one thread per row: (seq, pos) of the row from the locate shortcut, g = start[seq] + pos;
 // isa[g] = row, and BWT[row] is the symbol at g - 1 (a delimiter when pos == 0: those positions keep code 0, no read window reaches
 // them).  flags[0] = a row outside its sequence, flags[1] = the largest LF step count of any row.
@@ -1119,7 +1125,54 @@ __global__ void __launch_bounds__(256) sample_rate_kernel(const uint2* __restric
     const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     if (i < count && samples[i].y % rate) atomicOr(bad, 1u);
 }
+// the locate shortcut turned into the suffix array in place (text-regular sampling, after text_tables_kernel checked every row):
+// rows[r] = start[seq] + pos of the row's sample + the row's steps
+__global__ void __launch_bounds__(256) sa_from_locrow_kernel(const uint2* __restrict__ samples, const uint32_t* __restrict__ start, uint32_t step_bits,
+                                                             uint64_t n, uint32_t* rows) {
+    const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (r >= n) return;
+    const uint32_t w = rows[r];
+    const uint2 s = __ldg(samples + (w >> step_bits));
+    rows[r] = __ldg(start + s.x) + s.y + (w & ((1u << step_bits) - 1u));
+}
 
+// K4d: locate through the suffix array (fmb_index::sa): one fetch per row plus the (cached) sequence lookup.  Sampling is text-regular at
+// rate `rate`, so the LF walk to the row's sample would take pos % rate steps; rows the text check of exact search found (at, as in
+// locate_shortcut_kernel) need no fetch at all.
+__global__ void __launch_bounds__(256) locate_sa_kernel(const HitRec* __restrict__ hits, const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total,
+                                                        uint32_t single, const uint2* __restrict__ at, uint32_t rate, const uint32_t* __restrict__ sa,
+                                                        const uint2* __restrict__ seq_of_block, const uint32_t* __restrict__ seq_start,
+                                                        LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
+    uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t steps = 0;
+    if (t < total) {
+        uint32_t lo = single ? t : 0, hi = single ? t + 1 : nh;
+        while (hi - lo > 1) {
+            uint32_t mid = (lo + hi) >> 1;
+            if (__ldg(starts + mid) <= t) lo = mid; else hi = mid;
+        }
+        const HitRec* h = hits + lo;
+        LocRec r;
+        r.qidx = __ldg(&h->qidx); r.e = __ldg(&h->e);
+        const uint2 a = at ? __ldg(at + lo) : make_uint2(kNoSeq, 0u);      // a checked hit is a single row
+        if (a.x != kNoSeq) {
+            r.seq = a.x; r.pos = a.y;
+        } else {
+            const row_t row = __ldg(&h->lb) + (single ? 0u : t - __ldg(starts + lo));
+            const uint32_t g = __ldg(sa + row);
+            uint32_t lines = 0;
+            const SeqStart ss = seq_of(seq_of_block, seq_start, g, lines);
+            r.seq = ss.seq; r.pos = g - ss.start;
+        }
+        steps = r.pos % rate;
+        out[t] = r;
+    }
+    // the LF steps the walk WOULD take: the algorithmic work of SURVEY.md §8d stays reported
+    block_count2(counters, 2, steps, 1, steps);
+}
+
+// at (may be nullptr): (seq, pos) per record found by the text check of exact search (kNoSeq: not checked); with text-regular sampling
+// at rate `rate` such a row needs pos % rate LF steps and no index access
 template <class OCC>
 __global__ void __launch_bounds__(256) locate_shortcut_kernel(const __grid_constant__ IndexView<OCC> ix, const HitRec* __restrict__ hits,
                                                               const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,

@@ -243,6 +243,8 @@ fmb::Occ2View fmb_index::view_occ2() const {
     v.isa = isa.p;
     v.text32 = text2.p;
     v.seq_start = seq_start_d.p;
+    v.sa = sa.p;
+    v.seq_of_block = seq_of_block.p;
     v.locrow = locrow.p;
     v.samples = samples.p;
     v.loc_step_bits = loc_step_bits;
@@ -311,7 +313,7 @@ static uint32_t budget_tables(const fmb_index* ix, uint64_t n_samples) {
         if (allowed & FMB_TABLE_LOCBLOCK) admit(FMB_TABLE_LOCROW, 4 * n);
         if (j0) admit(FMB_TABLE_JUMP32, 8 * n);
         if (j0) admit(FMB_TABLE_JUMP4, 8 * n * (j1 ? 2 : 1));
-        if (allowed & FMB_TABLE_LOCROW) admit(kTableTextCheck, 4.25 * n);
+        if (allowed & FMB_TABLE_LOCROW) admit(kTableTextCheck | kTableSuffixArray, 4.25 * n + n / 512);      // + the sequence lookup of sa
     } else {
         admit(FMB_TABLE_JUMP4, 8 * n * (ix->bidirectional ? 2 : 1));      // generic layout: byte-symbol LF^4 tables ...
         admit(FMB_TABLE_LOCROW, 4 * n);                                    // ... the locate shortcut ...
@@ -334,7 +336,10 @@ static uint32_t budget_tables(const fmb_index* ix, uint64_t n_samples) {
 //   FMB_NO_LOCBLOCKS   LOCBLOCK, LOCROW (the shortcut walks the blocks) -
 //   FMB_NO_LOCROW      LOCROW                                           LOCROW
 //   FMB_NO_TEXTCHECK   the text check tables (kTableTextCheck)          -
-// (the text check tables are built from the locate shortcut: without LOCROW there are none)
+//   FMB_NO_SA          the suffix array (kTableSuffixArray): LOCROW     -
+//                      keeps the form sample index + steps
+// (the text check tables are built from the locate shortcut: without LOCROW there are none; the suffix array replaces the shortcut
+// when the text check finds the sampling text-regular)
 // FMB_KMER_K (build_occ2) sizes the exact-search k-mer table; FMB_KMER_K=0 leaves it out.
 uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
     static const struct { const char* name; uint32_t dna, gen; } knobs[] = {
@@ -345,6 +350,7 @@ uint32_t plan_tables(const fmb_index* ix, uint64_t n_samples) {
         {"FMB_NO_LOCBLOCKS", FMB_TABLE_LOCBLOCK | FMB_TABLE_LOCROW, 0},
         {"FMB_NO_LOCROW", FMB_TABLE_LOCROW, FMB_TABLE_LOCROW},
         {"FMB_NO_TEXTCHECK", kTableTextCheck, 0},
+        {"FMB_NO_SA", kTableSuffixArray, 0},
     };
     uint32_t allowed = budget_tables(ix, n_samples);
     for (const auto& k : knobs)
@@ -661,7 +667,8 @@ int build_search_tables(fmb_index* ix) {
 // Text check tables of exact search (DNA layout): ISA (4 bytes per row), the text as 2-bit codes and the sequence starts, built from
 // the locate shortcut (every row's text position).  Skipped without the shortcut, when the plan does not allow them, when the device
 // cannot hold them or when the samples do not describe a collection (the search then keeps its LF jumps).  text_rate is set when the
-// sampling is text-regular, the condition under which locate can report the step counts of the rows the check finds.
+// sampling is text-regular, the condition under which locate can report the step counts of the rows the check finds; the locate
+// shortcut then becomes the suffix array (kTableSuffixArray, knob FMB_NO_SA).
 static int build_text_check(fmb_index* ix) {
     if (!ix->dna || !ix->locrow.p || !(ix->allowed_tables & kTableTextCheck)) return FMB_OK;
     const uint64_t n = ix->n, words = (n / 512 + 2) * 32;       // whole 128-byte lines and one more
@@ -697,8 +704,31 @@ static int build_text_check(fmb_index* ix) {
     note_launches(2);
     ix->isa = std::move(isa);
     ix->text2 = std::move(text);
-    ix->seq_start_d = std::move(start);
     ix->text_rate = h_flags[2] ? 0u : rate;
+    // text-regular sampling: every row's step count is pos % text_rate, so the shortcut's sample index and steps say no more than the
+    // row's text position -- the suffix array takes its place (same 4 bytes per row) and locates a row with one fetch
+    if (ix->text_rate && (ix->allowed_tables & kTableSuffixArray) && nseq < (uint64_t(1) << 31)) {
+        const uint64_t nb = (n >> 12) + 2;          // every block of a position < n, and the one after the last
+        std::vector<uint2> sob(nb);
+        uint64_t s = 0;
+        for (uint64_t b = 0; b < nb; ++b) {
+            const uint64_t first = b << 12;
+            while (s + 1 < nseq && h_start[s + 1] <= first) ++s;
+            const bool inner = s + 1 < nseq && h_start[s + 1] < first + 4096;
+            sob[b] = make_uint2((uint32_t)s | (inner ? 1u << 31 : 0u), h_start[s]);
+        }
+        DevBuf<uint2> d_sob;
+        FMB_TRY(d_sob.alloc(nb));
+        FMB_CUDA(cudaMemcpyAsync(d_sob.p, sob.data(), nb * sizeof(uint2), cudaMemcpyHostToDevice, st));
+        sa_from_locrow_kernel<<<grid_for(n, 256), 256, 0, st>>>(ix->samples.p, start.p, ix->loc_step_bits, n, ix->locrow.p);
+        FMB_CUDA(cudaGetLastError());
+        FMB_CUDA(cudaStreamSynchronize(st));
+        note_launches(1);
+        ix->sa = std::move(ix->locrow);
+        ix->loc_step_bits = 0;
+        ix->seq_of_block = std::move(d_sob);
+    }
+    ix->seq_start_d = std::move(start);
     return FMB_OK;
 }
 
@@ -919,7 +949,7 @@ int fmb_index_get_info(const fmb_index* ix, fmb_index_info* info) {
     info->device = ix->device;
     info->flags = (ix->first_symb ? 0u : FMB_INDEX_NO_DELIM) | (ix->reuse_rev ? FMB_INDEX_REUSE_REV : 0u);
     info->tables = (ix->occ2.p ? FMB_TABLE_PAIR : 0) | (ix->kmer.p ? FMB_TABLE_KMER : 0) | (ix->jump[0].p ? FMB_TABLE_JUMP : 0) |
-                   (ix->jump[1].p ? FMB_TABLE_JUMP_REV : 0) | (ix->locblocks.p ? FMB_TABLE_LOCBLOCK : 0) | (ix->locrow.p ? FMB_TABLE_LOCROW : 0) |
+                   (ix->jump[1].p ? FMB_TABLE_JUMP_REV : 0) | (ix->locblocks.p ? FMB_TABLE_LOCBLOCK : 0) | (ix->locrow.p || ix->sa.p ? FMB_TABLE_LOCROW : 0) |
                    (ix->bikmer.p ? FMB_TABLE_BIKMER : 0) | (ix->jump4[0].p ? FMB_TABLE_JUMP4 : 0) | (ix->jump_shift[0] ? FMB_TABLE_JUMP32 : 0);
     info->tables |= ix->anchor_pos.p ? FMB_TABLE_ANCHORS : 0;
     info->text_tables = (ix->isa.p ? FMB_TEXT_CHECK : 0u) | (ix->isa.p && ix->text_rate ? FMB_TEXT_LOCATE : 0u);
@@ -1367,7 +1397,11 @@ int fmb_locate(const fmb_index* ix, const fmb_results* hits, fmb_results** out) 
     cudaEventCreate(&ev_m1);
     if (total) {
         cudaEventRecord(ev_m0, st);
-        if (ix->locrow.p && ix->locate_mode != FMB_LOCATE_WALK) {
+        if (ix->sa.p && ix->locate_mode != FMB_LOCATE_WALK) {
+            const uint2* at = hits->dense ? hits->at.p : nullptr;
+            locate_sa_kernel<<<grid_for(total, 256), 256, 0, st>>>(hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, at, ix->text_rate, ix->sa.p,
+                                                                   ix->seq_of_block.p, ix->seq_start_d.p, res->locs.p, ctr.p);
+        } else if (ix->locrow.p && ix->locate_mode != FMB_LOCATE_WALK) {
             const uint2* at = hits->dense && ix->text_rate ? hits->at.p : nullptr;
             FMB_DISPATCH(ix, v, locate_shortcut_kernel<<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, at, ix->text_rate,
                                                                                              res->locs.p, ctr.p));

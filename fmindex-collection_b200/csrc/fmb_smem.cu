@@ -58,6 +58,8 @@ struct SmemArgs {
     uint32_t bikmer_k, bikmer_base;   // base 0: 2-bit key (DNA layout)
     const uint32_t* text32;       // nullptr: no text path
     const uint32_t* seq_start;
+    const uint32_t* sa;           // nullptr: locrow + samples
+    const uint2* seq_of_block;
     const uint32_t* locrow;
     const uint2* samples;
     uint32_t loc_step_bits;
@@ -88,15 +90,26 @@ __global__ void __launch_bounds__(256) smem_kernel(const __grid_constant__ Index
     const Cursor whole{0, 0, ix.n, 0};
     auto sym = [&](uint32_t p) -> uint32_t { return __ldg(a.qsym + off + p); };
     auto matches = [&](uint32_t c) { return c >= 1 && c < ix.sigma; };
-    // text position of the suffix of `row` (locate shortcut + sample) and the borders of its sequence
+    // text position of the suffix of `row` (suffix array, or locate shortcut + sample) and the borders of its sequence
     auto text_pos = [&](row_t row) -> uint32_t {
-        const uint32_t w = __ldg(a.locrow + row);
-        const uint2 smp = __ldg(a.samples + (w >> a.loc_step_bits));
-        tseq = smp.x;
-        tbeg = __ldg(a.seq_start + tseq);
+        uint32_t g;
+        if (a.sa) {
+            g = __ldg(a.sa + row);
+            lines += 1;
+            const SeqStart ss = seq_of(a.seq_of_block, a.seq_start, g, lines);
+            tseq = ss.seq;
+            tbeg = ss.start;
+        } else {
+            const uint32_t w = __ldg(a.locrow + row);
+            const uint2 smp = __ldg(a.samples + (w >> a.loc_step_bits));
+            tseq = smp.x;
+            tbeg = __ldg(a.seq_start + tseq);
+            lines += 3;
+            g = tbeg + smp.y + (w & ((1u << a.loc_step_bits) - 1u));
+        }
         tend = __ldg(a.seq_start + tseq + 1) - 1;          // the sequence's delimiter
-        lines += 3;
-        return tbeg + smp.y + (w & ((1u << a.loc_step_bits) - 1u));
+        lines += 1;
+        return g;
     };
     for (;;) {
         // ---- resolve: everything up to the next extension this lane needs --------------------------------------------------------
@@ -292,6 +305,8 @@ int fmb_search_smems(const fmb_index* ix, const fmb_queries* q, uint32_t min_len
     if (ix->isa.p && q->packed.p && q->flags.p) {
         args.text32 = ix->text2.p;
         args.seq_start = ix->seq_start_d.p;
+        args.sa = ix->sa.p;
+        args.seq_of_block = ix->seq_of_block.p;
         args.locrow = ix->locrow.p;
         args.samples = ix->samples.p;
         args.loc_step_bits = ix->loc_step_bits;

@@ -75,7 +75,7 @@ typedef struct {
 #define FMB_TABLE_JUMP     4u   /* LF^16 jump table, direction 0                   */
 #define FMB_TABLE_JUMP_REV 8u   /* LF^16 jump table, direction 1                   */
 #define FMB_TABLE_LOCBLOCK 16u  /* combined occ + marker records for locate        */
-#define FMB_TABLE_LOCROW   32u  /* locate shortcut table                           */
+#define FMB_TABLE_LOCROW   32u  /* locate shortcut table, or the suffix array that replaces it (text-regular sampling, sigma <= 5) */
 #define FMB_TABLE_BIKMER   64u  /* bidirectional k-mer table for scheme roots      */
 #define FMB_TABLE_JUMP4    128u /* LF^4 jump tables (tails shorter than 16 symbols) */
 #define FMB_TABLE_JUMP32   256u /* direction 0 holds merged LF^16 / LF^32 entries (32 symbols per lookup in exact search) */
