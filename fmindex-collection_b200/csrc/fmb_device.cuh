@@ -138,6 +138,20 @@ struct OccDna {
 //     u32 cnt[4]    absolute # rows before the block with code 4k .. 4k+3 (special rows count as code 0)
 //     u32 plane[4]  bit r of plane[j] = bit j of the code of row 128*b + 32*k + r
 // rank2(row, code) = sum over the 4 lanes of (popc(match(code) & rows-below-mask) + own counter) -> 2 SHFL.XOR.
+
+// Where the suffix of a row starts in the text (fmb_index::view_rowpos, row_pos below), from the locate shortcut table in either of its
+// forms: the suffix array (sa[row] = g of s0 0 s1 0 ..., its sequence through seq_of_block) or, without it, the shortcut word
+// locrow[row] = sample index << step_bits | LF steps to that sample.
+struct RowPosView {
+    const uint32_t* sa;          // nullptr: the shortcut form
+    const uint2* seq_of_block;
+    const uint32_t* seq_start;   // start of every sequence (+ n); nullptr before the text check tables exist
+    const uint32_t* locrow;
+    const uint2* samples;
+    uint32_t step_bits;
+    uint32_t rate;               // text-regular sampling at this rate (a row's LF steps are pos % rate); 0: irregular
+};
+
 struct Occ2View {
     const uint4* lines;          // 8 uint4 per block; nullptr when the table was not built
     const uint32_t* specials;    // sorted special rows, padded with 0xFFFFFFFF
@@ -157,18 +171,12 @@ struct Occ2View {
     // jump_wide != 0: `jump` holds 16-byte entries {LF^16(row), symbols 1..16, LF^32(row), symbols 17..32} -- one lookup serves a
     // 16- or a 32-symbol jump (.z = 0xFFFFFFFF when one of symbols 17..32 is a delimiter)
     uint32_t jump_wide;
-    // text check (fmb_index::isa / text2 / seq_start_d; isa == nullptr: none): a single-row interval r with pos query symbols left
-    // lies at text position g = sa[r] (or, without the suffix array, (seq, p) = samples[locrow[r] >> loc_step_bits] + the steps in the
-    // low bits); the read can only be the text [g - pos, g) of g's sequence, compared with the query a 128-byte line (512 symbols) at a
-    // time, and its row is isa[g - pos]
+    // text check (fmb_index::isa / text2; isa == nullptr: none): a single-row interval r with pos query symbols left lies at text
+    // position g = row_pos(r).g; the read can only be the text [g - pos, g) of g's sequence, compared with the query a 128-byte line
+    // (512 symbols) at a time, and its row is isa[g - pos]
     const uint32_t* isa;
     const uint32_t* text32;      // 16 symbols per word, 32 words per 128-byte line
-    const uint32_t* seq_start;
-    const uint32_t* sa;          // nullptr: locrow + samples
-    const uint2* seq_of_block;
-    const uint32_t* locrow;
-    const uint2* samples;
-    uint32_t loc_step_bits;
+    RowPosView rowpos;
 };
 constexpr uint32_t kJumpInvalid = 0xFFFFFFFFu;
 constexpr uint32_t kNoSeq = 0xFFFFFFFFu;      // fmb_results::at of a hit the text check did not find
@@ -191,6 +199,39 @@ __device__ __forceinline__ SeqStart seq_of(const uint2* __restrict__ blocks, con
             const uint32_t mid = (r.seq + hi) >> 1, v = __ldg(seq_start + mid);
             lines += 1;
             if (v <= g) r = SeqStart{mid, v}; else hi = mid;
+        }
+    }
+    return r;
+}
+
+// Text position of the suffix of `row`: its sequence, the position in it and the LF steps the walk to its sample takes; with kText also
+// the global position g and the sequence's start (the shortcut form then reads seq_start, which exists with the text check tables).
+// `lines` counts the loads of kText callers: 1 + seq_of's for the suffix array, 3 for the shortcut.
+struct RowPos {
+    uint32_t seq, pos, steps, g, start;
+};
+template <bool kText>
+__device__ __forceinline__ RowPos row_pos(const RowPosView& v, row_t row, uint32_t& lines) {
+    RowPos r;
+    if (v.sa) {
+        r.g = __ldg(v.sa + row);
+        lines += 1;
+        const SeqStart ss = seq_of(v.seq_of_block, v.seq_start, r.g, lines);
+        r.seq = ss.seq;
+        r.start = ss.start;
+        r.pos = r.g - ss.start;
+        r.steps = r.pos % v.rate;
+    } else {
+        const uint32_t w = __ldg(v.locrow + row);
+        const uint2 smp = __ldg(v.samples + (w >> v.step_bits));
+        r.steps = w & ((1u << v.step_bits) - 1u);
+        r.seq = smp.x;
+        r.pos = smp.y + r.steps;
+        lines += 2;
+        if (kText) {
+            r.start = __ldg(v.seq_start + smp.x);
+            r.g = r.start + r.pos;
+            lines += 1;
         }
     }
     return r;
@@ -328,10 +369,6 @@ struct IndexView {
     // u32, pad} so that one LF step of locate touches ONE line instead of two (occ block + marker word); a lane pair
     // fetches the two 32-byte halves with one request.  nullptr when not built.
     const uint4* locblocks;
-    // locate shortcut (optional): per row  sample_index << loc_step_bits | steps  -- the result of the row's LF walk to its
-    // nearest sampled row, precomputed at build time, so that locate(row) is two independent fetches (this word + the sample)
-    const uint32_t* locrow;
-    uint32_t loc_step_bits;
 };
 
 struct Cursor {             // BiFMIndexCursor{lb, lbRev, len, steps}, fmindex/BiFMIndexCursor.h:22-37
@@ -391,6 +428,79 @@ __device__ __forceinline__ Cursor extend_bi(const IndexView<OCC>& ix, const Curs
     o.len = r1 - r0;
     o.steps = c.steps + 1;
     return o;
+}
+
+// One LF step (fmindex/BiFMIndex.h:177-202): c = BWT[row], row' = C[c] + rank(row, c).  b = the occ block of row, loaded for symbol 0.
+template <class OCC>
+__device__ __forceinline__ row_t lf_step(const IndexView<OCC>& ix, typename OCC::Block b, row_t row, uint32_t& c) {
+    const OCC& occ = ix.occ[0];
+    c = occ.symbol(b, row);
+    if (OCC::kSymbolLoad) b = occ.load(row >> 6, c);
+    return ix.C[c] + occ.rank(b, row, c);
+}
+
+// LF walk of one thread from `row` to the nearest sampled row: the sample's index (adding the LF steps to `steps`), or kNoSample after
+// more than `limit` steps.  The marker word and the occ block of a row are independent loads and are issued together.
+constexpr uint32_t kNoSample = 0xFFFFFFFFu;
+template <class OCC>
+__device__ __forceinline__ uint32_t walk_to_sample(const IndexView<OCC>& ix, row_t row, uint32_t& steps, uint32_t limit = 0xFFFFFFFFu) {
+    for (;;) {
+        const uint4 m = __ldg(ix.marks + (row >> 6));
+        const typename OCC::Block b = ix.occ[0].load(row >> 6, 0);
+        const uint64_t bits = (uint64_t)m.x | ((uint64_t)m.y << 32);
+        const uint32_t o = row & 63;
+        if ((bits >> o) & 1) return m.z + __popcll(bits & low_mask(o));
+        uint32_t c;
+        row = lf_step(ix, b, row, c);
+        if (++steps > limit) return kNoSample;
+    }
+}
+
+// Work counters: one global atomic per BLOCK and counter.  (One per warp meant > 10^6 same-address atomics per launch, which
+// serialise in one L2 slice and cost more than the kernel's real work: locate went from 1.4 ms to the time of its loads.)
+// Every thread of the block must call this (it contains __syncthreads).
+__device__ __forceinline__ void block_count2(unsigned long long* counters, int slot_a, uint32_t a, int slot_b, uint32_t b) {
+    __shared__ unsigned int s_cnt[2];
+    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
+    __syncthreads();
+    for (int o = 16; o > 0; o >>= 1) {
+        a += __shfl_xor_sync(0xFFFFFFFFu, a, o);
+        b += __shfl_xor_sync(0xFFFFFFFFu, b, o);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (a) atomicAdd(&s_cnt[0], a);
+        if (b) atomicAdd(&s_cnt[1], b);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        if (s_cnt[0]) atomicAdd(counters + slot_a, (unsigned long long)s_cnt[0]);
+        if (slot_b >= 0 && s_cnt[1]) atomicAdd(counters + slot_b, (unsigned long long)s_cnt[1]);
+    }
+}
+
+// the same for three counters, the third one 64 bits wide (sum of interval lengths)
+__device__ __forceinline__ void block_count3(unsigned long long* counters, int slot_a, uint32_t a, int slot_b, uint32_t b, int slot_c, unsigned long long c) {
+    __shared__ unsigned int s_cnt[2];
+    __shared__ unsigned long long s_cnt64;
+    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
+    if (threadIdx.x == 2) s_cnt64 = 0;
+    __syncthreads();
+    for (int o = 16; o > 0; o >>= 1) {
+        a += __shfl_xor_sync(0xFFFFFFFFu, a, o);
+        b += __shfl_xor_sync(0xFFFFFFFFu, b, o);
+        c += __shfl_xor_sync(0xFFFFFFFFu, c, o);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (a) atomicAdd(&s_cnt[0], a);
+        if (b) atomicAdd(&s_cnt[1], b);
+        if (c) atomicAdd(&s_cnt64, c);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        if (s_cnt[0]) atomicAdd(counters + slot_a, (unsigned long long)s_cnt[0]);
+        if (s_cnt[1]) atomicAdd(counters + slot_b, (unsigned long long)s_cnt[1]);
+        if (s_cnt64) atomicAdd(counters + slot_c, s_cnt64);
+    }
 }
 
 }  // namespace fmb

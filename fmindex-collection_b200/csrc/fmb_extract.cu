@@ -24,34 +24,12 @@ namespace {
 
 constexpr uint32_t kNone = 0xFFFFFFFFu;
 
-// the two work counters of a block, added to counters[0] and counters[1] with one atomic each per block (as block_count2 of
-// fmb_kernels.cuh, which cannot be included here: it defines the library's other kernels).  Every thread of the block calls it.
-__device__ __forceinline__ void block_count(unsigned long long* counters, uint32_t a, uint32_t b) {
-    __shared__ unsigned int s_cnt[2];
-    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
-    __syncthreads();
-    for (int o = 16; o > 0; o >>= 1) {
-        a += __shfl_xor_sync(0xFFFFFFFFu, a, o);
-        b += __shfl_xor_sync(0xFFFFFFFFu, b, o);
-    }
-    if ((threadIdx.x & 31) == 0) {
-        if (a) atomicAdd(&s_cnt[0], a);
-        if (b) atomicAdd(&s_cnt[1], b);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        if (s_cnt[0]) atomicAdd(counters, (unsigned long long)s_cnt[0]);
-        if (s_cnt[1]) atomicAdd(counters + 1, (unsigned long long)s_cnt[1]);
-    }
-}
-
 // one thread per delimiter row: walk back to a sampled row or to position 0 of the sequence (see the header comment)
 template <class OCC>
 __global__ void __launch_bounds__(256) seq_end_kernel(const __grid_constant__ IndexView<OCC> ix, uint32_t nd, uint32_t* __restrict__ seq,
                                                       uint32_t* __restrict__ len, uint32_t* __restrict__ prev) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= nd) return;
-    const OCC& occ = ix.occ[0];
     row_t row = t;
     uint32_t steps = 0;
     for (;;) {
@@ -65,10 +43,8 @@ __global__ void __launch_bounds__(256) seq_end_kernel(const __grid_constant__ In
             prev[t] = kNone;
             return;
         }
-        typename OCC::Block b = occ.load(row >> 6, 0);
-        const uint32_t c = occ.symbol(b, row);
-        if (OCC::kSymbolLoad) b = occ.load(row >> 6, c);
-        const row_t next = ix.C[c] + occ.rank(b, row, c);
+        uint32_t c;
+        const row_t next = lf_step(ix, ix.occ[0].load(row >> 6, 0), row, c);
         if (c == 0) {                       // position 0 of the sequence: `next` is the delimiter row of the one before
             seq[t] = kNone;
             len[t] = steps;
@@ -147,7 +123,6 @@ __global__ void __launch_bounds__(256) extract_walk_kernel(const __grid_constant
         const uint32_t stop = max(below, r.x);
         const uint32_t end = min(P, r.y);
         uint8_t* const o = out + (__ldg(out_off + i) - r.x);   // o[pos] for pos in [gb, ge)
-        const OCC& occ = ix.occ[0];
         while (P > stop) {
             const uint32_t rem = P - stop;
             if (jump16 && rem >= 16) {
@@ -177,16 +152,14 @@ __global__ void __launch_bounds__(256) extract_walk_kernel(const __grid_constant
                     continue;
                 }
             }
-            typename OCC::Block b = occ.load(row >> 6, 0);
-            const uint32_t c = occ.symbol(b, row);
-            if (OCC::kSymbolLoad) b = occ.load(row >> 6, c);
-            row = ix.C[c] + occ.rank(b, row, c);
+            uint32_t c;
+            row = lf_step(ix, ix.occ[0].load(row >> 6, 0), row, c);
             --P;
             if (P < end) o[P] = (uint8_t)c;
             ++steps;
         }
     }
-    block_count(counters, requests, steps);
+    block_count2(counters, 0, requests, 1, steps);
 }
 
 int check_index(const fmb_index* ix) {

@@ -149,6 +149,7 @@ struct fmb_index {
     fmb::IndexView<fmb::OccDna> view_dna() const;
     fmb::IndexView<fmb::OccGen> view_gen() const;
     fmb::Occ2View view_occ2() const;
+    fmb::RowPosView view_rowpos() const;   // the locate shortcut table in either form
     uint64_t device_bytes() const;
 
     // The image's device buffers, the one list that device_bytes() and fmb_index_replicate walk: f(buffer of a, the same buffer of

@@ -6,53 +6,6 @@
 
 namespace fmb {
 
-// Work counters: one global atomic per BLOCK and counter.  (One per warp meant > 10^6 same-address atomics per launch, which
-// serialise in one L2 slice and cost more than the kernel's real work: locate went from 1.4 ms to the time of its loads.)
-// Every thread of the block must call this (it contains __syncthreads).
-__device__ __forceinline__ void block_count2(unsigned long long* counters, int slot_a, uint32_t a, int slot_b, uint32_t b) {
-    __shared__ unsigned int s_cnt[2];
-    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
-    __syncthreads();
-    for (int o = 16; o > 0; o >>= 1) {
-        a += __shfl_xor_sync(0xFFFFFFFFu, a, o);
-        b += __shfl_xor_sync(0xFFFFFFFFu, b, o);
-    }
-    if ((threadIdx.x & 31) == 0) {
-        if (a) atomicAdd(&s_cnt[0], a);
-        if (b) atomicAdd(&s_cnt[1], b);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        if (s_cnt[0]) atomicAdd(counters + slot_a, (unsigned long long)s_cnt[0]);
-        if (slot_b >= 0 && s_cnt[1]) atomicAdd(counters + slot_b, (unsigned long long)s_cnt[1]);
-    }
-}
-
-// the same for three counters, the third one 64 bits wide (sum of interval lengths)
-__device__ __forceinline__ void block_count3(unsigned long long* counters, int slot_a, uint32_t a, int slot_b, uint32_t b, int slot_c, unsigned long long c) {
-    __shared__ unsigned int s_cnt[2];
-    __shared__ unsigned long long s_cnt64;
-    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
-    if (threadIdx.x == 2) s_cnt64 = 0;
-    __syncthreads();
-    for (int o = 16; o > 0; o >>= 1) {
-        a += __shfl_xor_sync(0xFFFFFFFFu, a, o);
-        b += __shfl_xor_sync(0xFFFFFFFFu, b, o);
-        c += __shfl_xor_sync(0xFFFFFFFFu, c, o);
-    }
-    if ((threadIdx.x & 31) == 0) {
-        if (a) atomicAdd(&s_cnt[0], a);
-        if (b) atomicAdd(&s_cnt[1], b);
-        if (c) atomicAdd(&s_cnt64, c);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        if (s_cnt[0]) atomicAdd(counters + slot_a, (unsigned long long)s_cnt[0]);
-        if (s_cnt[1]) atomicAdd(counters + slot_b, (unsigned long long)s_cnt[1]);
-        if (s_cnt64) atomicAdd(counters + slot_c, s_cnt64);
-    }
-}
-
 __host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
     uint64_t z = x + 0x9e3779b97f4a7c15ull;
     z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
@@ -742,24 +695,12 @@ __global__ void __launch_bounds__(256, 8) exact_search2_kernel(const __grid_cons
                 if (len == 1 && pos >= kTextCheckMin && o2.isa) {
                     // single row with pos symbols left: where the row sits in the text decides the rest (Occ2View::isa).  Every lane
                     // issues the same single lookups (one request each); each lane compares one 32-byte quarter of a text line.
-                    uint32_t g;
-                    SeqStart ss;
-                    if (o2.sa) {
-                        g = __ldg(o2.sa + lb);
-                        lines += 1;
-                        ss = seq_of(o2.seq_of_block, o2.seq_start, g, lines);
-                    } else {
-                        const uint32_t w = __ldg(o2.locrow + lb);
-                        const uint2 smp = __ldg(o2.samples + (w >> o2.loc_step_bits));
-                        ss = SeqStart{smp.x, __ldg(o2.seq_start + smp.x)};
-                        g = ss.start + smp.y + (w & ((1u << o2.loc_step_bits) - 1u));
-                        lines += 3;
-                    }
-                    if (g - ss.start < pos) { len = 0; break; }    // the read would start before its sequence
-                    const uint32_t g0 = g - pos;
+                    const RowPos rp = row_pos<true>(o2.rowpos, lb, lines);
+                    if (rp.pos < pos) { len = 0; break; }    // the read would start before its sequence
+                    const uint32_t g0 = rp.g - pos;
                     lb = __ldg(o2.isa + g0);       // the final row, fetched together with the text lines (only kept on a match)
                     lines += 1;
-                    if (out_at && sub == 3) out_at[q] = make_uint2(ss.seq, g0 - ss.start);      // replaced by kNoSeq below on a mismatch
+                    if (out_at && sub == 3) out_at[q] = make_uint2(rp.seq, rp.pos - pos);      // replaced by kNoSeq below on a mismatch
                     // lane `sub` compares the read's words sub, sub + 4, ... (symbols [16 j, 16 j + 16)) with the text at g0 + 16 j: the
                     // group's four lanes read four consecutive text words per step, within one or two 128-byte lines
                     uint32_t bad = 0;
@@ -892,11 +833,24 @@ __global__ void hit_lengths_kernel(const HitRec* __restrict__ hits, uint64_t nh,
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// K4: locate.  One SA row per thread; LF walk to the nearest sampled row (fmindex/BiFMIndex.h:177-202):
+// K4: locate.  One SA row per thread; LF walk to the nearest sampled row (fmindex/BiFMIndex.h:177-202, walk_to_sample):
 //     while row not sampled: c = BWT[row]; row = C[c] + rank(row, c); ++steps
-// The marker word and the occ block of a row are independent loads and are issued together.
 // starts[] = exclusive prefix sum of the hit interval lengths; a thread finds its hit by binary search.
 // ---------------------------------------------------------------------------------------------------------
+// record of located row t: the largest h with starts[h] <= t (single: every record is exactly one row, h == t)
+__device__ __forceinline__ uint32_t hit_of(const uint32_t* __restrict__ starts, uint32_t nh, uint32_t t, uint32_t single) {
+    uint32_t lo = single ? t : 0, hi = single ? t + 1 : nh;
+    while (hi - lo > 1) {
+        uint32_t mid = (lo + hi) >> 1;
+        if (__ldg(starts + mid) <= t) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+// the row of located row t in its record h
+__device__ __forceinline__ row_t hit_row(const HitRec* __restrict__ hits, const uint32_t* __restrict__ starts, uint32_t h, uint32_t t, uint32_t single) {
+    return __ldg(&hits[h].lb) + (single ? 0u : t - __ldg(starts + h));
+}
+
 template <class OCC>
 __global__ void __launch_bounds__(256) locate_kernel(const __grid_constant__ IndexView<OCC> ix, const HitRec* __restrict__ hits,
                                                      const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,
@@ -904,32 +858,10 @@ __global__ void __launch_bounds__(256) locate_kernel(const __grid_constant__ Ind
     uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t steps = 0;
     if (t < total) {
-        // largest h with starts[h] <= t (single: every record is exactly one row, h == t)
-        uint32_t lo = single ? t : 0, hi = single ? t + 1 : nh;
-        while (hi - lo > 1) {
-            uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(starts + mid) <= t) lo = mid; else hi = mid;
-        }
-        HitRec h = hits[lo];
-        row_t row = h.lb + (single ? 0u : t - __ldg(starts + lo));
-        const OCC& occ = ix.occ[0];
-        uint2 sample;
-        for (;;) {
-            uint4 m = __ldg(ix.marks + (row >> 6));
-            typename OCC::Block b = occ.load(row >> 6, 0);
-            uint64_t bits = (uint64_t)m.x | ((uint64_t)m.y << 32);
-            uint32_t o = row & 63;
-            if ((bits >> o) & 1) {
-                sample = __ldg(ix.samples + (m.z + __popcll(bits & low_mask(o))));
-                break;
-            }
-            uint32_t c = occ.symbol(b, row);
-            if (OCC::kSymbolLoad) b = occ.load(row >> 6, c);
-            row = ix.C[c] + occ.rank(b, row, c);
-            ++steps;
-        }
+        const uint32_t h = hit_of(starts, nh, t, single);
+        const uint2 sample = __ldg(ix.samples + walk_to_sample(ix, hit_row(hits, starts, h, t, single), steps));
         LocRec r;
-        r.qidx = h.qidx; r.seq = sample.x; r.pos = sample.y + steps; r.e = h.e;
+        r.qidx = __ldg(&hits[h].qidx); r.seq = sample.x; r.pos = sample.y + steps; r.e = __ldg(&hits[h].e);
         out[t] = r;
     }
     block_count2(counters, 2, steps, 1, steps);
@@ -949,6 +881,33 @@ __global__ void build_locblocks_kernel(const DnaBlock* __restrict__ occ, const u
     out[b * 4 + 3] = make_uint4(0, 0, 0, 0);
 }
 
+// one step of the pair walk: 1 + the sample index when `row` is sampled, else 0 and `row` becomes the next row (role 0 = occ half,
+// role 1 = marker half; pmask = the pair's two lanes)
+__device__ __forceinline__ uint32_t pair_step(const IndexView<OccDna>& ix, uint32_t role, uint32_t pmask, row_t& row) {
+    uint32_t a0, a1, a2, a3, a4, a5, a6, a7;
+    asm volatile("ld.global.nc.L1::no_allocate.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(a3), "=r"(a4), "=r"(a5), "=r"(a6), "=r"(a7)
+                 : "l"(ix.locblocks + ((size_t)(row >> 6) * 4 + role * 2)));
+    uint32_t mine;                                       // role 1: sampled ? 1 + sample index : 0;  role 0: next row
+    if (role) {
+        uint64_t bits = (uint64_t)a0 | ((uint64_t)a1 << 32);
+        uint32_t o = row & 63;
+        mine = ((bits >> o) & 1) ? 1u + a2 + __popcll(bits & low_mask(o)) : 0u;
+    } else {
+        DnaBlock b;
+        b.cnt[0] = a0; b.cnt[1] = a1; b.cnt[2] = a2; b.cnt[3] = a3;
+        b.p0 = (uint64_t)a4 | ((uint64_t)a5 << 32);
+        b.p1 = (uint64_t)a6 | ((uint64_t)a7 << 32);
+        const OccDna& occ = ix.occ[0];
+        uint32_t c = occ.symbol(b, row);
+        mine = ix.C[c] + occ.rank(b, row, c);
+    }
+    uint32_t other = __shfl_xor_sync(pmask, mine, 1);
+    uint32_t sampled = role ? mine : other;
+    if (!sampled) row = role ? other : mine;
+    return sampled;
+}
+
 __global__ void __launch_bounds__(256) locate_pair_kernel(const __grid_constant__ IndexView<OccDna> ix, const HitRec* __restrict__ hits,
                                                           const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,
                                                           LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
@@ -957,46 +916,22 @@ __global__ void __launch_bounds__(256) locate_pair_kernel(const __grid_constant_
     // (t += number of pairs in the grid); all pairs run the same loop body, there is no divergence to pay for.
     const uint32_t npairs = (gridDim.x * blockDim.x) >> 1;
     uint32_t t = (blockIdx.x * blockDim.x + threadIdx.x) >> 1;
-    const uint32_t role = threadIdx.x & 1;                 // 0 = occ half, 1 = marker half
+    const uint32_t role = threadIdx.x & 1;
     const uint32_t pmask = 3u << (threadIdx.x & 30);
-    const OccDna& occ = ix.occ[0];
     uint32_t steps_total = 0, steps = 0;
     row_t row = 0;
     uint32_t qidx = 0, err = 0;
     auto fetch = [&]() {
-        uint32_t lo = single ? t : 0, hi = single ? t + 1 : nh;
-        while (hi - lo > 1) {
-            uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(starts + mid) <= t) lo = mid; else hi = mid;
-        }
-        const HitRec* h = hits + lo;
-        row = __ldg(&h->lb) + (single ? 0u : t - __ldg(starts + lo));
-        qidx = __ldg(&h->qidx);
-        err = __ldg(&h->e);
+        const uint32_t h = hit_of(starts, nh, t, single);
+        row = hit_row(hits, starts, h, t, single);
+        qidx = __ldg(&hits[h].qidx);
+        err = __ldg(&hits[h].e);
         steps = 0;
     };
     bool active = t < total;
     if (active) fetch();
     while (active) {
-        uint32_t a0, a1, a2, a3, a4, a5, a6, a7;
-        asm volatile("ld.global.nc.L1::no_allocate.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                     : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(a3), "=r"(a4), "=r"(a5), "=r"(a6), "=r"(a7)
-                     : "l"(ix.locblocks + ((size_t)(row >> 6) * 4 + role * 2)));
-        uint32_t mine;                                       // role 1: sampled ? 1 + sample index : 0;  role 0: next row
-        if (role) {
-            uint64_t bits = (uint64_t)a0 | ((uint64_t)a1 << 32);
-            uint32_t o = row & 63;
-            mine = ((bits >> o) & 1) ? 1u + a2 + __popcll(bits & low_mask(o)) : 0u;
-        } else {
-            DnaBlock b;
-            b.cnt[0] = a0; b.cnt[1] = a1; b.cnt[2] = a2; b.cnt[3] = a3;
-            b.p0 = (uint64_t)a4 | ((uint64_t)a5 << 32);
-            b.p1 = (uint64_t)a6 | ((uint64_t)a7 << 32);
-            uint32_t c = occ.symbol(b, row);
-            mine = ix.C[c] + occ.rank(b, row, c);
-        }
-        uint32_t other = __shfl_xor_sync(pmask, mine, 1);
-        uint32_t sampled = role ? mine : other;
+        const uint32_t sampled = pair_step(ix, role, pmask, row);
         if (sampled) {
             if (role == 0) {
                 uint2 sample = __ldg(ix.samples + (sampled - 1));
@@ -1009,7 +944,6 @@ __global__ void __launch_bounds__(256) locate_pair_kernel(const __grid_constant_
             active = t < total;
             if (active) fetch();
         } else {
-            row = role ? other : mine;
             ++steps;
         }
     }
@@ -1024,30 +958,11 @@ __global__ void __launch_bounds__(256) locrow_build_kernel(const __grid_constant
     uint64_t t = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
     const uint32_t role = threadIdx.x & 1;
     const uint32_t pmask = 3u << (threadIdx.x & 30);
-    const OccDna& occ = ix.occ[0];
     uint32_t steps = 0;
     row_t row = (row_t)t;
     bool active = t < ix.n;
     while (active) {
-        uint32_t a0, a1, a2, a3, a4, a5, a6, a7;
-        asm volatile("ld.global.nc.L1::no_allocate.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                     : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(a3), "=r"(a4), "=r"(a5), "=r"(a6), "=r"(a7)
-                     : "l"(ix.locblocks + ((size_t)(row >> 6) * 4 + role * 2)));
-        uint32_t mine;
-        if (role) {
-            uint64_t bits = (uint64_t)a0 | ((uint64_t)a1 << 32);
-            uint32_t o = row & 63;
-            mine = ((bits >> o) & 1) ? 1u + a2 + __popcll(bits & low_mask(o)) : 0u;
-        } else {
-            DnaBlock b;
-            b.cnt[0] = a0; b.cnt[1] = a1; b.cnt[2] = a2; b.cnt[3] = a3;
-            b.p0 = (uint64_t)a4 | ((uint64_t)a5 << 32);
-            b.p1 = (uint64_t)a6 | ((uint64_t)a7 << 32);
-            uint32_t c = occ.symbol(b, row);
-            mine = ix.C[c] + occ.rank(b, row, c);
-        }
-        uint32_t other = __shfl_xor_sync(pmask, mine, 1);
-        uint32_t sampled = role ? mine : other;
+        const uint32_t sampled = pair_step(ix, role, pmask, row);
         if (sampled) {
             if (role == 0) {
                 const uint32_t idx = sampled - 1;
@@ -1059,7 +974,6 @@ __global__ void __launch_bounds__(256) locrow_build_kernel(const __grid_constant
             row = (row_t)t;
             steps = 0;
         } else {
-            row = role ? other : mine;
             ++steps;
         }
     }
@@ -1071,45 +985,31 @@ __global__ void __launch_bounds__(256) locrow_build_gen_kernel(const __grid_cons
                                                                uint32_t* __restrict__ overflow) {
     const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= ix.n) return;
-    const OCC& occ = ix.occ[0];
-    row_t row = (row_t)t;
     uint32_t steps = 0;
-    for (;;) {
-        const uint4 m = __ldg(ix.marks + (row >> 6));
-        typename OCC::Block b = occ.load(row >> 6, 0);
-        const uint64_t bits = (uint64_t)m.x | ((uint64_t)m.y << 32);
-        const uint32_t o = row & 63;
-        if ((bits >> o) & 1) {
-            const uint32_t idx = m.z + __popcll(bits & low_mask(o));
-            if (steps >= (1u << step_bits) || idx >= (1u << (32 - step_bits))) atomicOr(overflow, 1u);
-            out[t] = (idx << step_bits) | steps;
-            return;
-        }
-        const uint32_t c = occ.symbol(b, row);
-        if (OCC::kSymbolLoad) b = occ.load(row >> 6, c);
-        row = ix.C[c] + occ.rank(b, row, c);
-        if (++steps > (1u << 20)) { atomicOr(overflow, 1u); out[t] = 0; return; }     // no sample on this walk (cannot be located anyway)
-    }
+    const uint32_t idx = walk_to_sample(ix, (row_t)t, steps, 1u << 20);
+    if (idx == kNoSample) { atomicOr(overflow, 1u); out[t] = 0; return; }     // no sample on this walk (cannot be located anyway)
+    if (steps >= (1u << step_bits) || idx >= (1u << (32 - step_bits))) atomicOr(overflow, 1u);
+    out[t] = (idx << step_bits) | steps;
 }
 
 // Text check tables (fmb_index::isa / text2), one thread per row: (seq, pos) of the row from the locate shortcut, g = start[seq] + pos;
 // isa[g] = row, and BWT[row] is the symbol at g - 1 (a delimiter when pos == 0: those positions keep code 0, no read window reaches
 // them).  flags[0] = a row outside its sequence, flags[1] = the largest LF step count of any row.
-__global__ void __launch_bounds__(256) text_tables_kernel(const __grid_constant__ IndexView<OccDna> ix, const uint32_t* __restrict__ start, uint32_t nseq,
-                                                          uint32_t* __restrict__ isa, uint32_t* __restrict__ text, uint32_t* __restrict__ flags) {
+__global__ void __launch_bounds__(256) text_tables_kernel(const __grid_constant__ IndexView<OccDna> ix, const __grid_constant__ RowPosView rp,
+                                                          const uint32_t* __restrict__ start, uint32_t nseq, uint32_t* __restrict__ isa,
+                                                          uint32_t* __restrict__ text, uint32_t* __restrict__ flags) {
     const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     uint32_t steps = 0;
     if (r < ix.n) {
-        const uint32_t w = __ldg(ix.locrow + r);
-        steps = w & ((1u << ix.loc_step_bits) - 1u);
-        const uint2 s = __ldg(ix.samples + (w >> ix.loc_step_bits));
-        const uint32_t p = s.y + steps;
-        if (s.x >= nseq || p >= __ldg(start + s.x + 1) - __ldg(start + s.x)) {
+        uint32_t lines = 0;
+        const RowPos p = row_pos<false>(rp, (row_t)r, lines);
+        steps = p.steps;
+        if (p.seq >= nseq || p.pos >= __ldg(start + p.seq + 1) - __ldg(start + p.seq)) {
             atomicOr(flags, 1u);
         } else {
-            const uint32_t g = __ldg(start + s.x) + p;
+            const uint32_t g = __ldg(start + p.seq) + p.pos;
             isa[g] = (uint32_t)r;
-            if (p) {
+            if (p.pos) {
                 const DnaBlock b = ix.occ[0].load((uint32_t)(r >> 6), 0);
                 const uint32_t c = ix.occ[0].symbol(b, (row_t)r);
                 atomicOr(text + ((g - 1) >> 4), ((c - 1) & 3u) << (2 * ((g - 1) & 15)));
@@ -1126,79 +1026,37 @@ __global__ void __launch_bounds__(256) sample_rate_kernel(const uint2* __restric
     if (i < count && samples[i].y % rate) atomicOr(bad, 1u);
 }
 // the locate shortcut turned into the suffix array in place (text-regular sampling, after text_tables_kernel checked every row):
-// rows[r] = start[seq] + pos of the row's sample + the row's steps
-__global__ void __launch_bounds__(256) sa_from_locrow_kernel(const uint2* __restrict__ samples, const uint32_t* __restrict__ start, uint32_t step_bits,
-                                                             uint64_t n, uint32_t* rows) {
+// rows[r] = g of row r, rows = rp.locrow (each thread reads its own word once, before it overwrites it)
+__global__ void __launch_bounds__(256) sa_from_locrow_kernel(const __grid_constant__ RowPosView rp, uint64_t n, uint32_t* rows) {
     const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     if (r >= n) return;
-    const uint32_t w = rows[r];
-    const uint2 s = __ldg(samples + (w >> step_bits));
-    rows[r] = __ldg(start + s.x) + s.y + (w & ((1u << step_bits) - 1u));
+    uint32_t lines = 0;
+    rows[r] = row_pos<true>(rp, (row_t)r, lines).g;
 }
 
-// K4d: locate through the suffix array (fmb_index::sa): one fetch per row plus the (cached) sequence lookup.  Sampling is text-regular at
-// rate `rate`, so the LF walk to the row's sample would take pos % rate steps; rows the text check of exact search found (at, as in
-// locate_shortcut_kernel) need no fetch at all.
-__global__ void __launch_bounds__(256) locate_sa_kernel(const HitRec* __restrict__ hits, const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total,
-                                                        uint32_t single, const uint2* __restrict__ at, uint32_t rate, const uint32_t* __restrict__ sa,
-                                                        const uint2* __restrict__ seq_of_block, const uint32_t* __restrict__ seq_start,
-                                                        LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
-    uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    uint32_t steps = 0;
-    if (t < total) {
-        uint32_t lo = single ? t : 0, hi = single ? t + 1 : nh;
-        while (hi - lo > 1) {
-            uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(starts + mid) <= t) lo = mid; else hi = mid;
-        }
-        const HitRec* h = hits + lo;
-        LocRec r;
-        r.qidx = __ldg(&h->qidx); r.e = __ldg(&h->e);
-        const uint2 a = at ? __ldg(at + lo) : make_uint2(kNoSeq, 0u);      // a checked hit is a single row
-        if (a.x != kNoSeq) {
-            r.seq = a.x; r.pos = a.y;
-        } else {
-            const row_t row = __ldg(&h->lb) + (single ? 0u : t - __ldg(starts + lo));
-            const uint32_t g = __ldg(sa + row);
-            uint32_t lines = 0;
-            const SeqStart ss = seq_of(seq_of_block, seq_start, g, lines);
-            r.seq = ss.seq; r.pos = g - ss.start;
-        }
-        steps = r.pos % rate;
-        out[t] = r;
-    }
-    // the LF steps the walk WOULD take: the algorithmic work of SURVEY.md §8d stays reported
-    block_count2(counters, 2, steps, 1, steps);
-}
-
+// K4d: locate through the shortcut table in either form (RowPosView): the suffix array (one fetch per row plus the cached sequence
+// entry; sampling is text-regular, so the walk would take pos % rate steps) or the shortcut word plus the sample.
 // at (may be nullptr): (seq, pos) per record found by the text check of exact search (kNoSeq: not checked); with text-regular sampling
-// at rate `rate` such a row needs pos % rate LF steps and no index access
-template <class OCC>
-__global__ void __launch_bounds__(256) locate_shortcut_kernel(const __grid_constant__ IndexView<OCC> ix, const HitRec* __restrict__ hits,
+// at rate rp.rate such a row needs pos % rate LF steps and no index access
+__global__ void __launch_bounds__(256) locate_shortcut_kernel(const __grid_constant__ RowPosView rp, const HitRec* __restrict__ hits,
                                                               const uint32_t* __restrict__ starts, uint32_t nh, uint32_t total, uint32_t single,
-                                                              const uint2* __restrict__ at, uint32_t rate,
-                                                              LocRec* __restrict__ out, unsigned long long* __restrict__ counters) {
+                                                              const uint2* __restrict__ at, LocRec* __restrict__ out,
+                                                              unsigned long long* __restrict__ counters) {
     uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t steps = 0;
     if (t < total) {
-        uint32_t lo = single ? t : 0, hi = single ? t + 1 : nh;
-        while (hi - lo > 1) {
-            uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(starts + mid) <= t) lo = mid; else hi = mid;
-        }
-        const HitRec* h = hits + lo;
+        const uint32_t h = hit_of(starts, nh, t, single);
         LocRec r;
-        r.qidx = __ldg(&h->qidx); r.e = __ldg(&h->e);
-        const uint2 a = at ? __ldg(at + lo) : make_uint2(kNoSeq, 0u);      // a checked hit is a single row
+        r.qidx = __ldg(&hits[h].qidx); r.e = __ldg(&hits[h].e);
+        const uint2 a = at ? __ldg(at + h) : make_uint2(kNoSeq, 0u);      // a checked hit is a single row
         if (a.x != kNoSeq) {
-            steps = a.y % rate;
+            steps = a.y % rp.rate;
             r.seq = a.x; r.pos = a.y;
         } else {
-            const row_t row = __ldg(&h->lb) + (single ? 0u : t - __ldg(starts + lo));
-            const uint32_t w = __ldg(ix.locrow + row);
-            steps = w & ((1u << ix.loc_step_bits) - 1u);
-            const uint2 sample = __ldg(ix.samples + (w >> ix.loc_step_bits));
-            r.seq = sample.x; r.pos = sample.y + steps;
+            uint32_t lines = 0;
+            const RowPos p = row_pos<false>(rp, hit_row(hits, starts, h, t, single), lines);
+            steps = p.steps;
+            r.seq = p.seq; r.pos = p.pos;
         }
         out[t] = r;
     }
@@ -1212,26 +1070,11 @@ __global__ void __launch_bounds__(256) locate_rows_kernel(const __grid_constant_
                                                           uint32_t* __restrict__ seq, uint32_t* __restrict__ pos, uint64_t* __restrict__ steps_out) {
     uint64_t t = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     if (t >= count) return;
-    row_t row = (row_t)rows[t];
-    const OCC& occ = ix.occ[0];
     uint32_t steps = 0;
-    for (;;) {
-        uint4 m = __ldg(ix.marks + (row >> 6));
-        typename OCC::Block b = occ.load(row >> 6, 0);
-        uint64_t bits = (uint64_t)m.x | ((uint64_t)m.y << 32);
-        uint32_t o = row & 63;
-        if ((bits >> o) & 1) {
-            uint2 sample = __ldg(ix.samples + (m.z + __popcll(bits & low_mask(o))));
-            seq[t] = sample.x;
-            pos[t] = sample.y;
-            steps_out[t] = steps;
-            return;
-        }
-        uint32_t c = occ.symbol(b, row);
-        if (OCC::kSymbolLoad) b = occ.load(row >> 6, c);
-        row = ix.C[c] + occ.rank(b, row, c);
-        ++steps;
-    }
+    const uint2 sample = __ldg(ix.samples + walk_to_sample(ix, (row_t)rows[t], steps));
+    seq[t] = sample.x;
+    pos[t] = sample.y;
+    steps_out[t] = steps;
 }
 
 // Measurement aid (SURVEY.md §8d "empirical ceiling"): independent -- not pointer chasing -- random gathers over one of the index's

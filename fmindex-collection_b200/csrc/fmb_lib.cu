@@ -190,8 +190,6 @@ fmb::IndexView<fmb::OccDna> fmb_index::view_dna() const {
     v.marks = marks.p;
     v.samples = samples.p;
     v.locblocks = locblocks.p;
-    v.locrow = locrow.p;
-    v.loc_step_bits = loc_step_bits;
     return v;
 }
 
@@ -210,8 +208,6 @@ fmb::IndexView<fmb::OccGen> fmb_index::view_gen() const {
     v.marks = marks.p;
     v.samples = samples.p;
     v.locblocks = nullptr;
-    v.locrow = locrow.p;
-    v.loc_step_bits = loc_step_bits;
     return v;
 }
 
@@ -242,13 +238,12 @@ fmb::Occ2View fmb_index::view_occ2() const {
     v.kmer_k = kmer_k;
     v.isa = isa.p;
     v.text32 = text2.p;
-    v.seq_start = seq_start_d.p;
-    v.sa = sa.p;
-    v.seq_of_block = seq_of_block.p;
-    v.locrow = locrow.p;
-    v.samples = samples.p;
-    v.loc_step_bits = loc_step_bits;
+    v.rowpos = view_rowpos();
     return v;
+}
+
+fmb::RowPosView fmb_index::view_rowpos() const {
+    return fmb::RowPosView{sa.p, seq_of_block.p, seq_start_d.p, locrow.p, samples.p, loc_step_bits, text_rate};
 }
 
 uint64_t fmb_index::device_bytes() const {
@@ -690,7 +685,7 @@ static int build_text_check(fmb_index* ix) {
     FMB_CUDA(cudaMemcpyAsync(start.p, h_start.data(), (nseq + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     FMB_CUDA(cudaMemsetAsync(text.p, 0, words * sizeof(uint32_t), st));
     FMB_CUDA(cudaMemsetAsync(flags.p, 0, 3 * sizeof(uint32_t), st));
-    text_tables_kernel<<<grid_for(n, 256), 256, 0, st>>>(ix->view_dna(), start.p, (uint32_t)nseq, isa.p, text.p, flags.p);
+    text_tables_kernel<<<grid_for(n, 256), 256, 0, st>>>(ix->view_dna(), ix->view_rowpos(), start.p, (uint32_t)nseq, isa.p, text.p, flags.p);
     FMB_CUDA(cudaGetLastError());
     uint32_t h_flags[3] = {0, 0, 0};
     FMB_CUDA(cudaMemcpyAsync(h_flags, flags.p, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
@@ -704,6 +699,7 @@ static int build_text_check(fmb_index* ix) {
     note_launches(2);
     ix->isa = std::move(isa);
     ix->text2 = std::move(text);
+    ix->seq_start_d = std::move(start);
     ix->text_rate = h_flags[2] ? 0u : rate;
     // text-regular sampling: every row's step count is pos % text_rate, so the shortcut's sample index and steps say no more than the
     // row's text position -- the suffix array takes its place (same 4 bytes per row) and locates a row with one fetch
@@ -720,7 +716,7 @@ static int build_text_check(fmb_index* ix) {
         DevBuf<uint2> d_sob;
         FMB_TRY(d_sob.alloc(nb));
         FMB_CUDA(cudaMemcpyAsync(d_sob.p, sob.data(), nb * sizeof(uint2), cudaMemcpyHostToDevice, st));
-        sa_from_locrow_kernel<<<grid_for(n, 256), 256, 0, st>>>(ix->samples.p, start.p, ix->loc_step_bits, n, ix->locrow.p);
+        sa_from_locrow_kernel<<<grid_for(n, 256), 256, 0, st>>>(ix->view_rowpos(), n, ix->locrow.p);
         FMB_CUDA(cudaGetLastError());
         FMB_CUDA(cudaStreamSynchronize(st));
         note_launches(1);
@@ -728,7 +724,6 @@ static int build_text_check(fmb_index* ix) {
         ix->loc_step_bits = 0;
         ix->seq_of_block = std::move(d_sob);
     }
-    ix->seq_start_d = std::move(start);
     return FMB_OK;
 }
 
@@ -1397,14 +1392,10 @@ int fmb_locate(const fmb_index* ix, const fmb_results* hits, fmb_results** out) 
     cudaEventCreate(&ev_m1);
     if (total) {
         cudaEventRecord(ev_m0, st);
-        if (ix->sa.p && ix->locate_mode != FMB_LOCATE_WALK) {
-            const uint2* at = hits->dense ? hits->at.p : nullptr;
-            locate_sa_kernel<<<grid_for(total, 256), 256, 0, st>>>(hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, at, ix->text_rate, ix->sa.p,
-                                                                   ix->seq_of_block.p, ix->seq_start_d.p, res->locs.p, ctr.p);
-        } else if (ix->locrow.p && ix->locate_mode != FMB_LOCATE_WALK) {
+        if ((ix->sa.p || ix->locrow.p) && ix->locate_mode != FMB_LOCATE_WALK) {
             const uint2* at = hits->dense && ix->text_rate ? hits->at.p : nullptr;
-            FMB_DISPATCH(ix, v, locate_shortcut_kernel<<<grid_for(total, 256), 256, 0, st>>>(v, hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, at, ix->text_rate,
-                                                                                             res->locs.p, ctr.p));
+            locate_shortcut_kernel<<<grid_for(total, 256), 256, 0, st>>>(ix->view_rowpos(), hits->hits.p, starts.p, (uint32_t)nh, total, single ? 1u : 0u, at,
+                                                                         res->locs.p, ctr.p);
         } else if (ix->dna && ix->locblocks.p) {
             auto v = ix->view_dna();
             // persistent grid: every SM full of lane pairs (8 blocks x 256 threads), rows handed out with a grid stride

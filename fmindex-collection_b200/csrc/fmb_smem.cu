@@ -20,7 +20,7 @@
 // one scatter put them in (qidx, begin) order.  The staging list grows and the search reruns when it was too small.
 //
 // Text path (FMB_TEXT_CHECK: DNA layout with delimiter; queries without a non-matching symbol).  Once the interval of Q[x:j] is one
-// row, Q[x:j] occurs once, at the text position g of that row (locate shortcut + sample + sequence start), and Q[x:j+1] occurs iff
+// row, Q[x:j] occurs once, at the text position g of that row (row_pos: suffix array or locate shortcut), and Q[x:j+1] occurs iff
 // the text continues with Q[j] inside the same sequence: the rest of the right phase compares the 2-bit text with the packed query
 // 16 symbols (one 32-bit word) at a time, the first mismatch coming from the XOR of the two words; the row does not change.  The
 // text gives delimiter positions the code of symbol 1, so every comparison is bounded by the sequence borders, never by codes.
@@ -57,12 +57,7 @@ struct SmemArgs {
     const uint4* bikmer;          // nullptr: no k-mer seeding
     uint32_t bikmer_k, bikmer_base;   // base 0: 2-bit key (DNA layout)
     const uint32_t* text32;       // nullptr: no text path
-    const uint32_t* seq_start;
-    const uint32_t* sa;           // nullptr: locrow + samples
-    const uint2* seq_of_block;
-    const uint32_t* locrow;
-    const uint2* samples;
-    uint32_t loc_step_bits;
+    RowPosView rowpos;
     SmemStage* stage;
     unsigned long long cap;       // records the staging list holds
     uint32_t* counts;             // per query: SMEMs reported
@@ -90,26 +85,14 @@ __global__ void __launch_bounds__(256) smem_kernel(const __grid_constant__ Index
     const Cursor whole{0, 0, ix.n, 0};
     auto sym = [&](uint32_t p) -> uint32_t { return __ldg(a.qsym + off + p); };
     auto matches = [&](uint32_t c) { return c >= 1 && c < ix.sigma; };
-    // text position of the suffix of `row` (suffix array, or locate shortcut + sample) and the borders of its sequence
+    // text position of the suffix of `row` and the borders of its sequence
     auto text_pos = [&](row_t row) -> uint32_t {
-        uint32_t g;
-        if (a.sa) {
-            g = __ldg(a.sa + row);
-            lines += 1;
-            const SeqStart ss = seq_of(a.seq_of_block, a.seq_start, g, lines);
-            tseq = ss.seq;
-            tbeg = ss.start;
-        } else {
-            const uint32_t w = __ldg(a.locrow + row);
-            const uint2 smp = __ldg(a.samples + (w >> a.loc_step_bits));
-            tseq = smp.x;
-            tbeg = __ldg(a.seq_start + tseq);
-            lines += 3;
-            g = tbeg + smp.y + (w & ((1u << a.loc_step_bits) - 1u));
-        }
-        tend = __ldg(a.seq_start + tseq + 1) - 1;          // the sequence's delimiter
+        const RowPos p = row_pos<true>(a.rowpos, row, lines);
+        tseq = p.seq;
+        tbeg = p.start;
+        tend = __ldg(a.rowpos.seq_start + tseq + 1) - 1;          // the sequence's delimiter
         lines += 1;
-        return g;
+        return p.g;
     };
     for (;;) {
         // ---- resolve: everything up to the next extension this lane needs --------------------------------------------------------
@@ -128,7 +111,7 @@ __global__ void __launch_bounds__(256) smem_kernel(const __grid_constant__ Index
                 off = a.qoff[q];
                 m = (uint32_t)(a.qoff[q + 1] - off);
                 x = 0; k = 0; tg = kNone;
-                text = a.text32 && !a.qflags[q];
+                text = !OCC::kSymbolLoad && a.text32 && !a.qflags[q];      // the text tables exist on the DNA layout only
                 ph = PH_NEW;
             } else if (ph == PH_NEW) {
                 if (x >= m) { a.counts[q] = k; ph = PH_IDLE; continue; }
@@ -304,12 +287,7 @@ int fmb_search_smems(const fmb_index* ix, const fmb_queries* q, uint32_t min_len
     }
     if (ix->isa.p && q->packed.p && q->flags.p) {
         args.text32 = ix->text2.p;
-        args.seq_start = ix->seq_start_d.p;
-        args.sa = ix->sa.p;
-        args.seq_of_block = ix->seq_of_block.p;
-        args.locrow = ix->locrow.p;
-        args.samples = ix->samples.p;
-        args.loc_step_bits = ix->loc_step_bits;
+        args.rowpos = ix->view_rowpos();
     }
     args.counts = counts.p;
     args.ctr = ctr.p;

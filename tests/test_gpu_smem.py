@@ -221,7 +221,7 @@ def test_against_oracle(gpu, sigma, kind):
         assert r.stats.line_requests > 0
 
 
-@pytest.mark.parametrize("knobs", [("FMB_NO_BIKMER",), ("FMB_NO_TEXTCHECK",), ("FMB_NO_JUMP",),
+@pytest.mark.parametrize("knobs", [("FMB_NO_BIKMER",), ("FMB_NO_TEXTCHECK",), ("FMB_NO_JUMP",), ("FMB_NO_SA",),
                                    ("FMB_NO_BIKMER", "FMB_NO_TEXTCHECK", "FMB_NO_JUMP")])
 @pytest.mark.parametrize("sigma", [5, 21])
 def test_table_knobs(gpu, monkeypatch, sigma, knobs):
